@@ -14,6 +14,11 @@ all-reduce.  With N GPUs the reads are sharded N ways (strong scaling).
 `value` times the pass with the FASTQ image already resident in HBM; `e2e`
 times the same job through tdg_submit from PINNED HOST memory (H2D inside the
 timed region) plus the device-to-host read of the count matrix.
+
+`--dump-outputs DIR` writes the count matrix of the last timed step to
+DIR/counts.npy (float64, exact for int32 counts; 96 x 40,000 cells = 31 MB).
+The reads come from a seeded generator, so two builds given the same arguments
+count the same job and their files can be compared cell for cell.
 """
 
 import argparse
@@ -352,7 +357,13 @@ def main():
     ap.add_argument("--file-reads", type=int, default=8_000_000, help="reads in the files of the file -> matrix legs")
     ap.add_argument("--verify-reads", type=int, default=20_000_000,
                     help="reads of the job compared exactly with the C oracle (outside the timed region)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the count matrix of the last timed step to DIR/counts.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours (the reference arm keeps no count matrix)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -458,6 +469,10 @@ def main():
         tag_hits = tot[2] // nsteps_total
     ok = bool((matrix >= exp_t).all().item()) and msum == tag_hits and reads_seen == nreads
     check = "ok" if ok else "FAILED"
+    if rank == 0 and args.dump_outputs:
+        # before the legs below, which count into the same matrix
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "counts.npy"), matrix.cpu().numpy().astype(np.float64))
 
     # ---- roofline of the count kernel (rank 0's launches) --------------------------
     peaks = {}
@@ -696,7 +711,7 @@ def usable_procs(per_proc_gb=2.0):
 
 
 def reference_arm(args, world):
-    """CPU arm: the unmodified reference (oracle/_ref, staged from /root/reference by
+    """CPU arm: the unmodified reference (oracle/_ref, staged from $TAGDIGGER_REFERENCE by
     oracle/stage_ref.py) on all host cores, each step a bounded sample of the same workload."""
     import shutil
     import tempfile

@@ -64,16 +64,15 @@ def in_tmp(tmp_path):
         os.chdir(old)
 
 
+NO_REFERENCE = "the original tagdigger is not staged in oracle/_ref (oracle/stage_ref.py)"
+
+
 def have_reference():
-    return os.path.exists("/root/reference/tagdigger_fun.py")
+    from oracle import stage_ref
+    return stage_ref.staged()
 
 
 def import_reference():
-    """The live reference (build container only)."""
-    import importlib
-    import warnings
-    if "/root/reference" not in sys.path:
-        sys.path.append("/root/reference")
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        return importlib.import_module("tagdigger_fun")
+    """The live reference: the unmodified copy staged in oracle/_ref."""
+    from oracle import stage_ref
+    return stage_ref.import_ref()

@@ -1,10 +1,9 @@
 #!/usr/bin/env python3
 """Generate the golden vectors under tests/golden/ by RUNNING THE REFERENCE.
 
-Run in the build container only (it imports /root/reference/tagdigger_fun.py,
-which does not exist on the GPU box):
+Run where a checkout of the reference exists (it imports its tagdigger_fun.py):
 
-    python tests/golden/make_golden.py
+    TAGDIGGER_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 Every case is recorded as: the function called, the input files (text, or
 base64 for gzip), the arguments, and what the reference did -- return value,
@@ -30,7 +29,9 @@ import warnings
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("TAGDIGGER_REFERENCE")
+if not REF or not os.path.isfile(os.path.join(REF, "tagdigger_fun.py")):
+    sys.exit("usage: TAGDIGGER_REFERENCE=<checkout of the original TagDigger> python tests/golden/make_golden.py")
 sys.path.insert(0, REF)
 sys.path.insert(0, REPO)
 warnings.simplefilter("ignore")

@@ -1,5 +1,5 @@
-"""Live differential fuzzing of the host API mirror against the reference (build container only:
-skipped where /root/reference does not exist).  Every recorded reader case is re-run on randomly
+"""Live differential fuzzing of the host API mirror against the reference (skipped where the
+reference is not staged in oracle/_ref).  Every recorded reader case is re-run on randomly
 damaged copies of its input files -- lines dropped, duplicated, swapped, characters substituted --
 and the mirror must agree with the reference on return value, printed messages and exception."""
 
@@ -9,10 +9,10 @@ import random
 
 import pytest
 
-from conftest import file_bytes, have_reference, import_reference, load_golden
+from conftest import NO_REFERENCE, file_bytes, have_reference, import_reference, load_golden
 from tagdigger_b200 import hostio
 
-pytestmark = pytest.mark.skipif(not have_reference(), reason="/root/reference not present")
+pytestmark = pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 
 READERS = load_golden("readers.json")
 

@@ -1,5 +1,5 @@
 """The oracle (oracle/tagdigger_oracle.py) against the golden vectors recorded
-from the reference, and -- when /root/reference exists -- against the live
+from the reference, and -- when it is staged in oracle/_ref -- against the live
 reference on fresh random inputs.  CPU only."""
 
 import base64
@@ -10,7 +10,7 @@ import random
 import numpy as np
 import pytest
 
-from conftest import file_bytes, have_reference, import_reference, load_golden, materialize
+from conftest import NO_REFERENCE, file_bytes, have_reference, import_reference, load_golden, materialize
 from oracle import tagdigger_oracle as orc
 
 FIND = load_golden("find_tags.json") + load_golden("find_tags_text.json")     # + text-mode cases (UTF-8, maxreads stop)
@@ -93,9 +93,9 @@ def test_splitter_golden(in_tmp):
             assert buf.getvalue().encode() == base64.b64decode(case["outfiles"][name])
 
 
-# ---- live differential tests (build container only) ------------------------
+# ---- live differential tests (where the reference is staged in oracle/_ref) --
 
-needs_ref = pytest.mark.skipif(not have_reference(), reason="/root/reference not present")
+needs_ref = pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 
 
 def _rand_seq(r, n):

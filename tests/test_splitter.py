@@ -12,7 +12,7 @@ import random
 
 import pytest
 
-from conftest import have_reference, import_reference, load_golden, materialize
+from conftest import NO_REFERENCE, have_reference, import_reference, load_golden, materialize
 from helpers import rand_seq
 from oracle import tagdigger_oracle as orc
 from tagdigger_b200 import barcode_splitter_script, hostio
@@ -219,7 +219,7 @@ def test_streaming_splitter_progress_lines(in_tmp, monkeypatch):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not have_reference(), reason="/root/reference not present")
+@pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 def test_splitter_stdout_matches_reference(in_tmp):
     from tagdigger_b200 import splitter
     ref = import_reference()

@@ -9,7 +9,7 @@ import random
 
 import pytest
 
-from conftest import have_reference, import_reference, load_golden
+from conftest import NO_REFERENCE, have_reference, import_reference, load_golden
 from helpers import rand_seq
 from oracle import tagdigger_oracle as orc
 from tagdigger_b200 import hostio, trimming
@@ -95,13 +95,14 @@ def test_tables_equal_oracle_trie(name):
 def test_tables_golden_model():
     for case in GOLD:
         adapter = [tuple(x) for x in case["adapter"]]
+        assert hostio.adapters[case["adapter_name"]] == adapter      # recorded from the reference's adapters
         with contextlib.redirect_stdout(io.StringIO()):
             tables = trimming.trim_tables(adapter, case["barcodes"])
         for s, b, st, want in zip(case["seqs"], case["barindex"], case["searchstart"], case["slice2"]):
             assert tables_decide(s, tables, b, st) == want
 
 
-@pytest.mark.skipif(not have_reference(), reason="/root/reference not present")
+@pytest.mark.skipif(not have_reference(), reason=NO_REFERENCE)
 def test_fallback_messages_match_reference():
     ref = import_reference()
     rng = random.Random(5)
