@@ -32,6 +32,10 @@
 extern "C" {
 #endif
 
+/* The splitter's BGZF entry points (tdg_split_bgzf, tdg_bgzf_append, tdg_bgzf_finish) were added
+ * to version 2 without changing any existing signature or behaviour: every version-2 caller keeps
+ * working, and the version stays 2 because the test suite pins the ABI at 2.  A library built
+ * before them fails at symbol lookup when the binding loads it, not silently. */
 #define TDG_ABI_VERSION 2
 
 #define TDG_OK            0
@@ -237,7 +241,8 @@ int         tdg_memcpy_d2h(tdg_ctx *ctx, void *host, const void *dev, size_t n);
 uint64_t    tdg_launch_count(const tdg_ctx *ctx);
 /* Device time in milliseconds of the counting kernels launched between
  * tdg_timing_begin and tdg_timing_end (CUDA events on the context's stream,
- * one pair per kernel launch; at most 4096 launches).  tdg_timing_end
+ * one pair per kernel launch; at most 4096 launches), and of the BGZF writer's
+ * kernels (one pair per deflate-scan-pack sequence).  tdg_timing_end
  * synchronises; *nlaunch receives the number of kernels timed. */
 int         tdg_timing_begin(tdg_ctx *ctx);
 int         tdg_timing_end(tdg_ctx *ctx, double *kernel_ms, uint32_t *nlaunch);
@@ -288,13 +293,34 @@ int         tdg_split_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off,
  * caller handles bytes[0 .. consumed) itself.  Otherwise out[out_off[b] .. out_off[b+1]) are
  * the bytes to append to barcode b's file and flags[r] = 1 (barcode and cut site found)
  * | 2 (clipped on the 3' end) for every record; the three pointers are pinned host memory
- * owned by the context, valid until the next call. */
+ * owned by the context, valid until the next call.  With BGZF output on (tdg_split_bgzf), out /
+ * out_off carry the completed BGZF members of every barcode's file instead of plain bytes. */
 int         tdg_split_begin(tdg_ctx *ctx, const char *barcodes, const uint32_t *bar_off, uint32_t nbar,
                             uint32_t cutlen);
 int         tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block,
                             uint64_t max_records, uint64_t *n_records, uint64_t *consumed,
                             int *needs_host, const uint8_t **out, const uint64_t **out_off,
                             const uint8_t **flags);
+
+/* BGZF output files for the streaming splitter (the reference writes plain text only).  Every
+ * barcode's file is the series of gzip members bgzip writes: member k holds bytes
+ * [k * 65280, (k+1) * 65280) of the file's uncompressed stream (the last one may be short), with the
+ * `BC` extra field (FLG = 4, XLEN = 6, BSIZE = member size - 1), CRC32 and ISIZE; a member is at
+ * most 65,536 bytes (a dynamic-Huffman block, or stored blocks when those are not larger).  The cuts
+ * depend on the stream alone: every barcode's pending tail (< 65,280 bytes) is kept in the context
+ * between calls, and tdg_split_block and tdg_bgzf_append append to the same streams, in call order.
+ * tdg_split_bgzf: after tdg_split_begin; on != 0 switches BGZF output on and empties the tails
+ * (on = 0 switches it off; tdg_split_begin does too).
+ * tdg_bgzf_append: bytes[off[b] .. off[b+1]) (host memory, nbar + 1 offsets, at most 1 GiB in all)
+ * are appended to barcode b's stream -- the records the caller wrote itself after needs_host.
+ * tdg_bgzf_finish: the tails become the last members and every file ends with the 28-byte BGZF
+ * end-of-file member (a barcode without reads gets that member alone); the tails are empty after.
+ * Both return, like tdg_split_block, out[out_off[b] .. out_off[b+1]) = the bytes to append to
+ * barcode b's file, in pinned host memory owned by the context and valid until the next call. */
+int         tdg_split_bgzf(tdg_ctx *ctx, int on);
+int         tdg_bgzf_append(tdg_ctx *ctx, const uint8_t *bytes, const uint64_t *off,
+                            const uint8_t **out, const uint64_t **out_off);
+int         tdg_bgzf_finish(tdg_ctx *ctx, const uint8_t **out, const uint64_t **out_off);
 
 /* The host feed by itself (what tdg_count_file reads through): the uncompressed bytes of a
  * plain, gzip or BGZF file -- gzip.open(f, 'rt') / open(f, 'r') of tagdigger_fun.py:240-243

@@ -17,7 +17,7 @@ _CSRC = os.path.join(_HERE, "csrc")
 _INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_PATH = os.environ.get("TDG_LIB") or os.path.join(_HERE, "libtagdigger_b200.so")   # TDG_LIB: tuning builds (scripts/sweep.py)
 _SOURCES = ["tdg_api.cu", "tdg_text.h", "tdg_comm.h", "tdg_kernel.cuh", "tdg_match.h", "tdg_tables.h", "tdg_trim.cuh", "tdg_split.cuh", "tdg_feed.h", "tdg_pgz.h", "tdg_csv.h",
-            "tdg_gzlane.h", "tdg_gzchain.h", "tdg_gzdev.cuh", "tdg_gzfeed.cuh", "tdg_pool.h"]
+            "tdg_gzlane.h", "tdg_gzchain.h", "tdg_gzdev.cuh", "tdg_gzfeed.cuh", "tdg_pool.h", "tdg_bgzf.cuh"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-diag-suppress", "20014,20011", "-shared"]
@@ -37,7 +37,7 @@ tdg_bind_matrix tdg_zero_matrix tdg_begin_file tdg_reset_file tdg_submit tdg_end
 tdg_count_lines_device tdg_count_file tdg_count_file2 tdg_last_file_info tdg_gz_inflate_host tdg_release_scratch tdg_sync tdg_file_totals tdg_read_matrix tdg_matrix_min tdg_comm_unique_id tdg_comm_init tdg_allreduce_matrix tdg_finish
 tdg_matrix_device_ptr tdg_stream tdg_stream_wait tdg_other_stream_wait tdg_host_alloc
 tdg_host_free tdg_device_alloc tdg_device_free tdg_memcpy_h2d tdg_memcpy_d2h tdg_launch_count
-tdg_timing_begin tdg_timing_end tdg_set_trim tdg_trim_batch tdg_split_batch tdg_split_begin tdg_split_block tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
+tdg_timing_begin tdg_timing_end tdg_set_trim tdg_trim_batch tdg_split_batch tdg_split_begin tdg_split_block tdg_split_bgzf tdg_bgzf_append tdg_bgzf_finish tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
 
 
 class TdgError(RuntimeError):
@@ -142,6 +142,9 @@ def lib():
         "tdg_split_begin": (i32, [vp, vp, vp, u32, u32]),
         "tdg_split_block": (i32, [vp, vp, sz, i32, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32),
                                   ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp)]),
+        "tdg_split_bgzf": (i32, [vp, i32]),
+        "tdg_bgzf_append": (i32, [vp, vp, vp, ctypes.POINTER(vp), ctypes.POINTER(vp)]),
+        "tdg_bgzf_finish": (i32, [vp, ctypes.POINTER(vp), ctypes.POINTER(vp)]),
         "tdg_feed_open": (i32, [ctypes.POINTER(vp), ctypes.c_char_p, i32]),
         "tdg_feed_read": (ctypes.c_longlong, [vp, vp, sz]),
         "tdg_feed_close": (None, [vp]),
@@ -519,13 +522,41 @@ class Engine(object):
                                          ctypes.byref(off), ctypes.byref(flags)))
         if host.value or not out.value:
             return nrec.value, used.value, bool(host.value), None, None
-        nbar = self._split_nbar
-        offs = np.ctypeslib.as_array(ctypes.cast(off, ctypes.POINTER(u64)), shape=(nbar + 1,))
-        total = int(offs[nbar])
-        data = np.ctypeslib.as_array(ctypes.cast(out, ctypes.POINTER(ctypes.c_uint8)), shape=(max(total, 1),))
-        pieces = [data[int(offs[b]):int(offs[b + 1])] for b in range(nbar)]
+        pieces = self._pieces(out, off)
         fl = np.ctypeslib.as_array(ctypes.cast(flags, ctypes.POINTER(ctypes.c_uint8)), shape=(max(nrec.value, 1),))[:nrec.value]
         return nrec.value, used.value, False, pieces, fl
+
+    def _pieces(self, out, off):
+        """Per-barcode views of out[off[b] .. off[b+1]) (pinned memory of the context)."""
+        nbar = self._split_nbar
+        offs = np.ctypeslib.as_array(ctypes.cast(off, ctypes.POINTER(ctypes.c_uint64)), shape=(nbar + 1,))
+        total = int(offs[nbar])
+        data = np.ctypeslib.as_array(ctypes.cast(out, ctypes.POINTER(ctypes.c_uint8)), shape=(max(total, 1),))
+        return [data[int(offs[b]):int(offs[b + 1])] for b in range(nbar)]
+
+    def split_bgzf(self, on):
+        """BGZF output files for the split started by split_begin (empties every barcode's pending
+        tail).  While on, split_block's pieces are completed BGZF members; bgzf_append takes the
+        records written on the host, bgzf_finish ends the files."""
+        self._ck(self._L.tdg_split_bgzf(self._h, 1 if on else 0))
+
+    def bgzf_append(self, parts):
+        """parts[b]: bytes appended to barcode b's uncompressed stream.  Returns the BGZF pieces to
+        append to every barcode's file (views valid until the next call)."""
+        if len(parts) != self._split_nbar:
+            raise ValueError("one part per barcode: %d given, %d barcodes" % (len(parts), self._split_nbar))
+        blob = b"".join(bytes(p) for p in parts)
+        off = np.zeros(self._split_nbar + 1, dtype=np.uint64)
+        np.cumsum([len(p) for p in parts], out=off[1:])
+        out, o = ctypes.c_void_p(), ctypes.c_void_p()
+        self._ck(self._L.tdg_bgzf_append(self._h, blob, off.ctypes.data, ctypes.byref(out), ctypes.byref(o)))
+        return self._pieces(out, o)
+
+    def bgzf_finish(self):
+        """The last member of every barcode's file and the BGZF end-of-file member."""
+        out, o = ctypes.c_void_p(), ctypes.c_void_p()
+        self._ck(self._L.tdg_bgzf_finish(self._h, ctypes.byref(out), ctypes.byref(o)))
+        return self._pieces(out, o)
 
     def match_batch(self, seqs):
         """seqs: list of stripped sequence lines (bytes/str).  Returns (row, col) arrays, -1 = no match."""

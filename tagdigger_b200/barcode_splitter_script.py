@@ -19,6 +19,8 @@ def build_parser():
     p.add_argument("-b", "--barcodefile", help="Name of barcode key file", required=True)
     p.add_argument("-a", "--adapter", help="Name of the adapter set", required=True,
                    choices=sorted(hostio.adapters.keys()))
+    p.add_argument("--bgzf", action="store_true",
+                   help="Write the output files BGZF-compressed (bgzip's format; their names must end in 'gz')")
     return p
 
 
@@ -36,7 +38,7 @@ def main(argv=None):
         print([f for f, ok in zip(fqfiles, fqok) if not ok])
         raise Exception("Cannot read all FASTQ files.")
     for f in fqfiles:
-        splitter.barcodeSplitter(f, bckeys[f][0], bckeys[f][1], cutsite=cutsite, adapter=adapter)
+        splitter.barcodeSplitter(f, bckeys[f][0], bckeys[f][1], cutsite=cutsite, adapter=adapter, bgzf=args.bgzf)
     return 0
 
 

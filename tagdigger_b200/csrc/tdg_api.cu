@@ -27,6 +27,7 @@
 #include "tdg_split.cuh"
 #include "tdg_gzchain.h"
 #include "tdg_gzdev.cuh"
+#include "tdg_bgzf.cuh"
 
 static_assert(TDG_HALO_BYTES >= tdg::HALO, "the allocation slack promised by the header must cover the kernel halo");
 static_assert(TDG_TILE_BYTES >= tdg::TILE, "the allocation granule promised by the header must cover a kernel tile");
@@ -200,6 +201,15 @@ struct tdg_ctx {
     Grow sp_hout, sp_hflags, sp_hbase;                                                          // pinned host
     uint32_t sp_nbar = 0, sp_cutlen = 0;
     bool have_split = false;
+
+    // BGZF output of the splitter (tdg_split_bgzf, tdg_bgzf.cuh): every barcode's pending tail
+    // (< 65,280 bytes) waits in bz_tail between calls
+    bool bz_on = false, bz_attr = false;
+    Grow bz_tail, bz_src, bz_mem, bz_copy, bz_match, bz_work, bz_size, bz_out;      // device
+    Grow bz_hmem, bz_hcopy, bz_hsize, bz_hout;                                     // pinned host
+    std::vector<uint32_t> bz_tail_len;
+    std::vector<uint64_t> bz_off;
+    uint32_t bz_op[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 
     // pinned buffers of tdg_count_file (kept between files: pinning 192 MiB costs ~0.1 s)
     uint8_t *file_buf[3] = {nullptr, nullptr, nullptr};
@@ -731,6 +741,10 @@ void tdg_destroy(tdg_ctx *ctx)
                                  &ctx->sp_base, &ctx->sp_out, &ctx->sp_tabs})
             if (g->p) cudaFree(g->p);
         for (tdg_ctx::Grow *g : {&ctx->sp_hout, &ctx->sp_hflags, &ctx->sp_hbase})
+            if (g->p) cudaFreeHost(g->p);
+        for (tdg_ctx::Grow *g : {&ctx->bz_tail, &ctx->bz_src, &ctx->bz_mem, &ctx->bz_copy, &ctx->bz_match, &ctx->bz_work, &ctx->bz_size, &ctx->bz_out})
+            if (g->p) cudaFree(g->p);
+        for (tdg_ctx::Grow *g : {&ctx->bz_hmem, &ctx->bz_hcopy, &ctx->bz_hsize, &ctx->bz_hout})
             if (g->p) cudaFreeHost(g->p);
         for (tdg_ctx::Grow *g : {&ctx->gz_comp, &ctx->gz_comp2, &ctx->gz_syms, &ctx->gz_sym2, &ctx->gz_ntok, &ctx->gz_meta, &ctx->gz_cand, &ctx->gz_ncand, &ctx->gz_windows,
                                  &ctx->gz_text, &ctx->gz_crc, &ctx->gz_lens, &ctx->gz_offs, &ctx->gz_tabs, &ctx->gz_carry, &ctx->gz_cold})
@@ -1614,6 +1628,164 @@ int tdg_split_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, uint32_
 // ---------------------------------------------------------------------------
 // Streaming barcode splitter, csrc/tdg_split.cuh
 
+// BGZF members of the splitter's streams (tdg_bgzf.cuh).  Barcode b's stream gains the device bytes
+// d_new[off[b] .. off[b+1]) behind its pending tail; every complete 65,280 bytes become a member and the
+// rest is the new tail.  finish: the tails become the last members, and every file gets the EOF member.
+// Members are planned here, one CTA each deflates them, and they come back end to end in barcode order:
+// *out (pinned, owned by the context) with barcode b's bytes at [(*out_off)[b], (*out_off)[b+1]).
+static int bgzf_run(tdg_ctx *ctx, const uint8_t *d_new, const uint64_t *off, bool finish, const uint8_t **out,
+                    const uint64_t **out_off)
+{
+    namespace bz = tdg::bz;
+    const uint32_t nbar = ctx->sp_nbar;
+    cudaStream_t st = ctx->stream;
+    uint8_t *tails = (uint8_t *)ctx->bz_tail.p;
+    std::vector<bz::Member> mem;
+    std::vector<bz::Copy> cp;
+    std::vector<uint32_t> first(nbar + 1);
+    uint64_t in_total = 0, slot_total = 0;
+    auto add = [&](const uint8_t *s0, uint32_t l0, const uint8_t *s1, uint32_t l1) {
+        bz::Member m;
+        m.src0 = s0;
+        m.len0 = l0;
+        m.src1 = s1;
+        m.len1 = l1;
+        m.in_off = in_total;
+        m.slot = slot_total;
+        in_total += l0 + l1;
+        slot_total += round_up(l0 + l1 + bz::SLOT_EXTRA, 16);
+        mem.push_back(m);
+    };
+    for (uint32_t b = 0; b < nbar; b++) {
+        first[b] = (uint32_t)mem.size();
+        uint8_t *tail = tails + (size_t)b * bz::BLOCK;
+        const uint32_t t = ctx->bz_tail_len[b];
+        if (finish) {
+            if (t) add(tail, t, nullptr, 0);
+            add(nullptr, 0, nullptr, 0);                 // the end-of-file member
+            ctx->bz_tail_len[b] = 0;
+            continue;
+        }
+        const uint64_t L = off[b + 1] - off[b];
+        const uint8_t *src = d_new + off[b];
+        if (t + L < bz::BLOCK) {
+            if (L) cp.push_back(bz::Copy{src, tail + t, L});
+            ctx->bz_tail_len[b] = (uint32_t)(t + L);
+            continue;
+        }
+        add(tail, t, src, bz::BLOCK - t);
+        uint64_t p = bz::BLOCK - t;
+        for (; p + bz::BLOCK <= L; p += bz::BLOCK) add(nullptr, 0, src + p, bz::BLOCK);
+        if (p < L) cp.push_back(bz::Copy{src + p, tail, L - p});
+        ctx->bz_tail_len[b] = (uint32_t)(L - p);
+    }
+    first[nbar] = (uint32_t)mem.size();
+    const uint32_t nm = (uint32_t)mem.size();
+    int rc;
+    if (nm) {
+        if ((rc = grow(ctx, ctx->bz_hmem, nm * sizeof(bz::Member), true))) return rc;
+        if ((rc = grow(ctx, ctx->bz_mem, nm * sizeof(bz::Member), false))) return rc;
+        if ((rc = grow(ctx, ctx->bz_match, in_total * 4 + 16, false))) return rc;
+        if ((rc = grow(ctx, ctx->bz_work, slot_total, false))) return rc;
+        if ((rc = grow(ctx, ctx->bz_out, slot_total, false))) return rc;
+        if ((rc = grow(ctx, ctx->bz_size, (size_t)(nm + 1) * 4, false))) return rc;
+        if ((rc = grow(ctx, ctx->bz_hsize, (size_t)(nm + 1) * 4, true))) return rc;
+        memcpy(ctx->bz_hmem.p, mem.data(), nm * sizeof(bz::Member));
+        CK(cudaMemcpyAsync(ctx->bz_mem.p, ctx->bz_hmem.p, nm * sizeof(bz::Member), cudaMemcpyHostToDevice, st));
+        bz::DeflateArgs a;
+        a.mem = (const bz::Member *)ctx->bz_mem.p;
+        a.n = nm;
+        a.match = (uint32_t *)ctx->bz_match.p;
+        a.work = (uint8_t *)ctx->bz_work.p;
+        a.size = (uint32_t *)ctx->bz_size.p;
+        a.table = (const uint32_t *)((const uint8_t *)ctx->gz_tabs.p + 512);
+        for (int j = 0; j < 8; j++) a.op[j] = ctx->bz_op[j];
+        const bool timed = ctx->timing && ctx->tev_used + 2 <= MAX_TIMED * 2;     // tdg_timing_*: the three as one
+        if (timed) CK(cudaEventRecord(ctx->tev[ctx->tev_used++], st));
+        bz::bgzf_deflate<<<nm, bz::THREADS, sizeof(bz::Shared), st>>>(a);
+        tdg::tile_scan<<<1, 1024, 0, st>>>(a.size, nm);
+        bz::bgzf_pack<<<nm, 256, 0, st>>>(a.mem, a.work, a.size, (uint8_t *)ctx->bz_out.p);
+        if (timed) CK(cudaEventRecord(ctx->tev[ctx->tev_used++], st));
+        ctx->launches += 3;
+    }
+    if (!cp.empty()) {                                   // after the members have read the old tails
+        if ((rc = grow(ctx, ctx->bz_hcopy, cp.size() * sizeof(bz::Copy), true))) return rc;
+        if ((rc = grow(ctx, ctx->bz_copy, cp.size() * sizeof(bz::Copy), false))) return rc;
+        memcpy(ctx->bz_hcopy.p, cp.data(), cp.size() * sizeof(bz::Copy));
+        CK(cudaMemcpyAsync(ctx->bz_copy.p, ctx->bz_hcopy.p, cp.size() * sizeof(bz::Copy), cudaMemcpyHostToDevice, st));
+        bz::bgzf_copy<<<(unsigned)cp.size(), 256, 0, st>>>((const bz::Copy *)ctx->bz_copy.p);
+        ctx->launches += 1;
+    }
+    CK(cudaGetLastError());
+    ctx->bz_off.assign(nbar + 1, 0);
+    if ((rc = grow(ctx, ctx->bz_hout, 16, true))) return rc;
+    if (nm) {
+        const uint32_t *hsize = (const uint32_t *)ctx->bz_hsize.p;
+        CK(cudaMemcpyAsync(ctx->bz_hsize.p, ctx->bz_size.p, (size_t)(nm + 1) * 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        const uint32_t total = hsize[nm];
+        if ((rc = grow(ctx, ctx->bz_hout, (size_t)total + 16, true))) return rc;
+        if (total) CK(cudaMemcpyAsync(ctx->bz_hout.p, ctx->bz_out.p, total, cudaMemcpyDeviceToHost, st));
+        for (uint32_t b = 0; b <= nbar; b++) ctx->bz_off[b] = hsize[first[b]];
+    }
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    *out = (const uint8_t *)ctx->bz_hout.p;
+    *out_off = ctx->bz_off.data();
+    return TDG_OK;
+}
+
+int tdg_split_bgzf(tdg_ctx *ctx, int on)
+{
+    int rc = need_device(ctx);
+    if (rc) return rc;
+    if (!ctx->have_split) return fail(ctx, TDG_ERR_STATE, "tdg_split_begin has not been called");
+    CK(cudaSetDevice(ctx->device));
+    ctx->bz_on = false;
+    if (!on) return TDG_OK;
+    if ((rc = gz_tables(ctx))) return rc;                // the CRC-32 table
+    if ((rc = grow(ctx, ctx->bz_tail, (size_t)ctx->sp_nbar * tdg::bz::BLOCK, false))) return rc;
+    if (!ctx->bz_attr) {
+        CK(cudaFuncSetAttribute(tdg::bz::bgzf_deflate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(tdg::bz::Shared)));
+        for (int j = 0; j < 8; j++) ctx->bz_op[j] = (uint32_t)crc32_combine_gen((z_off_t)(tdg::bz::SEG << j));
+        ctx->bz_attr = true;
+    }
+    ctx->bz_tail_len.assign(ctx->sp_nbar, 0);
+    ctx->bz_on = true;
+    return TDG_OK;
+}
+
+int tdg_bgzf_append(tdg_ctx *ctx, const uint8_t *bytes, const uint64_t *off, const uint8_t **out, const uint64_t **out_off)
+{
+    int rc = need_device(ctx);
+    if (rc) return rc;
+    if (!ctx->have_split || !ctx->bz_on) return fail(ctx, TDG_ERR_STATE, "tdg_split_bgzf has not been called");
+    if (!off || !out || !out_off) return fail(ctx, TDG_ERR_ARG, "null argument");
+    const uint32_t nbar = ctx->sp_nbar;
+    std::vector<uint64_t> rel(nbar + 1);
+    for (uint32_t b = 0; b <= nbar; b++) {
+        if (b && off[b] < off[b - 1]) return fail(ctx, TDG_ERR_ARG, "offsets must be non-decreasing");
+        rel[b] = off[b] - off[0];
+    }
+    const uint64_t n = rel[nbar];
+    if (n && !bytes) return fail(ctx, TDG_ERR_ARG, "null argument");
+    if (n > ((uint64_t)1 << 30)) return fail(ctx, TDG_ERR_ARG, "tdg_bgzf_append: at most 1 GiB per call");
+    CK(cudaSetDevice(ctx->device));
+    if ((rc = grow(ctx, ctx->bz_src, n + 16, false))) return rc;
+    if (n) CK(cudaMemcpyAsync(ctx->bz_src.p, bytes + off[0], n, cudaMemcpyHostToDevice, ctx->stream));
+    return bgzf_run(ctx, (const uint8_t *)ctx->bz_src.p, rel.data(), false, out, out_off);
+}
+
+int tdg_bgzf_finish(tdg_ctx *ctx, const uint8_t **out, const uint64_t **out_off)
+{
+    int rc = need_device(ctx);
+    if (rc) return rc;
+    if (!ctx->have_split || !ctx->bz_on) return fail(ctx, TDG_ERR_STATE, "tdg_split_bgzf has not been called");
+    if (!out || !out_off) return fail(ctx, TDG_ERR_ARG, "null argument");
+    CK(cudaSetDevice(ctx->device));
+    return bgzf_run(ctx, nullptr, nullptr, true, out, out_off);
+}
+
 int tdg_split_begin(tdg_ctx *ctx, const char *barcodes, const uint32_t *bar_off, uint32_t nbar, uint32_t cutlen)
 {
     int rc = need_device(ctx);
@@ -1642,6 +1814,7 @@ int tdg_split_begin(tdg_ctx *ctx, const char *barcodes, const uint32_t *bar_off,
     ctx->sp_nbar = nbar;
     ctx->sp_cutlen = cutlen;
     ctx->have_split = true;
+    ctx->bz_on = false;
     return TDG_OK;
 }
 
@@ -1749,10 +1922,16 @@ int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_bloc
     // ---- the bytes of every barcode's file
     const size_t total_out = (size_t)hbase[nbar];
     if ((rc = grow(ctx, ctx->sp_out, total_out + 16, false))) return rc;
-    if ((rc = grow(ctx, ctx->sp_hout, total_out + 16, true))) return rc;
     w.out = (uint8_t *)ctx->sp_out.p;
     tdg::split_write<<<n_rtiles, tdg::SPLIT_REC_TILE, nbar * sizeof(uint32_t), st>>>(w);
     ctx->launches += 1;
+    if (ctx->bz_on) {                                // the bytes stay on the device and become members
+        CK(cudaMemcpyAsync(ctx->sp_hflags.p, w.flags, nrec, cudaMemcpyDeviceToHost, st));
+        if ((rc = bgzf_run(ctx, w.out, (const uint64_t *)hbase, false, out, out_off))) return rc;
+        *flags = (const uint8_t *)ctx->sp_hflags.p;
+        return TDG_OK;
+    }
+    if ((rc = grow(ctx, ctx->sp_hout, total_out + 16, true))) return rc;
     if (total_out) CK(cudaMemcpyAsync(ctx->sp_hout.p, w.out, total_out, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(ctx->sp_hflags.p, w.flags, nrec, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));

@@ -11,6 +11,11 @@ inflate, csrc/tdg_feed.h), appends the returned pieces to the output files and p
 reference's progress lines.  A block in which some sequence or quality line holds a non-ASCII
 character is handled record by record on the host instead -- str.upper() and character
 indices are Python's there -- with the two decisions still taken on the GPU (``tdg_split_batch``).
+
+With ``bgzf=True`` every output file is BGZF (what bgzip writes) instead of plain text: the bytes of
+both paths go to the device encoder (``tdg_split_bgzf``, csrc/tdg_bgzf.cuh), which cuts each file's
+stream into 65,280-byte members whatever the blocks were, and decompressed each file equals the plain
+one byte for byte.
 """
 
 import csv
@@ -116,13 +121,19 @@ def _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress):
 
 
 def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=hostio.adapters["PstI-MspI-Hall"],
-                    maxreads=500000000, device=None):
+                    maxreads=500000000, device=None, bgzf=False):
     assert set(cutsite) <= hostio.BASES, "Only ACGT cut sites allowed."
     assert all([set(bc) <= hostio.BASES for bc in barcodes]), "Found non-ACGT barcodes."
     assert len(adapter) == 2
     assert all([set(a[0]) <= set("ACGT^") for a in adapter])
     assert set(adapter[0][1]) <= hostio.BASES
     assert set(adapter[1][1]) <= set("[barcode]ACGT")
+    if bgzf:
+        # the counters (counting.py, the reference's find_tags_fastq) take a file for gzip by the last
+        # two characters of its name: a BGZF file under another name would be read as text
+        plain = [name for name in outputFiles if name[-2:].lower() != "gz"]
+        if plain:
+            raise ValueError("BGZF output needs file names ending in 'gz': %s" % ", ".join(plain))
 
     print("Building indices for rapid searching...")
     barlen = [len(bc) for bc in barcodes]
@@ -134,6 +145,8 @@ def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=h
     eng.set_trim(tables[0], tables[1], tables[2], tables[3], tables[4])
     cutlen = len(cutsite)
     eng.split_begin(barcodes, cutlen)
+    if bgzf:
+        eng.split_bgzf(True)
     print("Done with indexing setup.")
     print(inputFile)
 
@@ -148,6 +161,10 @@ def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=h
     cap = 2 * BLOCK_BYTES
     buf = eng.host_alloc(cap)
     pool = ThreadPoolExecutor(max_workers=8)
+
+    def write(pieces):
+        list(pool.map(lambda t: t[0].write(t[1]), [(o, p) for o, p in zip(outcons, pieces) if len(p)]))
+
     try:
         fill, eof = 0, False
         while left > 0:
@@ -167,14 +184,21 @@ def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=h
                 continue
             if needs_host:
                 text = ctypes.string_at(buf, used).decode("utf-8")
-                _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress)
+                if bgzf:
+                    parts = [io.BytesIO() for _ in outcons]
+                    _host_records(eng, text, barcodes, barlen, cutlen, parts, progress)
+                    write(eng.bgzf_append([p.getvalue() for p in parts]))
+                else:
+                    _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress)
             else:
-                list(pool.map(lambda t: t[0].write(t[1]), [(o, p) for o, p in zip(outcons, pieces) if len(p)]))
+                write(pieces)
                 progress.many(flags)
             left -= nrec
             fill -= used
             if fill:
                 ctypes.memmove(buf, buf + used, fill)
+        if bgzf:
+            write(eng.bgzf_finish())
     except _native.TdgError as e:
         if e.code == _native.TDG_ERR_GZIP:
             raise _gzip_exception(e.message)
