@@ -174,7 +174,8 @@ int         tdg_count_file2(tdg_ctx *ctx, const char *path, int gz, uint64_t rea
 int         tdg_last_file_info(tdg_ctx *ctx, int64_t info[3]);
 
 /* Frees the working buffers of the device-side gzip feed (tokens, symbols, windows, text: about ten
- * times the compressed bytes of a round, at most ~12 GB); they are kept between files otherwise. */
+ * times the compressed bytes of a round, at most ~12 GB) and the staging buffer of tdg_trim_batch,
+ * tdg_split_batch and tdg_match_batch; they are kept between calls otherwise. */
 int         tdg_release_scratch(tdg_ctx *ctx);
 
 /* The gzip feed of tdg_count_file by itself (tests, profiling): inflates `path` into the host

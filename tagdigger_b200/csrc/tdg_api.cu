@@ -38,12 +38,56 @@ constexpr int NSLOT = 3;
 constexpr int MAX_TIMED = 4096;
 std::string g_create_error;
 
+// A device or pinned buffer of the context.  Allocated by reserve() (below), freed by its destructor.
+struct Buf {
+    void *p = nullptr;
+    size_t cap = 0;
+    bool host = false;
+
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    Buf(Buf &&o) noexcept : p(o.p), cap(o.cap), host(o.host) { o.p = nullptr, o.cap = 0; }
+    Buf &operator=(Buf &&o) noexcept
+    {
+        if (this != &o) {
+            reset();
+            p = o.p, cap = o.cap, host = o.host;
+            o.p = nullptr, o.cap = 0;
+        }
+        return *this;
+    }
+    ~Buf() { reset(); }
+    void reset()
+    {
+        if (p) {
+            if (host) cudaFreeHost(p); else cudaFree(p);
+        }
+        p = nullptr;
+        cap = 0;
+    }
+};
+
+// An event of the context.  Created on first use by make_event() (below), destroyed by its destructor.
+struct Event {
+    cudaEvent_t e = nullptr;
+
+    Event() = default;
+    Event(const Event &) = delete;
+    Event &operator=(const Event &) = delete;
+    Event(Event &&o) noexcept : e(o.e) { o.e = nullptr; }
+    ~Event()
+    {
+        if (e) cudaEventDestroy(e);
+    }
+    operator cudaEvent_t() const { return e; }
+};
+
 struct Slot {
-    uint8_t *dev = nullptr;
-    uint8_t *carry = nullptr;      // pinned: partial last line of the previous piece
-    size_t carry_cap = 0;
-    cudaEvent_t copied = nullptr;  // H2D of this slot finished
-    cudaEvent_t done = nullptr;    // kernel on this slot finished
+    Buf dev;
+    Buf carry;       // pinned: partial last line of the previous piece
+    Event copied;    // H2D of this slot finished
+    Event done;      // kernel on this slot finished
 };
 
 }  // namespace
@@ -59,6 +103,15 @@ struct GzHandover {
     std::vector<uint8_t> window;
     std::string why;
 };
+
+// The host feeder of `path`: from the start, or where the device gzip feed handed over (ho->active)
+static int open_feed(tdg::Feeder &feed, const char *path, bool gz, const GzHandover *ho)
+{
+    if (!ho || !ho->active) return feed.open(path, gz);
+    if (ho->bgzf) return feed.open_resume_bgzf(path, ho->bgzf_off, ho->delivered);
+    return feed.open_resume(path, ho->pos_bit, ho->to_zlib ? nullptr : ho->window.data(), ho->hist, ho->crc, ho->member_len,
+                            ho->delivered);
+}
 
 // The host side of tdg_count_file for one file: a thread that reads (or inflates) the file through
 // tdg_feed.h into three pinned buffers, one ahead of the other.  It can be started BEFORE its
@@ -89,11 +142,7 @@ struct FileReader {
         th = std::thread([this]() {
             // host feed: parallel pread / parallel BGZF inflate / zlib, see tdg_feed.h
             tdg::Feeder feed;
-            const char *p = path.c_str();
-            int orc = !ho.active ? feed.open(p, gz)
-                      : ho.bgzf  ? feed.open_resume_bgzf(p, ho.bgzf_off, ho.delivered)
-                                 : feed.open_resume(p, ho.pos_bit, ho.to_zlib ? nullptr : ho.window.data(), ho.hist, ho.crc, ho.member_len,
-                                                    ho.delivered);
+            int orc = open_feed(feed, path.c_str(), gz, &ho);
             int bi = 0;
             for (;;) {
                 Buf &b = bufs[bi];
@@ -143,86 +192,76 @@ struct tdg_ctx {
 
     cudaStream_t stream = nullptr;       // kernels
     cudaStream_t copy_stream = nullptr;  // H2D
-    cudaEvent_t handoff = nullptr;       // tdg_stream_wait / tdg_other_stream_wait
+    Event handoff;                       // tdg_stream_wait / tdg_other_stream_wait
 
     // tables
     tdg::HostTagTable tags;
     bool have_tags = false;
-    tdg::TagEntry *d_entries = nullptr;
-    uint64_t *d_ext = nullptr;
-    size_t d_entries_cap = 0, d_ext_cap = 0;
+    Buf d_entries, d_ext;                // TagEntry[], uint64_t[]
     std::vector<uint8_t> bar_blob;
     bool have_bar = false;
-    uint8_t *d_bar = nullptr;
-    size_t d_bar_cap = 0;
+    Buf d_bar;
 
-    // matrix
+    // matrix: the context's own (tdg_set_matrix) or the caller's (tdg_bind_matrix)
     int32_t *d_matrix = nullptr;
-    bool own_matrix = false;
+    Buf matrix;
     uint32_t rows = 0, cols = 0;
     uint32_t max_row = 0, max_col = 0;   // largest indices the loaded tables refer to
     // extra zero-initialised copies of a small matrix (see ChunkArgs::replicas); always all-zero between launches
-    int32_t *d_replicas = nullptr;
+    Buf d_replicas;
     uint32_t n_replicas = 1;
-    size_t replicas_cap = 0;             // int32 elements allocated
 
     // per-launch scratch (ScratchHeader, SegInfo[], FixEntry[])
-    unsigned long long *d_sync = nullptr;
-    size_t sync_cap = 0;          // in 8-byte words
+    Buf d_sync;
     int occ[3] = {0, 0, 0};              // resident CTAs per SM of the three kernel instantiations, at
     size_t occ_smem[3] = {0, 0, 0};      //   this much dynamic shared memory
     uint32_t force_seg_tiles = 0; // test hook (TDG_SEG_TILES)
     bool force_general = false;   // test hook (TDG_GENERAL=1): never use the fast matcher
-    tdg::LineState *d_state = nullptr;   // [2]
+    Buf d_state;                  // LineState[2]
     int state_cur = 0;
-    unsigned long long *d_totals = nullptr;   // [4]
+    Buf d_totals;                 // unsigned long long[4]
 
     // streaming
     Slot slot[NSLOT];
-    size_t slot_cap = 0;
+    bool have_slots = false;
     int next_slot = 0;
     size_t carry_len = 0;        // bytes waiting in slot[next_slot].carry
     bool file_open = false;
 
     // trim decision tables (tdg_set_trim): one device blob
-    uint8_t *d_trim = nullptr;
-    size_t d_trim_cap = 0;
+    Buf d_trim;
     tdg::TrimArgs trim;          // device pointers into d_trim
     uint32_t trim_nbar = 0;
     bool have_trim = false;
 
+    // staging of tdg_trim_batch, tdg_split_batch and tdg_match_batch
+    Buf batch;
+
     // streaming splitter (tdg_split_begin / tdg_split_block): growable device and pinned buffers
-    struct Grow {
-        void *p = nullptr;
-        size_t cap = 0;
-        bool host = false;
-    };
-    Grow sp_in, sp_tiles, sp_ends, sp_rec, sp_flags, sp_sums, sp_base, sp_out, sp_tabs;      // device
-    Grow sp_hout, sp_hflags, sp_hbase;                                                          // pinned host
+    Buf sp_in, sp_tiles, sp_ends, sp_rec, sp_flags, sp_sums, sp_base, sp_out, sp_tabs;      // device
+    Buf sp_hout, sp_hflags, sp_hbase;                                                          // pinned host
     uint32_t sp_nbar = 0, sp_cutlen = 0;
     bool have_split = false;
 
     // BGZF output of the splitter (tdg_split_bgzf, tdg_bgzf.cuh): every barcode's pending tail
     // (< 65,280 bytes) waits in bz_tail between calls
     bool bz_on = false, bz_attr = false;
-    Grow bz_tail, bz_src, bz_mem, bz_copy, bz_match, bz_work, bz_size, bz_out;      // device
-    Grow bz_hmem, bz_hcopy, bz_hsize, bz_hout;                                     // pinned host
+    Buf bz_tail, bz_src, bz_mem, bz_copy, bz_match, bz_work, bz_size, bz_out;      // device
+    Buf bz_hmem, bz_hcopy, bz_hsize, bz_hout;                                     // pinned host
     std::vector<uint32_t> bz_tail_len;
     std::vector<uint64_t> bz_off;
     uint32_t bz_op[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 
-    // pinned buffers of tdg_count_file (kept between files: pinning 192 MiB costs ~0.1 s)
-    uint8_t *file_buf[3] = {nullptr, nullptr, nullptr};
-    size_t file_buf_cap = 0;
-    uint8_t *file_buf2[3] = {nullptr, nullptr, nullptr};     // a second set: the reader that runs ahead for the next file
-    size_t file_buf2_cap = 0;
+    // pinned buffers of tdg_count_file (kept between files: pinning 192 MiB costs ~0.1 s), chunk_bytes each;
+    // set 1 is for the reader that runs ahead for the next file
+    Buf file_buf[2][FileReader::NBUF];
     std::unique_ptr<FileReader> ahead;                        // started by tdg_count_file2's next_path
 
     // device-side gzip feed (tdg_gzdev.cuh): growable buffers, kept between files
-    Grow gz_comp, gz_comp2, gz_syms, gz_sym2, gz_ntok, gz_meta, gz_cand, gz_ncand, gz_windows, gz_text, gz_crc, gz_lens, gz_offs, gz_tabs, gz_carry, gz_cold;   // device
-    Grow gz_hmeta, gz_hcrc, gz_htail;                                                                                       // pinned host
-    cudaEvent_t gz_up[3] = {nullptr, nullptr, nullptr};
-    cudaEvent_t gz_pre = nullptr;
+    Buf gz_comp, gz_comp2, gz_syms, gz_sym2, gz_ntok, gz_meta, gz_cand, gz_ncand, gz_windows, gz_text, gz_crc, gz_lens, gz_offs, gz_tabs, gz_carry, gz_cold;   // device
+    Buf gz_hmeta, gz_hcrc, gz_htail;                                                                                       // pinned host
+    Event gz_up[3];
+    Event gz_pre;
     int64_t last_file[3] = {0, 0, 0};    // tdg_count_file: device gzip rounds, chunks accepted, 0 all on the device / 1 host feeder took over / -1 host feeder only
     bool gz_tables = false;
     uint32_t gz_op[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -234,8 +273,11 @@ struct tdg_ctx {
     // accounting
     uint64_t launches = 0;
     bool timing = false;
-    std::vector<cudaEvent_t> tev;
+    std::vector<Event> tev;      // 2 * MAX_TIMED
     int tev_used = 0;
+
+    // test hook (TDG_FAIL_ALLOC=k): the k-th buffer allocation or event creation after tdg_create fails
+    uint64_t fail_at = 0, allocs = 0;
 };
 
 namespace {
@@ -255,24 +297,39 @@ int fail(tdg_ctx *ctx, int code, const std::string &msg)
 
 size_t round_up(size_t x, size_t m) { return (x + m - 1) / m * m; }
 
-// growable device / pinned buffers (contents are NOT kept)
-int grow(tdg_ctx *ctx, tdg_ctx::Grow &g, size_t need, bool host)
+bool simulated_failure(tdg_ctx *ctx) { return ctx->fail_at && ++ctx->allocs == ctx->fail_at; }
+
+// Every buffer of the context comes from here: when b holds fewer than `need` bytes, it is replaced by
+// a buffer of `cap` bytes (contents are NOT kept).  The old buffer is freed only once the new one is
+// had, so it stays whole when the allocation fails.
+int reserve(tdg_ctx *ctx, Buf &b, size_t need, size_t cap, bool host)
 {
-    if (need <= g.cap) return TDG_OK;
+    if (need <= b.cap) return TDG_OK;
     CK(cudaStreamSynchronize(ctx->stream));
-    const size_t cap = need + need / 4 + 4096;
     void *fresh = nullptr;
-    cudaError_t e = host ? cudaHostAlloc(&fresh, cap, cudaHostAllocDefault) : cudaMalloc(&fresh, cap);
+    const bool sim = simulated_failure(ctx);
+    cudaError_t e = sim ? cudaErrorMemoryAllocation : host ? cudaHostAlloc(&fresh, cap, cudaHostAllocDefault) : cudaMalloc(&fresh, cap);
     if (e != cudaSuccess) {
         cudaGetLastError();                                  // (the failed allocation must not show up as the next launch's error)
-        return fail(ctx, TDG_ERR_NOMEM, std::string("buffer of ") + std::to_string(cap) + " bytes: " + cudaGetErrorString(e));
+        return fail(ctx, TDG_ERR_NOMEM, std::string("buffer of ") + std::to_string(cap) + " bytes: " +
+                                            (sim ? "simulated (TDG_FAIL_ALLOC)" : cudaGetErrorString(e)));
     }
-    if (g.p) {
-        if (g.host) cudaFreeHost(g.p); else cudaFree(g.p);   // (the old buffer stays whole when the new one cannot be had)
-    }
-    g.p = fresh;
-    g.cap = cap;
-    g.host = host;
+    b.reset();
+    b.p = fresh;
+    b.cap = cap;
+    b.host = host;
+    return TDG_OK;
+}
+
+// growable buffers: a quarter more than asked for
+int grow(tdg_ctx *ctx, Buf &b, size_t need, bool host) { return reserve(ctx, b, need, need + need / 4 + 4096, host); }
+int grow_exact(tdg_ctx *ctx, Buf &b, size_t need, bool host) { return reserve(ctx, b, need, need, host); }
+
+int make_event(tdg_ctx *ctx, Event &ev, unsigned flags = cudaEventDisableTiming)
+{
+    if (ev.e) return TDG_OK;
+    if (simulated_failure(ctx)) return fail(ctx, TDG_ERR_NOMEM, "event: simulated (TDG_FAIL_ALLOC)");
+    CK(cudaEventCreateWithFlags(&ev.e, flags));
     return TDG_OK;
 }
 
@@ -288,14 +345,20 @@ static_assert(sizeof(ScratchHeader::run_total) / 8 == tdg::VERIFY_MAX_CTAS * (td
 
 int ensure_sync(tdg_ctx *ctx, size_t segs)
 {
-    size_t need = (sizeof(ScratchHeader) + segs * (sizeof(tdg::SegInfo) + sizeof(tdg::FixEntry)) + 7) / 8;
-    if (need <= ctx->sync_cap) return TDG_OK;
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (ctx->d_sync) CK(cudaFree(ctx->d_sync));
-    ctx->d_sync = nullptr;
-    size_t cap = need + need / 2;
-    CK(cudaMalloc(&ctx->d_sync, cap * sizeof(unsigned long long)));
-    ctx->sync_cap = cap;
+    size_t need = (sizeof(ScratchHeader) + segs * (sizeof(tdg::SegInfo) + sizeof(tdg::FixEntry)) + 7) / 8;     // 8-byte words
+    return reserve(ctx, ctx->d_sync, need * 8, (need + need / 2) * 8, false);
+}
+
+// tdg_timing_begin: a pair of events around the launches of one call, on ctx->stream.  Both are created
+// (on first use) before the first is recorded; the caller records the second behind its launches.
+int timed_start(tdg_ctx *ctx, bool &timed)
+{
+    timed = ctx->timing && ctx->tev_used + 2 <= MAX_TIMED * 2;
+    if (!timed) return TDG_OK;
+    int rc;
+    if ((rc = make_event(ctx, ctx->tev[ctx->tev_used], cudaEventDefault)) || (rc = make_event(ctx, ctx->tev[ctx->tev_used + 1], cudaEventDefault)))
+        return rc;
+    CK(cudaEventRecord(ctx->tev[ctx->tev_used++], ctx->stream));
     return TDG_OK;
 }
 
@@ -365,7 +428,7 @@ int launch_chunk(tdg_ctx *ctx, const void *dev_bytes, size_t n, uint64_t line_ba
 
     int rc = ensure_sync(ctx, segs);
     if (rc) return rc;
-    ScratchHeader *hdr = (ScratchHeader *)ctx->d_sync;
+    ScratchHeader *hdr = (ScratchHeader *)ctx->d_sync.p;
     SegInfo *seginfo = (SegInfo *)(hdr + 1);
     FixEntry *fix = (FixEntry *)(seginfo + segs);
     CK(cudaMemsetAsync(hdr, 0, offsetof(ScratchHeader, run_total), ctx->stream));
@@ -389,8 +452,9 @@ int launch_chunk(tdg_ctx *ctx, const void *dev_bytes, size_t n, uint64_t line_ba
         a.line_base = v.line_base = line_base;
         a.prev_kind = v.prev_kind = (uint32_t)prev_kind;
     }
-    a.state_in = v.state_in = ctx->d_state + ctx->state_cur;
-    v.state_out = ctx->d_state + (ctx->state_cur ^ 1);
+    LineState *state = (LineState *)ctx->d_state.p;
+    a.state_in = v.state_in = state + ctx->state_cur;
+    v.state_out = state + (ctx->state_cur ^ 1);
     ctx->state_cur ^= 1;
     a.ticket = &hdr->ticket_main;
     a.seginfo = seginfo;
@@ -422,18 +486,18 @@ int launch_chunk(tdg_ctx *ctx, const void *dev_bytes, size_t n, uint64_t line_ba
                 }
             }
         }
-        a.bar = (const BarTable *)ctx->d_bar;
+        a.bar = (const BarTable *)ctx->d_bar.p;
         a.bar_bytes = (uint32_t)ctx->bar_blob.size();
         a.bar_in_smem = bar_smem != 0;
         a.cols = ctx->cols;
         a.tags = ctx->tags.t;
-        a.tags.entries = ctx->d_entries;
-        a.tags.ext = ctx->d_ext;
+        a.tags.entries = (const TagEntry *)ctx->d_entries.p;
+        a.tags.ext = (const uint64_t *)ctx->d_ext.p;
         a.matrix = ctx->d_matrix;
-        a.replicas = ctx->d_replicas;
+        a.replicas = (int32_t *)ctx->d_replicas.p;
         a.n_replicas = ctx->n_replicas;
         a.cells = ctx->rows * ctx->cols;
-        a.totals = ctx->d_totals;
+        a.totals = (unsigned long long *)ctx->d_totals.p;
     }
     v.num_segs = (uint32_t)segs;
     v.make_fixes = MATCH ? 1 : 0;
@@ -444,8 +508,8 @@ int launch_chunk(tdg_ctx *ctx, const void *dev_bytes, size_t n, uint64_t line_ba
     v.n_fix = &hdr->n_fix;
     v.run_total = hdr->run_total;
 
-    bool timed = ctx->timing && ctx->tev_used + 2 <= MAX_TIMED * 2;
-    if (timed) CK(cudaEventRecord(ctx->tev[ctx->tev_used++], ctx->stream));
+    bool timed;
+    if ((rc = timed_start(ctx, timed))) return rc;
     kern<<<(unsigned)grid, THREADS, smem, ctx->stream>>>(a);
     CK(cudaGetLastError());
     // every warp of the verify launches takes >= 256 segments
@@ -465,7 +529,7 @@ int launch_chunk(tdg_ctx *ctx, const void *dev_bytes, size_t n, uint64_t line_ba
         ctx->launches += 1;
         if (ctx->n_replicas > 1) {
             unsigned fold_grid = (unsigned)std::min<size_t>(((size_t)a.cells + 255) / 256, (size_t)ctx->sm_count * 8);
-            fold_kernel<<<fold_grid, 256, 0, ctx->stream>>>(ctx->d_matrix, ctx->d_replicas, a.cells, ctx->n_replicas - 1);
+            fold_kernel<<<fold_grid, 256, 0, ctx->stream>>>(ctx->d_matrix, a.replicas, a.cells, ctx->n_replicas - 1);
             CK(cudaGetLastError());
             ctx->launches += 1;
         }
@@ -486,15 +550,10 @@ int size_replicas(tdg_ctx *ctx)
     if (const char *e = getenv("TDG_REPLICAS")) want = (uint32_t)std::max(1, atoi(e));
     ctx->n_replicas = 1;
     if (want > 1) {
-        size_t need = (size_t)(want - 1) * cells;
-        if (need > ctx->replicas_cap) {
-            if (ctx->d_replicas) CK(cudaFree(ctx->d_replicas));
-            ctx->d_replicas = nullptr;
-            ctx->replicas_cap = 0;
-            CK(cudaMalloc(&ctx->d_replicas, need * sizeof(int32_t)));
-            ctx->replicas_cap = need;
-        }
-        CK(cudaMemsetAsync(ctx->d_replicas, 0, need * sizeof(int32_t), ctx->stream));
+        size_t need = (size_t)(want - 1) * cells * sizeof(int32_t);
+        int rc = grow_exact(ctx, ctx->d_replicas, need, false);
+        if (rc) return rc;
+        CK(cudaMemsetAsync(ctx->d_replicas.p, 0, need, ctx->stream));
         ctx->n_replicas = want;
     }
     return TDG_OK;
@@ -520,31 +579,30 @@ int need_ready(tdg_ctx *ctx)
 
 int ensure_slots(tdg_ctx *ctx)
 {
-    if (ctx->slot_cap) return TDG_OK;
+    if (ctx->have_slots) return TDG_OK;
     // a piece is the carried partial line (<= chunk_bytes) plus up to chunk_bytes new bytes
     size_t cap = round_up(2 * ctx->chunk_bytes, TDG_TILE_BYTES) + TDG_TILE_BYTES + TDG_HALO_BYTES;
-    for (int i = 0; i < NSLOT; i++) {
-        CK(cudaMalloc(&ctx->slot[i].dev, cap));
-        ctx->slot[i].carry_cap = 1 << 20;
-        CK(cudaHostAlloc(&ctx->slot[i].carry, ctx->slot[i].carry_cap, cudaHostAllocDefault));
-        CK(cudaEventCreateWithFlags(&ctx->slot[i].copied, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ctx->slot[i].done, cudaEventDisableTiming));
+    for (Slot &s : ctx->slot) {
+        int rc;
+        if ((rc = grow_exact(ctx, s.dev, cap, false)) || (rc = grow_exact(ctx, s.carry, 1 << 20, true)) ||
+            (rc = make_event(ctx, s.copied)) || (rc = make_event(ctx, s.done)))
+            return rc;
     }
-    ctx->slot_cap = cap;
+    ctx->have_slots = true;
     return TDG_OK;
 }
 
-int grow_carry(tdg_ctx *ctx, Slot &s, size_t need, size_t keep)
+// a slot's carry doubles until it holds `need` bytes, and keeps its first `keep`
+int grow_carry(tdg_ctx *ctx, Buf &carry, size_t need, size_t keep)
 {
-    if (need <= s.carry_cap) return TDG_OK;
-    size_t cap = s.carry_cap;
+    if (need <= carry.cap) return TDG_OK;
+    size_t cap = carry.cap;
     while (cap < need) cap *= 2;
-    uint8_t *p = nullptr;
-    CK(cudaHostAlloc(&p, cap, cudaHostAllocDefault));
-    if (keep) memcpy(p, s.carry, keep);
-    CK(cudaFreeHost(s.carry));
-    s.carry = p;
-    s.carry_cap = cap;
+    Buf fresh;
+    int rc = grow_exact(ctx, fresh, cap, true);
+    if (rc) return rc;
+    if (keep) memcpy(fresh.p, carry.p, keep);
+    carry = std::move(fresh);
     return TDG_OK;
 }
 
@@ -580,19 +638,20 @@ int submit_piece(tdg_ctx *ctx, const uint8_t *bytes, size_t n, size_t cut, uint6
     if (cut > 0) {      // the piece holds a line end: carried bytes + everything up to the cut form whole lines
         // the slot's previous kernel must be finished before its buffer is overwritten
         CK(cudaStreamWaitEvent(ctx->copy_stream, s.done, 0));
-        if (ctx->carry_len) CK(cudaMemcpyAsync(s.dev, s.carry, ctx->carry_len, cudaMemcpyHostToDevice, ctx->copy_stream));
-        if (cut) CK(cudaMemcpyAsync(s.dev + ctx->carry_len, bytes, cut, cudaMemcpyHostToDevice, ctx->copy_stream));
+        uint8_t *dev = (uint8_t *)s.dev.p;
+        if (ctx->carry_len) CK(cudaMemcpyAsync(dev, s.carry.p, ctx->carry_len, cudaMemcpyHostToDevice, ctx->copy_stream));
+        if (cut) CK(cudaMemcpyAsync(dev + ctx->carry_len, bytes, cut, cudaMemcpyHostToDevice, ctx->copy_stream));
         CK(cudaEventRecord(s.copied, ctx->copy_stream));
         CK(cudaStreamWaitEvent(ctx->stream, s.copied, 0));
-        int rc = launch_chunk<true>(ctx, s.dev, total, TDG_LINE_CHAINED, 0, reads_limit);
+        int rc = launch_chunk<true>(ctx, dev, total, TDG_LINE_CHAINED, 0, reads_limit);
         if (rc) return rc;
         CK(cudaEventRecord(s.done, ctx->stream));
         // new carry goes to the next slot's pinned buffer, once its last H2D has drained
         CK(cudaEventSynchronize(sn.copied));
         size_t rest = n - cut;
-        int rc2 = grow_carry(ctx, sn, rest, 0);
+        int rc2 = grow_carry(ctx, sn.carry, rest, 0);
         if (rc2) return rc2;
-        if (rest) memcpy(sn.carry, bytes + cut, rest);
+        if (rest) memcpy(sn.carry.p, bytes + cut, rest);
         ctx->carry_len = rest;
         ctx->next_slot = nxt;
     } else {
@@ -600,9 +659,9 @@ int submit_piece(tdg_ctx *ctx, const uint8_t *bytes, size_t n, size_t cut, uint6
         size_t rest = n;
         if (ctx->carry_len + rest > ctx->chunk_bytes)
             return fail(ctx, TDG_ERR_ARG, "a single text line is longer than chunk_bytes");
-        int rc2 = grow_carry(ctx, s, ctx->carry_len + rest, ctx->carry_len);
+        int rc2 = grow_carry(ctx, s.carry, ctx->carry_len + rest, ctx->carry_len);
         if (rc2) return rc2;
-        memcpy(s.carry + ctx->carry_len, bytes, rest);
+        memcpy((uint8_t *)s.carry.p + ctx->carry_len, bytes, rest);
         ctx->carry_len += rest;
     }
     return TDG_OK;
@@ -642,10 +701,10 @@ int end_file_impl(tdg_ctx *ctx, uint64_t reads_limit)
         int si = ctx->next_slot;
         Slot &s = ctx->slot[si];
         CK(cudaStreamWaitEvent(ctx->copy_stream, s.done, 0));
-        CK(cudaMemcpyAsync(s.dev, s.carry, ctx->carry_len, cudaMemcpyHostToDevice, ctx->copy_stream));
+        CK(cudaMemcpyAsync(s.dev.p, s.carry.p, ctx->carry_len, cudaMemcpyHostToDevice, ctx->copy_stream));
         CK(cudaEventRecord(s.copied, ctx->copy_stream));
         CK(cudaStreamWaitEvent(ctx->stream, s.copied, 0));
-        int rc = launch_chunk<true>(ctx, s.dev, ctx->carry_len, TDG_LINE_CHAINED, 0, reads_limit);
+        int rc = launch_chunk<true>(ctx, s.dev.p, ctx->carry_len, TDG_LINE_CHAINED, 0, reads_limit);
         if (rc) return rc;
         CK(cudaEventRecord(s.done, ctx->stream));
         CK(cudaEventSynchronize(s.copied));
@@ -655,6 +714,53 @@ int end_file_impl(tdg_ctx *ctx, uint64_t reads_limit)
     return TDG_OK;
 }
 
+// One array of a batch call: copied from `in` before the kernel, or to `out` after it
+struct BatchPart {
+    const void *in;
+    void *out;
+    size_t bytes;
+};
+
+// The batch calls (tdg_trim_batch, tdg_split_batch, tdg_match_batch) stage the reads' bytes, their
+// offsets from the first read and `parts` in one device buffer the context keeps, each part 16-byte
+// aligned.  launch(seqs, off, part) enqueues the kernel on those device addresses; then the output
+// parts come back and the stream is synchronised.  Errors are reported as "<what>: ...".
+template <class Launch>
+int batch_run(tdg_ctx *ctx, const char *what, const char *seqs, const uint64_t *off, uint32_t n, std::initializer_list<BatchPart> parts,
+              Launch launch)
+{
+    const size_t nbytes = (size_t)(off[n] - off[0]);
+    std::vector<unsigned long long> rel(n + 1);
+    for (uint32_t i = 0; i <= n; i++) rel[i] = off[i] - off[0];
+    const size_t o_off = round_up(nbytes + 16, 16);
+    size_t total = o_off + round_up((n + 1) * sizeof(uint64_t), 16);
+    std::vector<size_t> at;
+    for (const BatchPart &p : parts) {
+        at.push_back(total);
+        total += round_up(p.bytes, 16);
+    }
+    if (int rc = grow(ctx, ctx->batch, total, false)) return fail(ctx, rc, std::string(what) + ": " + ctx->err);
+    uint8_t *d = (uint8_t *)ctx->batch.p;
+    std::vector<uint8_t *> dev;
+    for (size_t a : at) dev.push_back(d + a);
+    const BatchPart *part = parts.begin();
+    cudaError_t e = cudaSuccess;
+    if (nbytes) e = cudaMemcpyAsync(d, seqs + off[0], nbytes, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_off, rel.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream);
+    for (size_t k = 0; k < parts.size() && e == cudaSuccess; k++)
+        if (part[k].in) e = cudaMemcpyAsync(dev[k], part[k].in, part[k].bytes, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) {
+        launch(d, (const unsigned long long *)(d + o_off), dev.data());
+        e = cudaGetLastError();
+        ctx->launches += 1;
+    }
+    for (size_t k = 0; k < parts.size() && e == cudaSuccess; k++)
+        if (part[k].out) e = cudaMemcpyAsync(part[k].out, dev[k], part[k].bytes, cudaMemcpyDeviceToHost, ctx->stream);
+    cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
+    if (e2 != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e2));
+    return TDG_OK;
+}
 
 #include "tdg_gzfeed.cuh"      // the host side of the device gzip feed (part of this unit)
 
@@ -697,18 +803,21 @@ int tdg_create(tdg_ctx **out, int device, size_t chunk_bytes)
     if (const char *e = getenv("TDG_SEG_TILES")) c->force_seg_tiles = (uint32_t)atoi(e);
     if (const char *e = getenv("TDG_GENERAL")) c->force_general = atoi(e) != 0;
     if (c->chunk_bytes < 4096) c->chunk_bytes = 4096;
-    cudaError_t e2 = cudaSuccess;
-    if (e2 == cudaSuccess) e2 = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
+    std::string why;
+    cudaError_t e2 = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
     if (e2 == cudaSuccess) e2 = cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking);
-    if (e2 == cudaSuccess) e2 = cudaMalloc(&c->d_state, 2 * sizeof(tdg::LineState));
-    if (e2 == cudaSuccess) e2 = cudaMalloc(&c->d_totals, 4 * sizeof(unsigned long long));
-    if (e2 == cudaSuccess) e2 = cudaMemset(c->d_state, 0, 2 * sizeof(tdg::LineState));
-    if (e2 == cudaSuccess) e2 = cudaMemset(c->d_totals, 0, 4 * sizeof(unsigned long long));
-    if (e2 != cudaSuccess) {
-        std::string msg = std::string("context set-up failed: ") + cudaGetErrorString(e2);
+    if (e2 != cudaSuccess)
+        why = cudaGetErrorString(e2);
+    else if (grow_exact(c, c->d_state, 2 * sizeof(tdg::LineState), false) || grow_exact(c, c->d_totals, 4 * sizeof(unsigned long long), false))
+        why = c->err;
+    else if ((e2 = cudaMemset(c->d_state.p, 0, 2 * sizeof(tdg::LineState))) != cudaSuccess ||
+             (e2 = cudaMemset(c->d_totals.p, 0, 4 * sizeof(unsigned long long))) != cudaSuccess)
+        why = cudaGetErrorString(e2);
+    if (!why.empty()) {
         tdg_destroy(c);
-        return fail(nullptr, TDG_ERR_CUDA, msg);
+        return fail(nullptr, TDG_ERR_CUDA, "context set-up failed: " + why);
     }
+    if (const char *e = getenv("TDG_FAIL_ALLOC")) c->fail_at = strtoull(e, nullptr, 10);
     *out = c;
     return TDG_OK;
 }
@@ -716,54 +825,15 @@ int tdg_create(tdg_ctx **out, int device, size_t chunk_bytes)
 void tdg_destroy(tdg_ctx *ctx)
 {
     if (!ctx) return;
-    {
-        cudaSetDevice(ctx->device);
-        if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-        if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
-        for (int i = 0; i < NSLOT; i++) {
-            if (ctx->slot[i].dev) cudaFree(ctx->slot[i].dev);
-            if (ctx->slot[i].carry) cudaFreeHost(ctx->slot[i].carry);
-            if (ctx->slot[i].copied) cudaEventDestroy(ctx->slot[i].copied);
-            if (ctx->slot[i].done) cudaEventDestroy(ctx->slot[i].done);
-        }
-        for (cudaEvent_t ev : ctx->tev) cudaEventDestroy(ev);
-        if (ctx->handoff) cudaEventDestroy(ctx->handoff);
-        if (ctx->comm && tdg::nccl().CommDestroy) tdg::nccl().CommDestroy(ctx->comm);
-        if (ctx->d_entries) cudaFree(ctx->d_entries);
-        if (ctx->d_ext) cudaFree(ctx->d_ext);
-        if (ctx->d_bar) cudaFree(ctx->d_bar);
-        if (ctx->own_matrix && ctx->d_matrix) cudaFree(ctx->d_matrix);
-        if (ctx->d_sync) cudaFree(ctx->d_sync);
-        if (ctx->d_state) cudaFree(ctx->d_state);
-        if (ctx->d_totals) cudaFree(ctx->d_totals);
-        if (ctx->d_trim) cudaFree(ctx->d_trim);
-        for (tdg_ctx::Grow *g : {&ctx->sp_in, &ctx->sp_tiles, &ctx->sp_ends, &ctx->sp_rec, &ctx->sp_flags, &ctx->sp_sums,
-                                 &ctx->sp_base, &ctx->sp_out, &ctx->sp_tabs})
-            if (g->p) cudaFree(g->p);
-        for (tdg_ctx::Grow *g : {&ctx->sp_hout, &ctx->sp_hflags, &ctx->sp_hbase})
-            if (g->p) cudaFreeHost(g->p);
-        for (tdg_ctx::Grow *g : {&ctx->bz_tail, &ctx->bz_src, &ctx->bz_mem, &ctx->bz_copy, &ctx->bz_match, &ctx->bz_work, &ctx->bz_size, &ctx->bz_out})
-            if (g->p) cudaFree(g->p);
-        for (tdg_ctx::Grow *g : {&ctx->bz_hmem, &ctx->bz_hcopy, &ctx->bz_hsize, &ctx->bz_hout})
-            if (g->p) cudaFreeHost(g->p);
-        for (tdg_ctx::Grow *g : {&ctx->gz_comp, &ctx->gz_comp2, &ctx->gz_syms, &ctx->gz_sym2, &ctx->gz_ntok, &ctx->gz_meta, &ctx->gz_cand, &ctx->gz_ncand, &ctx->gz_windows,
-                                 &ctx->gz_text, &ctx->gz_crc, &ctx->gz_lens, &ctx->gz_offs, &ctx->gz_tabs, &ctx->gz_carry, &ctx->gz_cold})
-            if (g->p) cudaFree(g->p);
-        for (tdg_ctx::Grow *g : {&ctx->gz_hmeta, &ctx->gz_hcrc, &ctx->gz_htail})
-            if (g->p) cudaFreeHost(g->p);
-        for (int i = 0; i < 3; i++)
-            if (ctx->gz_up[i]) cudaEventDestroy(ctx->gz_up[i]);
-        if (ctx->gz_pre) cudaEventDestroy(ctx->gz_pre);
-        if (ctx->d_replicas) cudaFree(ctx->d_replicas);
-        ctx->ahead.reset();
-        for (int i = 0; i < 3; i++)
-            if (ctx->file_buf[i]) cudaFreeHost(ctx->file_buf[i]);
-        for (int i = 0; i < 3; i++)
-            if (ctx->file_buf2[i]) cudaFreeHost(ctx->file_buf2[i]);
-        if (ctx->stream) cudaStreamDestroy(ctx->stream);
-        if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-    }
-    delete ctx;
+    cudaSetDevice(ctx->device);
+    if (ctx->stream) cudaStreamSynchronize(ctx->stream);
+    if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
+    ctx->ahead.reset();          // the read-ahead thread writes into the pinned file buffers: joined before they are freed
+    if (ctx->comm && tdg::nccl().CommDestroy) tdg::nccl().CommDestroy(ctx->comm);
+    cudaStream_t stream = ctx->stream, copy_stream = ctx->copy_stream;
+    delete ctx;                  // every buffer and event of the context
+    if (stream) cudaStreamDestroy(stream);
+    if (copy_stream) cudaStreamDestroy(copy_stream);
 }
 
 int tdg_set_tags(tdg_ctx *ctx, const char *bases, const uint64_t *off, const int32_t *col, uint32_t ntags,
@@ -781,21 +851,11 @@ int tdg_set_tags(tdg_ctx *ctx, const char *bases, const uint64_t *off, const int
     {
         CK(cudaSetDevice(ctx->device));
         CK(cudaStreamSynchronize(ctx->stream));
-        size_t ne = ctx->tags.entries.size(), nx = ctx->tags.ext.size();
-        if (ne > ctx->d_entries_cap) {
-            if (ctx->d_entries) CK(cudaFree(ctx->d_entries));
-            ctx->d_entries = nullptr;
-            CK(cudaMalloc(&ctx->d_entries, std::max<size_t>(ne, 1) * sizeof(tdg::TagEntry)));
-            ctx->d_entries_cap = ne;
-        }
-        if (nx > ctx->d_ext_cap || !ctx->d_ext) {
-            if (ctx->d_ext) CK(cudaFree(ctx->d_ext));
-            ctx->d_ext = nullptr;
-            CK(cudaMalloc(&ctx->d_ext, std::max<size_t>(nx, 1) * sizeof(uint64_t)));
-            ctx->d_ext_cap = nx;
-        }
-        if (ne) CK(cudaMemcpy(ctx->d_entries, ctx->tags.entries.data(), ne * sizeof(tdg::TagEntry), cudaMemcpyHostToDevice));
-        if (nx) CK(cudaMemcpy(ctx->d_ext, ctx->tags.ext.data(), nx * sizeof(uint64_t), cudaMemcpyHostToDevice));
+        size_t ne = ctx->tags.entries.size() * sizeof(tdg::TagEntry), nx = ctx->tags.ext.size() * sizeof(uint64_t);
+        int rc;
+        if ((rc = grow_exact(ctx, ctx->d_entries, ne, false)) || (rc = grow_exact(ctx, ctx->d_ext, std::max<size_t>(nx, 8), false))) return rc;
+        if (ne) CK(cudaMemcpy(ctx->d_entries.p, ctx->tags.entries.data(), ne, cudaMemcpyHostToDevice));
+        if (nx) CK(cudaMemcpy(ctx->d_ext.p, ctx->tags.ext.data(), nx, cudaMemcpyHostToDevice));
     }
     ctx->have_tags = true;
     return TDG_OK;
@@ -807,13 +867,12 @@ int tdg_set_matrix(tdg_ctx *ctx, uint32_t rows, uint32_t cols)
     if ((uint64_t)rows * cols >= 0xFFFFFFFFull) return fail(ctx, TDG_ERR_ARG, "matrix must have fewer than 2^32 - 1 cells");
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (ctx->own_matrix && ctx->d_matrix) CK(cudaFree(ctx->d_matrix));
-    ctx->d_matrix = nullptr;
-    CK(cudaMalloc(&ctx->d_matrix, (size_t)rows * cols * sizeof(int32_t)));
-    ctx->own_matrix = true;
+    int rc = grow_exact(ctx, ctx->matrix, (size_t)rows * cols * sizeof(int32_t), false);
+    if (rc) return rc;
+    ctx->d_matrix = (int32_t *)ctx->matrix.p;
     ctx->rows = rows;
     ctx->cols = cols;
-    int rc = size_replicas(ctx);
+    rc = size_replicas(ctx);
     if (rc) return rc;
     return tdg_zero_matrix(ctx);
 }
@@ -826,9 +885,8 @@ int tdg_bind_matrix(tdg_ctx *ctx, void *dev_int32, uint32_t rows, uint32_t cols)
     if ((uint64_t)rows * cols >= 0xFFFFFFFFull) return fail(ctx, TDG_ERR_ARG, "matrix must have fewer than 2^32 - 1 cells");
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (ctx->own_matrix && ctx->d_matrix) CK(cudaFree(ctx->d_matrix));
+    ctx->matrix.reset();
     ctx->d_matrix = (int32_t *)dev_int32;
-    ctx->own_matrix = false;
     ctx->rows = rows;
     ctx->cols = cols;
     return size_replicas(ctx);
@@ -861,16 +919,11 @@ int tdg_begin_file(tdg_ctx *ctx, const char *bases, const uint32_t *off, const i
         CK(cudaSetDevice(ctx->device));
         // the previous file's kernels read the old table
         CK(cudaStreamSynchronize(ctx->stream));
-        size_t nb = round_up(ctx->bar_blob.size(), 16);
-        if (nb > ctx->d_bar_cap) {
-            if (ctx->d_bar) CK(cudaFree(ctx->d_bar));
-            ctx->d_bar = nullptr;
-            CK(cudaMalloc(&ctx->d_bar, nb));
-            ctx->d_bar_cap = nb;
-        }
-        CK(cudaMemcpy(ctx->d_bar, ctx->bar_blob.data(), ctx->bar_blob.size(), cudaMemcpyHostToDevice));
-        CK(cudaMemsetAsync(ctx->d_state, 0, 2 * sizeof(tdg::LineState), ctx->stream));
-        CK(cudaMemsetAsync(ctx->d_totals, 0, 4 * sizeof(unsigned long long), ctx->stream));
+        int rc = grow_exact(ctx, ctx->d_bar, round_up(ctx->bar_blob.size(), 16), false);
+        if (rc) return rc;
+        CK(cudaMemcpy(ctx->d_bar.p, ctx->bar_blob.data(), ctx->bar_blob.size(), cudaMemcpyHostToDevice));
+        CK(cudaMemsetAsync(ctx->d_state.p, 0, 2 * sizeof(tdg::LineState), ctx->stream));
+        CK(cudaMemsetAsync(ctx->d_totals.p, 0, 4 * sizeof(unsigned long long), ctx->stream));
         ctx->state_cur = 0;
     }
     ctx->have_bar = true;
@@ -885,8 +938,8 @@ int tdg_reset_file(tdg_ctx *ctx)
     if (!ctx->have_bar) return fail(ctx, TDG_ERR_STATE, "tdg_begin_file has not been called");
     if (ctx->carry_len) return fail(ctx, TDG_ERR_STATE, "previous file was not ended (tdg_end_file)");
     CK(cudaSetDevice(ctx->device));
-    CK(cudaMemsetAsync(ctx->d_state, 0, 2 * sizeof(tdg::LineState), ctx->stream));
-    CK(cudaMemsetAsync(ctx->d_totals, 0, 4 * sizeof(unsigned long long), ctx->stream));
+    CK(cudaMemsetAsync(ctx->d_state.p, 0, 2 * sizeof(tdg::LineState), ctx->stream));
+    CK(cudaMemsetAsync(ctx->d_totals.p, 0, 4 * sizeof(unsigned long long), ctx->stream));
     ctx->state_cur = 0;
     return TDG_OK;
 }
@@ -898,7 +951,9 @@ int tdg_submit(tdg_ctx *ctx, const void *bytes, size_t n, uint64_t reads_limit)
     if (n == 0) return TDG_OK;
     if (!bytes) return fail(ctx, TDG_ERR_ARG, "null buffer");
     CK(cudaSetDevice(ctx->device));
-    return submit_impl(ctx, (const uint8_t *)bytes, n, reads_limit, true);
+    rc = submit_impl(ctx, (const uint8_t *)bytes, n, reads_limit, true);
+    if (rc) ctx->carry_len = 0;          // the file is given up, as in tdg_count_file: tdg_begin_file starts the next one
+    return rc;
 }
 
 int tdg_end_file(tdg_ctx *ctx, uint64_t reads_limit)
@@ -907,8 +962,9 @@ int tdg_end_file(tdg_ctx *ctx, uint64_t reads_limit)
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     rc = ensure_slots(ctx);
-    if (rc) return rc;
-    return end_file_impl(ctx, reads_limit);
+    if (rc == TDG_OK) rc = end_file_impl(ctx, reads_limit);
+    if (rc) ctx->carry_len = 0;
+    return rc;
 }
 
 int tdg_count_device(tdg_ctx *ctx, const void *dev_bytes, size_t n, uint64_t line_base, int prev_kind,
@@ -938,7 +994,7 @@ int tdg_count_lines_device(tdg_ctx *ctx, const void *dev_bytes, size_t n, uint64
     rc = launch_chunk<false>(ctx, dev_bytes, n, line_base, prev_kind, 0);
     if (rc) return rc;
     tdg::LineState st;
-    CK(cudaMemcpyAsync(&st, ctx->d_state + ctx->state_cur, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, (tdg::LineState *)ctx->d_state.p + ctx->state_cur, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     state[0] = st.next_line;
     state[1] = st.prev_kind;
@@ -963,8 +1019,8 @@ int tdg_file_totals(tdg_ctx *ctx, uint64_t totals[4])
     CK(cudaSetDevice(ctx->device));
     unsigned long long t[4];
     tdg::LineState st;
-    CK(cudaMemcpyAsync(t, ctx->d_totals, sizeof(t), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(&st, ctx->d_state + ctx->state_cur, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(t, ctx->d_totals.p, sizeof(t), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, (tdg::LineState *)ctx->d_state.p + ctx->state_cur, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     totals[0] = t[0];
     totals[1] = t[1];
@@ -993,7 +1049,7 @@ int tdg_matrix_min(tdg_ctx *ctx, int32_t *out)
     if (!ctx->d_matrix) return fail(ctx, TDG_ERR_STATE, "no matrix");
     if (!out) return fail(ctx, TDG_ERR_ARG, "null argument");
     CK(cudaSetDevice(ctx->device));
-    int32_t *d_min = (int32_t *)(ctx->d_totals + 3);          // the spare word behind the three totals
+    int32_t *d_min = (int32_t *)((unsigned long long *)ctx->d_totals.p + 3);          // the spare word behind the three totals
     const int32_t init = 0x7FFFFFFF;
     CK(cudaMemcpyAsync(d_min, &init, sizeof(init), cudaMemcpyHostToDevice, ctx->stream));
     const uint32_t cells = ctx->rows * ctx->cols;
@@ -1014,7 +1070,7 @@ int tdg_stream_wait(tdg_ctx *ctx, void *other_stream)
     int rc = need_device(ctx);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->handoff) CK(cudaEventCreateWithFlags(&ctx->handoff, cudaEventDisableTiming));
+    if ((rc = make_event(ctx, ctx->handoff))) return rc;
     CK(cudaEventRecord(ctx->handoff, (cudaStream_t)other_stream));
     CK(cudaStreamWaitEvent(ctx->stream, ctx->handoff, 0));
     return TDG_OK;
@@ -1025,7 +1081,7 @@ int tdg_other_stream_wait(tdg_ctx *ctx, void *other_stream)
     int rc = need_device(ctx);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->handoff) CK(cudaEventCreateWithFlags(&ctx->handoff, cudaEventDisableTiming));
+    if ((rc = make_event(ctx, ctx->handoff))) return rc;
     CK(cudaEventRecord(ctx->handoff, ctx->stream));
     CK(cudaStreamWaitEvent((cudaStream_t)other_stream, ctx->handoff, 0));
     return TDG_OK;
@@ -1149,10 +1205,7 @@ int tdg_timing_begin(tdg_ctx *ctx)
     int rc = need_device(ctx);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
-    if (ctx->tev.empty()) {
-        ctx->tev.resize(2 * MAX_TIMED);
-        for (auto &ev : ctx->tev) CK(cudaEventCreate(&ev));
-    }
+    ctx->tev.resize(2 * MAX_TIMED);      // (created as they are first used: timed_start)
     ctx->tev_used = 0;
     ctx->timing = true;
     return TDG_OK;
@@ -1184,25 +1237,10 @@ namespace {
 
 int ensure_file_bufs(tdg_ctx *ctx, int set)
 {
-    uint8_t **buf = set ? ctx->file_buf2 : ctx->file_buf;
-    size_t &cap = set ? ctx->file_buf2_cap : ctx->file_buf_cap;
-    if (cap >= ctx->chunk_bytes) return TDG_OK;
-    for (int i = 0; i < 3; i++) {
-        if (buf[i]) cudaFreeHost(buf[i]);
-        buf[i] = nullptr;
+    for (Buf &b : ctx->file_buf[set]) {
+        int rc = grow_exact(ctx, b, ctx->chunk_bytes, true);
+        if (rc) return rc;
     }
-    cap = 0;
-    for (int i = 0; i < 3; i++) {
-        cudaError_t e = cudaHostAlloc(&buf[i], ctx->chunk_bytes, cudaHostAllocDefault);
-        if (e != cudaSuccess) {
-            for (int k = 0; k <= i; k++) {
-                if (buf[k]) cudaFreeHost(buf[k]);
-                buf[k] = nullptr;
-            }
-            return fail(ctx, TDG_ERR_CUDA, std::string("cudaHostAlloc: ") + cudaGetErrorString(e));
-        }
-    }
-    cap = ctx->chunk_bytes;
     return TDG_OK;
 }
 
@@ -1218,8 +1256,7 @@ size_t file_chunk(const tdg_ctx *ctx, uint64_t reads_limit)
 std::unique_ptr<FileReader> start_reader(tdg_ctx *ctx, const char *path, bool gz, size_t chunk, int set, const GzHandover *ho)
 {
     std::unique_ptr<FileReader> r(new FileReader());
-    uint8_t **buf = set ? ctx->file_buf2 : ctx->file_buf;
-    for (int i = 0; i < FileReader::NBUF; i++) r->bufs[i].p = buf[i];
+    for (int i = 0; i < FileReader::NBUF; i++) r->bufs[i].p = (uint8_t *)ctx->file_buf[set][i].p;
     r->path = path;
     r->gz = gz;
     r->chunk = chunk;
@@ -1280,12 +1317,12 @@ int tdg_count_file2(tdg_ctx *ctx, const char *path, int gz, uint64_t reads_limit
         if (drc == TDG_OK && handled && dcarry) {
             // the bytes behind the last line end become the host path's carry
             Slot &cs = ctx->slot[ctx->next_slot];
-            drc = grow_carry(ctx, cs, dcarry, 0);
+            drc = grow_carry(ctx, cs.carry, dcarry, 0);
             if (drc == TDG_OK) {
-                CK(cudaMemcpyAsync(cs.carry, ctx->gz_text.p, dcarry, cudaMemcpyDeviceToHost, ctx->stream));
+                CK(cudaMemcpyAsync(cs.carry.p, ctx->gz_text.p, dcarry, cudaMemcpyDeviceToHost, ctx->stream));
                 CK(cudaStreamSynchronize(ctx->stream));
                 ctx->carry_len = dcarry;
-                lim.last_byte = cs.carry[dcarry - 1];
+                lim.last_byte = ((const uint8_t *)cs.carry.p)[dcarry - 1];
                 if (lim.careful) lim.ll.prev_cr = lim.last_byte == '\r';
             }
         }
@@ -1383,7 +1420,8 @@ int tdg_last_file_info(tdg_ctx *ctx, int64_t info[3])
 }
 
 // Gives the working buffers of the device-side gzip feed back (a 1.2 GB round holds about 12 GB:
-// tokens, symbols, windows, text).  They are kept between files otherwise.
+// tokens, symbols, windows, text), and the staging buffer of the batch calls.  They are kept between
+// calls otherwise.
 int tdg_release_scratch(tdg_ctx *ctx)
 {
     int rc = need_device(ctx);
@@ -1391,13 +1429,11 @@ int tdg_release_scratch(tdg_ctx *ctx)
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
     CK(cudaStreamSynchronize(ctx->copy_stream));
-    for (tdg_ctx::Grow *g : {&ctx->gz_comp, &ctx->gz_comp2, &ctx->gz_syms, &ctx->gz_sym2, &ctx->gz_ntok, &ctx->gz_meta, &ctx->gz_cand,
-                             &ctx->gz_ncand, &ctx->gz_windows, &ctx->gz_text, &ctx->gz_crc, &ctx->gz_lens, &ctx->gz_offs, &ctx->gz_carry,
-                             &ctx->gz_cold}) {
-        if (g->p) cudaFree(g->p);
-        g->p = nullptr;
-        g->cap = 0;
-    }
+    // gz_tabs stays: gz_tables uploads the tables once per context.  The pinned gz_h* buffers stay too:
+    // they are small (a round's chunk metadata and CRCs, the tail of its text searched for a line end).
+    for (Buf *b : {&ctx->gz_comp, &ctx->gz_comp2, &ctx->gz_syms, &ctx->gz_sym2, &ctx->gz_ntok, &ctx->gz_meta, &ctx->gz_cand, &ctx->gz_ncand,
+                   &ctx->gz_windows, &ctx->gz_text, &ctx->gz_crc, &ctx->gz_lens, &ctx->gz_offs, &ctx->gz_carry, &ctx->gz_cold, &ctx->batch})
+        b->reset();
     return TDG_OK;
 }
 
@@ -1441,10 +1477,7 @@ int tdg_gz_inflate_host(tdg_ctx *ctx, const char *path, void *dst, size_t cap, u
     size_t used = sink.used;
     if (!handled || ho.active) {
         tdg::Feeder feed;
-        int orc = !ho.active ? feed.open(path, true)
-                  : ho.bgzf  ? feed.open_resume_bgzf(path, ho.bgzf_off, ho.delivered)
-                             : feed.open_resume(path, ho.pos_bit, ho.to_zlib ? nullptr : ho.window.data(), ho.hist, ho.crc, ho.member_len,
-                                                ho.delivered);
+        int orc = open_feed(feed, path, true, &ho);
         if (orc) return fail(ctx, orc, feed.error());
         for (;;) {
             if (used == cap) return fail(ctx, TDG_ERR_ARG, "output buffer too small");
@@ -1504,24 +1537,21 @@ int tdg_set_trim(tdg_ctx *ctx, const char *site0, const char *site1, const char 
     if (ncand) memcpy(blob.data() + o_cand, cand.data(), ncand * sizeof(tdg::TrimCand));
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (total > ctx->d_trim_cap) {
-        if (ctx->d_trim) CK(cudaFree(ctx->d_trim));
-        ctx->d_trim = nullptr;
-        CK(cudaMalloc(&ctx->d_trim, total));
-        ctx->d_trim_cap = total;
-    }
-    CK(cudaMemcpy(ctx->d_trim, blob.data(), total, cudaMemcpyHostToDevice));
+    rc = grow_exact(ctx, ctx->d_trim, total, false);
+    if (rc) return rc;
+    const uint8_t *d = (const uint8_t *)ctx->d_trim.p;
+    CK(cudaMemcpy(ctx->d_trim.p, blob.data(), total, cudaMemcpyHostToDevice));
     tdg::TrimArgs &t = ctx->trim;
     memset(&t, 0, sizeof(t));
-    t.site0 = ctx->d_trim + o_site0;
-    t.site1 = ctx->d_trim + o_site1;
+    t.site0 = d + o_site0;
+    t.site1 = d + o_site1;
     t.len0 = (uint32_t)l0;
     t.len1 = (uint32_t)l1;
-    t.a0 = ctx->d_trim + o_a0;
-    t.a1 = ctx->d_trim + o_a1;
-    t.a1_off = (const uint32_t *)(ctx->d_trim + o_a1off);
-    t.cand_off = (const uint32_t *)(ctx->d_trim + o_coff);
-    t.cand = (const tdg::TrimCand *)(ctx->d_trim + o_cand);
+    t.a0 = d + o_a0;
+    t.a1 = d + o_a1;
+    t.a1_off = (const uint32_t *)(d + o_a1off);
+    t.cand_off = (const uint32_t *)(d + o_coff);
+    t.cand = (const tdg::TrimCand *)(d + o_cand);
     ctx->trim_nbar = nbar;
     ctx->have_trim = true;
     return TDG_OK;
@@ -1540,38 +1570,18 @@ int tdg_trim_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, const in
         if (off[i + 1] < off[i]) return fail(ctx, TDG_ERR_ARG, "offsets must be non-decreasing");
     }
     CK(cudaSetDevice(ctx->device));
-    const size_t nbytes = (size_t)(off[n] - off[0]);
-    const size_t o_off = round_up(nbytes + 16, 16), o_bar = o_off + round_up((n + 1) * sizeof(uint64_t), 16),
-                 o_start = o_bar + round_up(n * sizeof(int32_t), 16), o_out = o_start + round_up(n * sizeof(uint32_t), 16),
-                 total = o_out + round_up(n * sizeof(int32_t), 16);
-    uint8_t *d = nullptr;
-    CK(cudaMalloc(&d, total));
-    std::vector<unsigned long long> rel(n + 1);
-    for (uint32_t i = 0; i <= n; i++) rel[i] = off[i] - off[0];
-    cudaError_t e = cudaSuccess;
-    if (nbytes) e = cudaMemcpyAsync(d, seqs + off[0], nbytes, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_off, rel.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_bar, bar, n * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_start, start, n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) {
-        tdg::TrimArgs t = ctx->trim;
-        t.seqs = d;
-        t.off = (const unsigned long long *)(d + o_off);
-        t.bar = (const int32_t *)(d + o_bar);
-        t.start = (const uint32_t *)(d + o_start);
-        t.n = n;
-        t.out = (int32_t *)(d + o_out);
-        const unsigned per = tdg::TRIM_THREADS / 32;
-        tdg::trim_kernel<<<(n + per - 1) / per, tdg::TRIM_THREADS, 0, ctx->stream>>>(t);
-        e = cudaGetLastError();
-        ctx->launches += 1;
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(slice2, d + o_out, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
-    cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d);
-    if (e != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string("tdg_trim_batch: ") + cudaGetErrorString(e));
-    if (e2 != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string("tdg_trim_batch: ") + cudaGetErrorString(e2));
-    return TDG_OK;
+    return batch_run(ctx, "tdg_trim_batch", seqs, off, n, {{bar, nullptr, n * sizeof(int32_t)}, {start, nullptr, n * sizeof(uint32_t)}, {nullptr, slice2, n * sizeof(int32_t)}},
+                     [&](const uint8_t *d, const unsigned long long *d_off, uint8_t *const *part) {
+                         tdg::TrimArgs t = ctx->trim;
+                         t.seqs = d;
+                         t.off = d_off;
+                         t.bar = (const int32_t *)part[0];
+                         t.start = (const uint32_t *)part[1];
+                         t.n = n;
+                         t.out = (int32_t *)part[2];
+                         const unsigned per = tdg::TRIM_THREADS / 32;
+                         tdg::trim_kernel<<<(n + per - 1) / per, tdg::TRIM_THREADS, 0, ctx->stream>>>(t);
+                     });
 }
 
 int tdg_split_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, uint32_t n, const uint32_t *bar_len,
@@ -1588,41 +1598,22 @@ int tdg_split_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, uint32_
     for (uint32_t i = 0; i < n; i++)
         if (off[i + 1] < off[i]) return fail(ctx, TDG_ERR_ARG, "offsets must be non-decreasing");
     CK(cudaSetDevice(ctx->device));
-    const size_t nbytes = (size_t)(off[n] - off[0]);
-    const size_t o_off = round_up(nbytes + 16, 16), o_len = o_off + round_up((n + 1) * sizeof(uint64_t), 16),
-                 o_bar = o_len + round_up(nbar * sizeof(uint32_t), 16), o_out = o_bar + round_up(n * sizeof(int32_t), 16),
-                 total = o_out + round_up(n * sizeof(int32_t), 16);
-    uint8_t *d = nullptr;
-    CK(cudaMalloc(&d, total));
-    std::vector<unsigned long long> rel(n + 1);
-    for (uint32_t i = 0; i <= n; i++) rel[i] = off[i] - off[0];
-    cudaError_t e = cudaSuccess;
-    if (nbytes) e = cudaMemcpyAsync(d, seqs + off[0], nbytes, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_off, rel.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_len, bar_len, nbar * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) {
-        tdg::SplitArgs a;
-        a.t = ctx->trim;
-        a.t.seqs = d;
-        a.t.off = (const unsigned long long *)(d + o_off);
-        a.t.n = n;
-        a.t.out = (int32_t *)(d + o_out);
-        a.bar = (const tdg::BarTable *)ctx->d_bar;
-        a.bar_len = (const uint32_t *)(d + o_len);
-        a.cutlen = cutlen;
-        a.bar_out = (int32_t *)(d + o_bar);
-        const unsigned per = tdg::TRIM_THREADS / 32;
-        tdg::split_kernel<<<(n + per - 1) / per, tdg::TRIM_THREADS, 0, ctx->stream>>>(a);
-        e = cudaGetLastError();
-        ctx->launches += 1;
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(bar_out, d + o_bar, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(slice2, d + o_out, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
-    cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d);
-    if (e != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string("tdg_split_batch: ") + cudaGetErrorString(e));
-    if (e2 != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string("tdg_split_batch: ") + cudaGetErrorString(e2));
-    return TDG_OK;
+    return batch_run(ctx, "tdg_split_batch", seqs, off, n,
+                     {{bar_len, nullptr, nbar * sizeof(uint32_t)}, {nullptr, bar_out, n * sizeof(int32_t)}, {nullptr, slice2, n * sizeof(int32_t)}},
+                     [&](const uint8_t *d, const unsigned long long *d_off, uint8_t *const *part) {
+                         tdg::SplitArgs a;
+                         a.t = ctx->trim;
+                         a.t.seqs = d;
+                         a.t.off = d_off;
+                         a.t.n = n;
+                         a.t.out = (int32_t *)part[2];
+                         a.bar = (const tdg::BarTable *)ctx->d_bar.p;
+                         a.bar_len = (const uint32_t *)part[0];
+                         a.cutlen = cutlen;
+                         a.bar_out = (int32_t *)part[1];
+                         const unsigned per = tdg::TRIM_THREADS / 32;
+                         tdg::split_kernel<<<(n + per - 1) / per, tdg::TRIM_THREADS, 0, ctx->stream>>>(a);
+                     });
 }
 
 // ---------------------------------------------------------------------------
@@ -1700,8 +1691,8 @@ static int bgzf_run(tdg_ctx *ctx, const uint8_t *d_new, const uint64_t *off, boo
         a.size = (uint32_t *)ctx->bz_size.p;
         a.table = (const uint32_t *)((const uint8_t *)ctx->gz_tabs.p + 512);
         for (int j = 0; j < 8; j++) a.op[j] = ctx->bz_op[j];
-        const bool timed = ctx->timing && ctx->tev_used + 2 <= MAX_TIMED * 2;     // tdg_timing_*: the three as one
-        if (timed) CK(cudaEventRecord(ctx->tev[ctx->tev_used++], st));
+        bool timed;                                      // tdg_timing_*: the three as one
+        if ((rc = timed_start(ctx, timed))) return rc;
         bz::bgzf_deflate<<<nm, bz::THREADS, sizeof(bz::Shared), st>>>(a);
         tdg::tile_scan<<<1, 1024, 0, st>>>(a.size, nm);
         bz::bgzf_pack<<<nm, 256, 0, st>>>(a.mem, a.work, a.size, (uint8_t *)ctx->bz_out.p);
@@ -1894,7 +1885,7 @@ int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_bloc
     w.bar_base = bar_total + nbar;
     w.complex_flag = (uint32_t *)(bar_total + 2 * nbar + 1);
     w.s.t = ctx->trim;
-    w.s.bar = (const tdg::BarTable *)ctx->d_bar;
+    w.s.bar = (const tdg::BarTable *)ctx->d_bar.p;
     w.bar_off = (const uint32_t *)ctx->sp_tabs.p;
     w.s.bar_len = w.bar_off + nbar + 1;
     w.barcodes = (const uint8_t *)(w.s.bar_len + nbar);
@@ -1987,38 +1978,20 @@ int tdg_match_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, uint32_
     for (uint32_t i = 0; i < n; i++)
         if (off[i + 1] < off[i]) return fail(ctx, TDG_ERR_ARG, "offsets must be non-decreasing");
     CK(cudaSetDevice(ctx->device));
-    const size_t nbytes = (size_t)(off[n] - off[0]);
-    const size_t o_off = round_up(nbytes + 16, 16), o_row = o_off + round_up((n + 1) * sizeof(uint64_t), 16),
-                 o_col = o_row + round_up(n * sizeof(int32_t), 16), total = o_col + round_up(n * sizeof(int32_t), 16);
-    uint8_t *d = nullptr;
-    CK(cudaMalloc(&d, total));
-    std::vector<unsigned long long> rel(n + 1);
-    for (uint32_t i = 0; i <= n; i++) rel[i] = off[i] - off[0];
-    cudaError_t e = cudaSuccess;
-    if (nbytes) e = cudaMemcpyAsync(d, seqs + off[0], nbytes, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_off, rel.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) {
-        tdg::MatchArgs a;
-        a.seqs = d;
-        a.off = (const unsigned long long *)(d + o_off);
-        a.n = n;
-        a.bar = (const tdg::BarTable *)ctx->d_bar;
-        a.tags = ctx->tags.t;
-        a.tags.entries = ctx->d_entries;
-        a.tags.ext = ctx->d_ext;
-        a.row_out = (int32_t *)(d + o_row);
-        a.col_out = (int32_t *)(d + o_col);
-        tdg::match_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(a);
-        e = cudaGetLastError();
-        ctx->launches += 1;
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(row_out, d + o_row, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(col_out, d + o_col, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);
-    cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d);
-    if (e != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string("tdg_match_batch: ") + cudaGetErrorString(e));
-    if (e2 != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string("tdg_match_batch: ") + cudaGetErrorString(e2));
-    return TDG_OK;
+    return batch_run(ctx, "tdg_match_batch", seqs, off, n, {{nullptr, row_out, n * sizeof(int32_t)}, {nullptr, col_out, n * sizeof(int32_t)}},
+                     [&](const uint8_t *d, const unsigned long long *d_off, uint8_t *const *part) {
+                         tdg::MatchArgs a;
+                         a.seqs = d;
+                         a.off = d_off;
+                         a.n = n;
+                         a.bar = (const tdg::BarTable *)ctx->d_bar.p;
+                         a.tags = ctx->tags.t;
+                         a.tags.entries = (const tdg::TagEntry *)ctx->d_entries.p;
+                         a.tags.ext = (const uint64_t *)ctx->d_ext.p;
+                         a.row_out = (int32_t *)part[0];
+                         a.col_out = (int32_t *)part[1];
+                         tdg::match_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(a);
+                     });
 }
 
 // ---------------------------------------------------------------------------

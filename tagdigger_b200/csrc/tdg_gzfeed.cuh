@@ -3,7 +3,7 @@
 // tdg_gzdev.cuh, the per-lane inflater in tdg_gzlane.h, the chain of a round in tdg_gzchain.h.
 //
 // This file is PART OF tdg_api.cu (included there, inside its anonymous namespace, behind the
-// definitions of tdg_ctx, fail, CK, grow, launch_chunk, line_cut, grow_carry, ensure_slots): it is a
+// definitions of tdg_ctx, Buf, fail, CK, grow, make_event, launch_chunk, line_cut, ensure_slots): it is a
 // separate file for the reader's sake, not a separate unit.
 // ---------------------------------------------------------------------------
 // Device-side gzip feed (tdg_gzlane.h, tdg_gzchain.h, tdg_gzdev.cuh)
@@ -121,8 +121,9 @@ int gz_tables(tdg_ctx *ctx)
     }
     CK(cudaMemcpy(ctx->gz_tabs.p, blob.data(), blob.size(), cudaMemcpyHostToDevice));
     for (int j = 0; j < 8; j++) ctx->gz_op[j] = (uint32_t)crc32_combine_gen((z_off_t)(tdg::gzd::SUB << j));
-    for (int i = 0; i < 3; i++) CK(cudaEventCreateWithFlags(&ctx->gz_up[i], cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&ctx->gz_pre, cudaEventDisableTiming));
+    for (Event &ev : ctx->gz_up)
+        if ((rc = make_event(ctx, ev))) return rc;
+    if ((rc = make_event(ctx, ctx->gz_pre))) return rc;
     CK(cudaFuncSetAttribute(tdg::gzd::gz_decode, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tdg::gzd::DEC_SMEM));
     CK(cudaFuncSetAttribute(tdg::gzd::gz_scan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tdg::gzd::SCAN_SMEM));
     ctx->gz_tables = true;
@@ -145,17 +146,18 @@ struct GzMap {
 int gz_upload(tdg_ctx *ctx, const GzMap &map, const char *path, int threads, int &up_i, int which, size_t off, size_t end,
               cudaStream_t stream)
 {
-    tdg_ctx::Grow &g = which ? ctx->gz_comp2 : ctx->gz_comp;
+    Buf &g = which ? ctx->gz_comp2 : ctx->gz_comp;
     const size_t nb = end - off, padded = (nb + 3) / 4 * 4 + 256;
     int rc = grow(ctx, g, padded, false);
     if (rc) return rc;
-    const size_t piece = ctx->file_buf_cap;
+    const size_t piece = ctx->chunk_bytes;                  // the size of the pinned file buffers
     for (size_t at = 0; at < nb; at += piece, up_i = (up_i + 1) % 3) {
         const size_t m = std::min(piece, nb - at);
+        uint8_t *pinned = (uint8_t *)ctx->file_buf[0][up_i].p;
         CK(cudaEventSynchronize(ctx->gz_up[up_i]));
-        if (!gz_pread_parallel(map.fd, ctx->file_buf[up_i], m, off + at, threads))
+        if (!gz_pread_parallel(map.fd, pinned, m, off + at, threads))
             return fail(ctx, TDG_ERR_IO, std::string("read error on ") + path);
-        CK(cudaMemcpyAsync((uint8_t *)g.p + at, ctx->file_buf[up_i], m, cudaMemcpyHostToDevice, stream));
+        CK(cudaMemcpyAsync((uint8_t *)g.p + at, pinned, m, cudaMemcpyHostToDevice, stream));
         CK(cudaEventRecord(ctx->gz_up[up_i], stream));
     }
     CK(cudaMemsetAsync((uint8_t *)g.p + nb, 0, padded - nb, stream));
@@ -444,8 +446,9 @@ int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, 
     size_t pre_off = 0, pre_end = 0;
 
     // One round.  TDG_ERR_NOMEM from a buffer that cannot be had is not the file's fault: nothing of the round
-    // has been delivered then, and the host reader takes over at the state the round began in.
-    int round_no = 0;
+    // has been delivered then, and the host reader takes over at the state the round began in.  Not so once
+    // the sink has the round's text (st has moved past it): its failure ends the feed (sink_rc).
+    int round_no = 0, sink_rc = TDG_OK;
     const int oom_round = getenv("TDG_GZDEV_OOM_ROUND") ? atoi(getenv("TDG_GZDEV_OOM_ROUND")) : -1;      // test hook
     auto one_round = [&]() -> int {
         if (round_no++ == oom_round) return fail(ctx, TDG_ERR_NOMEM, "buffer of 0 bytes: simulated (TDG_GZDEV_OOM_ROUND)");
@@ -473,7 +476,7 @@ int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, 
             if (rc) return rc;
         }
         pre_valid = false;
-        tdg_ctx::Grow &comp = cur ? ctx->gz_comp2 : ctx->gz_comp;
+        Buf &comp = cur ? ctx->gz_comp2 : ctx->gz_comp;
         if ((rc = grow(ctx, ctx->gz_syms, (size_t)r.nchunks * tokcap * 2, false))) return rc;
         if ((rc = grow(ctx, ctx->gz_meta, (size_t)r.nchunks * sizeof(gzl::Meta), false))) return rc;
         if ((rc = grow(ctx, ctx->gz_cand, (size_t)r.nchunks * gzd::MAXC * 4, false))) return rc;
@@ -681,7 +684,7 @@ int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, 
             return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + path + ": incorrect data check");
         if (o.accepted && text_len) {
             rc = sink.text(ctx, (uint8_t *)ctx->gz_text.p, carry, (size_t)text_len);
-            if (rc) return rc;
+            if (rc) return sink_rc = rc;
         }
         auto t6 = now();
         if (stats) {
@@ -705,7 +708,7 @@ int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, 
     };
     while (!st.eof && !st.handover) {
         rc = one_round();
-        if (rc == TDG_ERR_NOMEM || rc == TDG_STOP_ROUND) {
+        if (!sink_rc && (rc == TDG_ERR_NOMEM || rc == TDG_STOP_ROUND)) {
             st.handover = true;
             st.why = rc == TDG_ERR_NOMEM ? "device memory" : "read limit within reach";
             pre_valid = false;
