@@ -101,7 +101,6 @@ struct GzHandover {
     uint64_t pos_bit = 0, member_len = 0, delivered = 0;
     uint32_t hist = 0, crc = 0;
     std::vector<uint8_t> window;
-    std::string why;
 };
 
 // The host feeder of `path`: from the start, or where the device gzip feed handed over (ho->active)
@@ -1305,20 +1304,22 @@ int tdg_count_file2(tdg_ctx *ctx, const char *path, int gz, uint64_t reads_limit
     // feeder below, which resumes exactly where the device feed stopped.
     tdg::Utf8State u8;
     GzHandover ho;
+    int result = TDG_OK;
+    bool at_eof = false;
     if (!reader && gz && gz_device_wanted(ctx, path, reads_limit)) {
         bool handled = false;
         size_t dcarry = 0;
         GzCountSink sink(reads_limit, &lim);
         GzStats gst;
-        int drc = gz_device_feed(ctx, path, sink, handled, ho, dcarry, &gst, &u8);
+        result = gz_device_feed(ctx, path, sink, handled, ho, dcarry, gst, &u8);
         ctx->last_file[0] = gst.rounds;
         ctx->last_file[1] = gst.accepted;
         ctx->last_file[2] = !handled ? -1 : (ho.active ? 1 : 0);
-        if (drc == TDG_OK && handled && dcarry) {
+        if (result == TDG_OK && handled && dcarry) {
             // the bytes behind the last line end become the host path's carry
             Slot &cs = ctx->slot[ctx->next_slot];
-            drc = grow_carry(ctx, cs.carry, dcarry, 0);
-            if (drc == TDG_OK) {
+            result = grow_carry(ctx, cs.carry, dcarry, 0);
+            if (result == TDG_OK) {
                 CK(cudaMemcpyAsync(cs.carry.p, ctx->gz_text.p, dcarry, cudaMemcpyDeviceToHost, ctx->stream));
                 CK(cudaStreamSynchronize(ctx->stream));
                 ctx->carry_len = dcarry;
@@ -1326,32 +1327,19 @@ int tdg_count_file2(tdg_ctx *ctx, const char *path, int gz, uint64_t reads_limit
                 if (lim.careful) lim.ll.prev_cr = lim.last_byte == '\r';
             }
         }
-        if (drc == TDG_OK && handled && !ho.active) {
-            // the whole file went through the device
-            if (tdg::utf8_finish(u8) >= 0)
-                drc = fail(ctx, TDG_ERR_UTF8, "position " + std::to_string(tdg::utf8_finish(u8)) + ": unexpected end of data in " + path);
-            if (drc == TDG_OK) drc = end_file_impl(ctx, reads_limit);
-        }
-        if (drc != TDG_OK || (handled && !ho.active)) {
-            if (drc != TDG_OK) ctx->carry_len = 0;
-            cudaStreamSynchronize(ctx->copy_stream);
-            cudaStreamSynchronize(ctx->stream);
-            if (drc == TDG_OK && totals) drc = tdg_file_totals(ctx, totals);
-            return drc;
-        }
+        at_eof = handled && !ho.active;                      // the whole file went through the device
     }
-    if (!reader) reader = start_reader(ctx, path, gz != 0, chunk, set, ho.active ? &ho : nullptr);
+    // the host feeder: from the start, or where the device feed handed over (none when that feed took the whole file or failed)
+    if (!reader && result == TDG_OK && !at_eof) reader = start_reader(ctx, path, gz != 0, chunk, set, ho.active ? &ho : nullptr);
 
-    FileReader &fr = *reader;
     const bool fdebug = getenv("TDG_FILE_DEBUG") != nullptr;
     const auto ft0 = std::chrono::steady_clock::now();
     double ms_wait = 0, ms_submit = 0;
     int bi = 0;
-    int result = TDG_OK;
     // the read with index maxreads-1 is line 4*maxreads-3: everything up to line end number
     // 4*maxreads-2 is needed, nothing beyond it is looked at (LimitState)
-    bool at_eof = false;
-    for (;;) {
+    while (reader) {
+        FileReader &fr = *reader;
         FileReader::Buf &b = fr.bufs[bi];
         const auto fw0 = std::chrono::steady_clock::now();
         {
@@ -1458,7 +1446,7 @@ int tdg_gz_inflate_host(tdg_ctx *ctx, const char *path, void *dst, size_t cap, u
     GzStats st;
     bool handled = false;
     size_t carry = 0;
-    rc = gz_device_feed(ctx, path, sink, handled, ho, carry, &st, nullptr);
+    rc = gz_device_feed(ctx, path, sink, handled, ho, carry, st, nullptr);
     if (rc) return rc;
     if (info) {
         info[0] = st.rounds;

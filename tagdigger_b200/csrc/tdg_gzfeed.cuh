@@ -164,236 +164,495 @@ int gz_upload(tdg_ctx *ctx, const GzMap &map, const char *path, int threads, int
     return TDG_OK;
 }
 
-// BGZF (bgzip): gzip members of at most 64 KiB of text that carry their compressed size in a 'BC'
+using GzClock = std::chrono::steady_clock;
+double gz_ms(GzClock::time_point a, GzClock::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); }
+
+// One device feed of one file: what its rounds share.  A round ends with its text at the sink.  Before
+// that, TDG_ERR_NOMEM (a buffer that cannot be had) and TDG_STOP_ROUND (the sink does not want the text)
+// are not the file's fault: the host feeder continues at the state the round began in (gz_device_feed).
+struct GzFeed {
+    tdg_ctx *ctx;
+    const char *path;
+    GzSink &sink;
+    size_t &carry;
+    GzStats &stats;
+    tdg::Utf8State *u8;
+    GzMap map;
+    uint32_t max_chunks = 0;
+    size_t fixed_chunk = 0;
+    uint32_t fixed_cap = 0;
+    bool debug = false;
+    int threads = 0;
+    int up_i = 0;                // the pinned buffer gz_upload fills next
+    bool sunk = false;           // the sink has had the round's text: a failure from here on is the call's
+    bool done = false;           // the device fed the whole file
+    bool handover = false;       // the host feeder continues at the position below
+    // a stream: where it stands, and the next round's bytes when they were read ahead
+    tdg::gzc::Stream st;
+    int cur = 0;                 // which compressed buffer the round reads
+    bool pre_valid = false;      // the other one holds [pre_off, pre_end) of the file
+    size_t pre_off = 0, pre_end = 0;
+    // BGZF: the next member, and the bytes of text in front of it
+    size_t off = 0;
+    uint64_t delivered = 0;
+
+    int upload(int which, size_t from, size_t end, cudaStream_t stream) { return gz_upload(ctx, map, path, threads, up_i, which, from, end, stream); }
+    int to_sink(uint64_t text_len)
+    {
+        sunk = true;
+        return sink.text(ctx, (uint8_t *)ctx->gz_text.p, carry, (size_t)text_len);
+    }
+};
+
+// what gz_scan and gz_decode read of a round (nb compressed bytes at `in`) and where the lanes put their tokens and reports
+tdg::gzd::RoundArgs gz_round_args(tdg_ctx *ctx, const void *in, size_t nb, uint32_t nchunks, uint32_t symcap, uint32_t tokcap)
+{
+    using namespace tdg;
+    gzd::RoundArgs a;
+    memset(&a, 0, sizeof(a));
+    a.in = (const uint32_t *)in;
+    a.nwords = (nb + 3) / 4;
+    a.in_bits = (uint64_t)nb * 8;
+    a.nchunks = nchunks;
+    a.symcap = symcap;
+    a.tokcap = tokcap;
+    a.syms = (uint16_t *)ctx->gz_syms.p;
+    a.meta = (gzl::Meta *)ctx->gz_meta.p;
+    a.cold = (uint16_t *)ctx->gz_cold.p;
+    return a;
+}
+
+// ---- the text stage: the steps both formats run alike, from the tokens of a round's chunks (or members) to the sink
+
+// gz_text[carry ..) must take text_len more bytes (and the counting kernel's tiles and halo); the carried bytes stay in front
+int gz_text_room(tdg_ctx *ctx, size_t carry, uint64_t text_len)
+{
+    const size_t need = round_up(carry + text_len, TDG_TILE_BYTES) + TDG_HALO_BYTES + 64;
+    if (need <= ctx->gz_text.cap) return TDG_OK;
+    int rc;
+    if (carry) {
+        if ((rc = grow(ctx, ctx->gz_carry, carry, false))) return rc;
+        CK(cudaMemcpyAsync(ctx->gz_carry.p, ctx->gz_text.p, carry, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    if ((rc = grow(ctx, ctx->gz_text, need, false))) return rc;
+    if (carry) CK(cudaMemcpyAsync(ctx->gz_text.p, ctx->gz_carry.p, carry, cudaMemcpyDeviceToDevice, ctx->stream));
+    return TDG_OK;
+}
+
+// tokens -> symbols: the ntok[k] tokens of chunk k in gz_syms (tokcap apart) become its symbols in gz_sym2 (symcap apart)
+int gz_expand_tokens(tdg_ctx *ctx, const std::vector<uint32_t> &ntok, uint32_t tokcap, uint32_t symcap)
+{
+    using namespace tdg;
+    CK(cudaMemcpyAsync(ctx->gz_ntok.p, ntok.data(), ntok.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));      // (ntok is the caller's)
+    gzd::ExpandArgs ea;
+    ea.tok = (uint16_t *)ctx->gz_syms.p;
+    ea.syms = (uint16_t *)ctx->gz_sym2.p;
+    ea.tokcap = tokcap;
+    ea.symcap = symcap;
+    ea.ntok = (const uint32_t *)ctx->gz_ntok.p;
+    ea.accepted = (uint32_t)ntok.size();
+    gzd::gz_expand<<<(ea.accepted + gzd::EXP_WARPS - 1) / gzd::EXP_WARPS, gzd::EXP_WARPS * 32, 0, ctx->stream>>>(ea);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    return TDG_OK;
+}
+
+// symbols -> the round's text at gz_text + carry.  gz_crc gets the raw CRC-32 of each of its `pieces` pieces and,
+// behind them, a flag with the high bit of every byte.
+int gz_resolve_text(tdg_ctx *ctx, uint32_t symcap, const uint64_t *text_off, uint32_t accepted, size_t carry, uint64_t text_len,
+                    uint32_t pieces)
+{
+    using namespace tdg;
+    uint32_t *d_flag = (uint32_t *)ctx->gz_crc.p + pieces;
+    CK(cudaMemsetAsync(d_flag, 0, 4, ctx->stream));
+    gzd::ResArgs ra;
+    ra.syms = (const uint16_t *)ctx->gz_sym2.p;
+    ra.symcap = symcap;
+    ra.text_off = text_off;
+    ra.accepted = accepted;
+    ra.ptrs = (const uint32_t *)ctx->gz_windows.p;
+    ra.text = (uint8_t *)ctx->gz_text.p + carry;
+    ra.text_len = text_len;
+    ra.crc = (uint32_t *)ctx->gz_crc.p;
+    ra.flag = d_flag;
+    ra.table = (const uint32_t *)((uint8_t *)ctx->gz_tabs.p + 512);
+    for (int j = 0; j < 8; j++) ra.op[j] = ctx->gz_op[j];
+    gzd::gz_resolve<<<pieces, gzd::RES_THREADS, 0, ctx->stream>>>(ra);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    return TDG_OK;
+}
+
+// text mode: bytes >= 0x80 (high_flag: the resolve kernel saw one) must form valid UTF-8 (open(f, 'rt'))
+int gz_check_utf8(GzFeed &f, uint32_t high_flag, uint64_t text_len)
+{
+    tdg_ctx *ctx = f.ctx;
+    if (!f.u8) return TDG_OK;
+    if ((high_flag & 0x80u) || f.u8->need) {
+        std::vector<uint8_t> host(text_len);
+        CK(cudaMemcpy(host.data(), (uint8_t *)ctx->gz_text.p + f.carry, text_len, cudaMemcpyDeviceToHost));
+        long long bad = tdg::utf8_feed(*f.u8, host.data(), host.size());
+        if (bad >= 0) return fail(ctx, TDG_ERR_UTF8, "position " + std::to_string(bad) + ": invalid UTF-8 in " + f.path);
+    } else {
+        f.u8->offset += text_len;
+    }
+    return TDG_OK;
+}
+
+// A round of BGZF (bgzip): gzip members of at most 64 KiB of text that carry their compressed size in a 'BC'
 // extra field -- every member is its own deflate stream, so nothing is speculative here: the host
 // walks the member headers, one lane inflates one member from its first bit to its final block
 // (gz_decode in member mode), gz_expand and gz_resolve lay the text out, gz_member_crc takes every
 // member's CRC-32, and the host holds length, end position and CRC against the member's trailer.
 // A member that fails any of that is what the host feeder calls a corrupt BGZF member; a member
 // header that is not BGZF (or a truncated one) ends the device feed, the host feeder continues there.
-int gz_device_feed_bgzf(tdg_ctx *ctx, const char *path, const GzMap &map, GzSink &sink, GzHandover &ho, size_t &carry, GzStats *stats,
-                        tdg::Utf8State *u8)
+int gz_bgzf_round(GzFeed &f)
 {
     using namespace tdg;
     struct Member {
         size_t off;
         uint32_t hlen, csize, isize, crc;
     };
-    int rc = gz_tables(ctx);
-    if (rc) return rc;
-    rc = ensure_slots(ctx);
-    if (rc) return rc;
-    uint32_t max_chunks = (uint32_t)ctx->sm_count * gzd::DEC_THREADS;
-    if (const char *e = getenv("TDG_GZDEV_MAXCHUNKS")) max_chunks = (uint32_t)std::max(1, atoi(e));
-    const bool debug = getenv("TDG_GZDEV_DEBUG") != nullptr;
-    const int threads = gz_io_threads();
+    tdg_ctx *ctx = f.ctx;
+    const GzMap &map = f.map;
     const uint32_t symcap = 65536 + 512, tokcap = 65536 + 64;
-    uint8_t *d_tabs = (uint8_t *)ctx->gz_tabs.p;
-    uint32_t op[5];
-    for (int j = 0; j < 5; j++) op[j] = (uint32_t)crc32_combine_gen((z_off_t)(2048u << j));
-    int up_i = 0;
-    carry = 0;
-    size_t off = 0;
-    uint64_t delivered = 0;
-    bool foreign = false, oom = false;         // oom: a buffer could not be had -- the host feeder continues at this round's first member
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-        return std::chrono::duration<double, std::milli>(b - a).count();
-    };
-    while (off < map.n && !foreign) {
-        // ---- the members of this round
-        auto t0 = now();
-        std::vector<Member> mem;
-        size_t end = off;
-        while (end < map.n && mem.size() < max_chunks && end - off < ((size_t)1 << 30)) {
-            uint32_t csize = 0, hlen = 0;
-            if (!Feeder::bgzf_member(map.p + end, std::min<size_t>(map.n - end, 1024), csize, hlen) || end + csize > map.n) {
-                foreign = true;
-                break;
-            }
-            Member m;
-            m.off = end;
-            m.hlen = hlen;
-            m.csize = csize;
-            memcpy(&m.crc, map.p + end + csize - 8, 4);
-            memcpy(&m.isize, map.p + end + csize - 4, 4);
-            if (m.isize > 65536) {
-                foreign = true;
-                break;
-            }
-            mem.push_back(m);
-            end += csize;
+    int rc;
+    // ---- the members of this round
+    auto t0 = GzClock::now();
+    std::vector<Member> mem;
+    size_t end = f.off;
+    while (end < map.n && mem.size() < f.max_chunks && end - f.off < ((size_t)1 << 30)) {
+        uint32_t csize = 0, hlen = 0;
+        if (!Feeder::bgzf_member(map.p + end, std::min<size_t>(map.n - end, 1024), csize, hlen) || end + csize > map.n) {
+            f.handover = true;
+            break;
         }
-        if (mem.empty()) break;
-        const uint32_t n = (uint32_t)mem.size();
-        const size_t nb = end - off, nwords = (nb + 3) / 4;
-        if ((rc = gz_upload(ctx, map, path, threads, up_i, 0, off, end, ctx->stream))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        if ((rc = grow(ctx, ctx->gz_syms, (size_t)n * tokcap * 2, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        if ((rc = grow(ctx, ctx->gz_sym2, (size_t)n * symcap * 2, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        if ((rc = grow(ctx, ctx->gz_meta, (size_t)n * sizeof(gzl::Meta), false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        if ((rc = grow(ctx, ctx->gz_hmeta, (size_t)n * sizeof(gzl::Meta), true))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        if ((rc = grow(ctx, ctx->gz_cold, (size_t)(n + 8) * gzl::COLD_U16 * 2, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        if ((rc = grow(ctx, ctx->gz_offs, ((size_t)n * 3 + 1) * 8, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }       // [n] start bits, [n] end bits, [n + 1] text offsets
-        if ((rc = grow(ctx, ctx->gz_lens, (size_t)n * 4, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        if ((rc = grow(ctx, ctx->gz_ntok, (size_t)n * 4, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-        std::vector<uint64_t> bits(2 * (size_t)n), text_off(n + 1, 0);
-        std::vector<uint32_t> lens(n);
-        for (uint32_t k = 0; k < n; k++) {
-            bits[k] = (uint64_t)(mem[k].off + mem[k].hlen - off) * 8;
-            bits[n + k] = (uint64_t)(mem[k].off + mem[k].csize - 8 - off) * 8;
-            lens[k] = mem[k].isize;
-            text_off[k + 1] = text_off[k] + mem[k].isize;
+        Member m;
+        m.off = end;
+        m.hlen = hlen;
+        m.csize = csize;
+        memcpy(&m.crc, map.p + end + csize - 8, 4);
+        memcpy(&m.isize, map.p + end + csize - 4, 4);
+        if (m.isize > 65536) {
+            f.handover = true;
+            break;
         }
-        const uint64_t text_len = text_off[n];
-        uint64_t *d_bits = (uint64_t *)ctx->gz_offs.p;
-        uint64_t *d_toff = d_bits + 2 * (size_t)n;
-        CK(cudaMemcpyAsync(d_bits, bits.data(), bits.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(d_toff, text_off.data(), text_off.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(ctx->gz_lens.p, lens.data(), lens.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-        gzd::RoundArgs a;
-        memset(&a, 0, sizeof(a));
-        a.in = (const uint32_t *)ctx->gz_comp.p;
-        a.nwords = nwords;
-        a.in_bits = (uint64_t)nb * 8;
-        a.nchunks = n;
-        a.symcap = symcap;
-        a.tokcap = tokcap;
-        a.syms = (uint16_t *)ctx->gz_syms.p;
-        a.meta = (gzl::Meta *)ctx->gz_meta.p;
-        a.cold = (uint16_t *)ctx->gz_cold.p;
-        a.m_start = d_bits;
-        a.m_end = d_bits + n;
-        gzd::gz_decode<<<(n + gzd::DEC_THREADS - 1) / gzd::DEC_THREADS, gzd::DEC_THREADS, gzd::DEC_SMEM, ctx->stream>>>(a);
+        mem.push_back(m);
+        end += csize;
+    }
+    if (mem.empty()) return TDG_OK;
+    const uint32_t n = (uint32_t)mem.size();
+    const size_t nb = end - f.off;
+    if ((rc = f.upload(0, f.off, end, ctx->stream))) return rc;
+    if ((rc = grow(ctx, ctx->gz_syms, (size_t)n * tokcap * 2, false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_sym2, (size_t)n * symcap * 2, false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_meta, (size_t)n * sizeof(gzl::Meta), false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_hmeta, (size_t)n * sizeof(gzl::Meta), true))) return rc;
+    if ((rc = grow(ctx, ctx->gz_cold, (size_t)(n + 8) * gzl::COLD_U16 * 2, false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_offs, ((size_t)n * 3 + 1) * 8, false))) return rc;       // [n] start bits, [n] end bits, [n + 1] text offsets
+    if ((rc = grow(ctx, ctx->gz_lens, (size_t)n * 4, false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_ntok, (size_t)n * 4, false))) return rc;
+    std::vector<uint64_t> bits(2 * (size_t)n), text_off(n + 1, 0);
+    std::vector<uint32_t> lens(n);
+    for (uint32_t k = 0; k < n; k++) {
+        bits[k] = (uint64_t)(mem[k].off + mem[k].hlen - f.off) * 8;
+        bits[n + k] = (uint64_t)(mem[k].off + mem[k].csize - 8 - f.off) * 8;
+        lens[k] = mem[k].isize;
+        text_off[k + 1] = text_off[k] + mem[k].isize;
+    }
+    const uint64_t text_len = text_off[n];
+    uint64_t *d_bits = (uint64_t *)ctx->gz_offs.p;
+    uint64_t *d_toff = d_bits + 2 * (size_t)n;
+    CK(cudaMemcpyAsync(d_bits, bits.data(), bits.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_toff, text_off.data(), text_off.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->gz_lens.p, lens.data(), lens.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    gzd::RoundArgs a = gz_round_args(ctx, ctx->gz_comp.p, nb, n, symcap, tokcap);
+    a.m_start = d_bits;
+    a.m_end = d_bits + n;
+    gzd::gz_decode<<<(n + gzd::DEC_THREADS - 1) / gzd::DEC_THREADS, gzd::DEC_THREADS, gzd::DEC_SMEM, ctx->stream>>>(a);
+    CK(cudaGetLastError());
+    gzl::Meta *meta = (gzl::Meta *)ctx->gz_hmeta.p;
+    CK(cudaMemcpyAsync(meta, ctx->gz_meta.p, (size_t)n * sizeof(gzl::Meta), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    auto t1 = GzClock::now();
+    // ---- every member must have ended with its final block, right in front of its trailer, at its length
+    std::vector<uint32_t> ntok(n);
+    for (uint32_t k = 0; k < n; k++) {
+        const gzl::Meta &c = meta[k];
+        const bool good = c.flags == (gzl::F_FOUND | gzl::F_FINAL) && c.out_len == mem[k].isize && (c.end_bit + 7) / 8 * 8 == bits[n + k];
+        if (!good) return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + f.path + ": corrupt BGZF member");
+        ntok[k] = c.ntok;
+    }
+    if (text_len) {
+        const int go = f.sink.may_take(ctx, (size_t)text_len);
+        if (go < 0) return go;
+        if (go == 0) return TDG_STOP_ROUND;
+        const uint32_t pieces = (uint32_t)((text_len + gzd::PIECE - 1) / gzd::PIECE);
+        if ((rc = grow(ctx, ctx->gz_crc, ((size_t)pieces + n) * 4 + 16, false))) return rc;
+        if ((rc = grow(ctx, ctx->gz_hcrc, ((size_t)n + 1) * 4 + 16, true))) return rc;
+        if ((rc = grow(ctx, ctx->gz_windows, gzl::WIN * 4, false))) return rc;          // (never read: a member has no history before it)
+        if ((rc = gz_text_room(ctx, f.carry, text_len))) return rc;
+        if ((rc = gz_expand_tokens(ctx, ntok, tokcap, symcap))) return rc;
+        if ((rc = gz_resolve_text(ctx, symcap, d_toff, n, f.carry, text_len, pieces))) return rc;
+        uint32_t *d_flag = (uint32_t *)ctx->gz_crc.p + pieces;
+        gzd::MemberCrcArgs ca;
+        ca.syms = (const uint16_t *)ctx->gz_sym2.p;
+        ca.stride = symcap;
+        ca.lens = (const uint32_t *)ctx->gz_lens.p;
+        ca.n = n;
+        ca.crc = d_flag + 1;
+        ca.table = (const uint32_t *)((uint8_t *)ctx->gz_tabs.p + 512);
+        for (int j = 0; j < 5; j++) ca.op[j] = (uint32_t)crc32_combine_gen((z_off_t)(2048u << j));
+        gzd::gz_member_crc<<<(n + 7) / 8, 256, 0, ctx->stream>>>(ca);
         CK(cudaGetLastError());
-        gzl::Meta *meta = (gzl::Meta *)ctx->gz_hmeta.p;
-        CK(cudaMemcpyAsync(meta, ctx->gz_meta.p, (size_t)n * sizeof(gzl::Meta), cudaMemcpyDeviceToHost, ctx->stream));
+        ctx->launches += 2;                  // gz_member_crc and gz_decode: a round that stops before its text kernels counts none
+        uint32_t *h = (uint32_t *)ctx->gz_hcrc.p;                                       // [0] the high-bit flag, [1..n] the members' CRCs
+        CK(cudaMemcpyAsync(h, d_flag, ((size_t)n + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
-        auto t1 = now();
-        // ---- every member must have ended with its final block, right in front of its trailer, at its length
-        std::vector<uint32_t> ntok(n);
-        for (uint32_t k = 0; k < n; k++) {
-            const gzl::Meta &c = meta[k];
-            const bool good = c.flags == (gzl::F_FOUND | gzl::F_FINAL) && c.out_len == mem[k].isize && (c.end_bit + 7) / 8 * 8 == bits[n + k];
-            if (!good) return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + path + ": corrupt BGZF member");
-            ntok[k] = c.ntok;
-        }
-        if (text_len) {
-            const int go = sink.may_take(ctx, (size_t)text_len);
-            if (go < 0) return go;
-            if (go == 0) {                                   // a read limit within reach: the host feeder continues at this round's first member
-                foreign = true;
-                break;
-            }
-        }
-        if (text_len) {
-            const uint32_t pieces = (uint32_t)((text_len + gzd::PIECE - 1) / gzd::PIECE);
-            if ((rc = grow(ctx, ctx->gz_crc, ((size_t)pieces + n) * 4 + 16, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-            if ((rc = grow(ctx, ctx->gz_hcrc, ((size_t)n + 1) * 4 + 16, true))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-            if ((rc = grow(ctx, ctx->gz_windows, gzl::WIN * 4, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }          // (never read: a member has no history before it)
-            const size_t need = round_up(carry + text_len, TDG_TILE_BYTES) + TDG_HALO_BYTES + 64;
-            if (need > ctx->gz_text.cap) {
-                if (carry) {
-                    if ((rc = grow(ctx, ctx->gz_carry, carry, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-                    CK(cudaMemcpyAsync(ctx->gz_carry.p, ctx->gz_text.p, carry, cudaMemcpyDeviceToDevice, ctx->stream));
-                }
-                if ((rc = grow(ctx, ctx->gz_text, need, false))) { if (rc == TDG_ERR_NOMEM) { oom = true; break; } return rc; }
-                if (carry) CK(cudaMemcpyAsync(ctx->gz_text.p, ctx->gz_carry.p, carry, cudaMemcpyDeviceToDevice, ctx->stream));
-            }
-            CK(cudaMemcpyAsync(ctx->gz_ntok.p, ntok.data(), ntok.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-            CK(cudaStreamSynchronize(ctx->stream));
-            gzd::ExpandArgs ea;
-            ea.tok = a.syms;
-            ea.syms = (uint16_t *)ctx->gz_sym2.p;
-            ea.tokcap = tokcap;
-            ea.symcap = symcap;
-            ea.ntok = (const uint32_t *)ctx->gz_ntok.p;
-            ea.accepted = n;
-            gzd::gz_expand<<<(n + gzd::EXP_WARPS - 1) / gzd::EXP_WARPS, gzd::EXP_WARPS * 32, 0, ctx->stream>>>(ea);
-            CK(cudaGetLastError());
-            uint32_t *d_piece_crc = (uint32_t *)ctx->gz_crc.p;
-            uint32_t *d_flag = d_piece_crc + pieces;
-            uint32_t *d_mcrc = d_flag + 1;
-            CK(cudaMemsetAsync(d_flag, 0, 4, ctx->stream));
-            gzd::ResArgs ra;
-            ra.syms = (const uint16_t *)ctx->gz_sym2.p;
-            ra.symcap = symcap;
-            ra.text_off = d_toff;
-            ra.accepted = n;
-            ra.ptrs = (const uint32_t *)ctx->gz_windows.p;
-            ra.text = (uint8_t *)ctx->gz_text.p + carry;
-            ra.text_len = text_len;
-            ra.crc = d_piece_crc;
-            ra.flag = d_flag;
-            ra.table = (const uint32_t *)(d_tabs + 512);
-            for (int j = 0; j < 8; j++) ra.op[j] = ctx->gz_op[j];
-            gzd::gz_resolve<<<pieces, gzd::RES_THREADS, 0, ctx->stream>>>(ra);
-            CK(cudaGetLastError());
-            gzd::MemberCrcArgs ca;
-            ca.syms = (const uint16_t *)ctx->gz_sym2.p;
-            ca.stride = symcap;
-            ca.lens = (const uint32_t *)ctx->gz_lens.p;
-            ca.n = n;
-            ca.crc = d_mcrc;
-            ca.table = (const uint32_t *)(d_tabs + 512);
-            for (int j = 0; j < 5; j++) ca.op[j] = op[j];
-            gzd::gz_member_crc<<<(n + 7) / 8, 256, 0, ctx->stream>>>(ca);
-            CK(cudaGetLastError());
-            ctx->launches += 4;
-            uint32_t *h = (uint32_t *)ctx->gz_hcrc.p;                                       // [0] the high-bit flag, [1..n] the members' CRCs
-            CK(cudaMemcpyAsync(h, d_flag, ((size_t)n + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaStreamSynchronize(ctx->stream));
-            for (uint32_t k = 0; k < n; k++)
-                if (h[1 + k] != mem[k].crc) return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + path + ": corrupt BGZF member");
-            if (u8) {
-                if ((h[0] & 0x80u) || u8->need) {
-                    std::vector<uint8_t> host(text_len);
-                    CK(cudaMemcpy(host.data(), (uint8_t *)ctx->gz_text.p + carry, text_len, cudaMemcpyDeviceToHost));
-                    long long bad = tdg::utf8_feed(*u8, host.data(), host.size());
-                    if (bad >= 0) return fail(ctx, TDG_ERR_UTF8, "position " + std::to_string(bad) + ": invalid UTF-8 in " + path);
-                } else {
-                    u8->offset += text_len;
-                }
-            }
-            rc = sink.text(ctx, (uint8_t *)ctx->gz_text.p, carry, (size_t)text_len);
-            if (rc) return rc;
-        } else {
-            ctx->launches += 1;
-        }
-        delivered += text_len;
-        off = end;
-        if (stats) {
-            stats->rounds++;
-            stats->chunks += n;
-            stats->accepted += n;
-            stats->ms_decode += ms(t0, t1);
-            stats->ms_resolve += ms(t1, now());
-        }
-        if (debug)
-            fprintf(stderr, "gzdev BGZF round: %u members, %zu compressed bytes, %llu bytes of text; upload + decode %.1f, rest %.1f ms\n", n, nb,
-                    (unsigned long long)text_len, ms(t0, t1), ms(t1, now()));
+        for (uint32_t k = 0; k < n; k++)
+            if (h[1 + k] != mem[k].crc) return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + f.path + ": corrupt BGZF member");
+        if ((rc = gz_check_utf8(f, h[0], text_len))) return rc;
+        if ((rc = f.to_sink(text_len))) return rc;
+    } else {
+        ctx->launches++;                                                                 // gz_decode
     }
-    if (foreign || oom || off < map.n) {
-        // something that is not a BGZF member follows (or the file stops inside one): the host feeder's to judge
-        ho.active = true;
-        ho.bgzf = true;
-        ho.bgzf_off = off;
-        ho.delivered = delivered;
-        ho.why = oom ? "device memory" : "not a BGZF member";
-    }
+    f.delivered += text_len;
+    f.off = end;
+    f.done = f.off == map.n;
+    f.stats.rounds++;
+    f.stats.chunks += n;
+    f.stats.accepted += n;
+    f.stats.ms_decode += gz_ms(t0, t1);
+    f.stats.ms_resolve += gz_ms(t1, GzClock::now());
+    if (f.debug)
+        fprintf(stderr, "gzdev BGZF round: %u members, %zu compressed bytes, %llu bytes of text; upload + decode %.1f, rest %.1f ms\n", n, nb,
+                (unsigned long long)text_len, gz_ms(t0, t1), gz_ms(t1, GzClock::now()));
     return TDG_OK;
 }
 
-// Inflates `path` (an ordinary gzip file) on the device round by round and hands every round's
+// A round of an ordinary gzip stream: plan -> upload (or the bytes read ahead in the round before) -> scan ->
+// decode -> which chunks continue the stream (chain) -> the text stage, with the windows passes and the CRC of
+// the text, which st.advance holds against the member's trailer.
+int gz_stream_round(GzFeed &f)
+{
+    using namespace tdg;
+    tdg_ctx *ctx = f.ctx;
+    gzc::Stream &st = f.st;
+    const size_t file_n = f.map.n;
+    const uint32_t max_chunks = std::min<uint32_t>(f.max_chunks, 65000);             // gz_ptr_*: a chunk index has 16 bits
+    uint8_t *d_tabs = (uint8_t *)ctx->gz_tabs.p;
+    uint8_t *d_window = d_tabs + 512 + 1024;
+    int rc;
+    // Chunk size, chosen per round from what is left of the file: every lane gets work when there is enough of
+    // it, in steps of 16 KiB between 32 and 128 KiB (a chunk should hold a block start: zlib's blocks are
+    // 10 - 30 KB of compressed data).  What a lane may produce: symbols up to 8 x its chunk (and room for a
+    // large block), token slots up to 3 x its chunk (literal codes of 4 bits and more: two slots per compressed
+    // byte); a chunk that needs more ends the device feed (the host reader takes over).
+    size_t chunk = f.fixed_chunk;
+    if (!chunk) {
+        const size_t left = file_n - (size_t)(st.pos_bit >> 3);
+        chunk = round_up((left + max_chunks - 1) / max_chunks, (size_t)16 << 10);
+        chunk = std::min<size_t>(std::max<size_t>(chunk, (size_t)32 << 10), (size_t)128 << 10);
+    }
+    const uint32_t symcap = f.fixed_cap ? f.fixed_cap : (uint32_t)std::max<size_t>(8 * chunk, (size_t)256 << 10);
+    const uint32_t tokcap = f.fixed_cap ? f.fixed_cap : (uint32_t)std::max<size_t>(3 * chunk, (size_t)128 << 10);
+    const gzc::Round r = st.plan(chunk, max_chunks);
+    const size_t nb = r.buf_end - r.buf_off;
+    // ---- the round's compressed bytes: file -> pinned pieces -> device (or already there: see below)
+    auto t0 = GzClock::now();
+    const bool prefetched = f.pre_valid && f.pre_off <= r.buf_off && f.pre_end >= r.buf_end && (r.buf_off - f.pre_off) % 16 == 0;
+    size_t comp_skip = 0;                                // where the round's bytes begin in the buffer
+    if (prefetched) {
+        f.cur ^= 1;                                      // the bytes sit in the other buffer: wait for their copies
+        comp_skip = r.buf_off - f.pre_off;
+        CK(cudaStreamWaitEvent(ctx->stream, ctx->gz_pre, 0));
+    } else {
+        rc = f.upload(f.cur, r.buf_off, r.buf_end, ctx->stream);
+        if (rc) return rc;
+    }
+    f.pre_valid = false;
+    Buf &comp = f.cur ? ctx->gz_comp2 : ctx->gz_comp;
+    if ((rc = grow(ctx, ctx->gz_syms, (size_t)r.nchunks * tokcap * 2, false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_meta, (size_t)r.nchunks * sizeof(gzl::Meta), false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_cand, (size_t)r.nchunks * gzd::MAXC * 4, false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_ncand, (size_t)r.nchunks * 4, false))) return rc;
+    if ((rc = grow(ctx, ctx->gz_hmeta, (size_t)r.nchunks * sizeof(gzl::Meta), true))) return rc;
+    if ((rc = grow(ctx, ctx->gz_cold, (size_t)(r.nchunks + 8) * gzl::COLD_U16 * 2, false))) return rc;
+    if (f.debug) CK(cudaStreamSynchronize(ctx->stream));
+    auto t1 = GzClock::now();
+    // ---- scan + decode
+    gzd::RoundArgs a = gz_round_args(ctx, (const uint8_t *)comp.p + comp_skip, nb, r.nchunks, symcap, tokcap);      // (m_start / m_end stay null: this is one stream, not BGZF members)
+    a.chunk_bytes = chunk;
+    a.file_left = file_n - r.grid;
+    a.pos_rel = r.pos_bit - (uint64_t)r.grid * 8;
+    a.base_bit = (uint64_t)r.grid * 8;
+    a.hist = r.hist;
+    a.cand = (uint32_t *)ctx->gz_cand.p;
+    a.ncand = (uint32_t *)ctx->gz_ncand.p;
+    a.kraft3 = d_tabs;
+    CK(cudaMemsetAsync(ctx->gz_ncand.p, 0, (size_t)r.nchunks * 4, ctx->stream));
+    if (r.nchunks > 1) {
+        const unsigned g = (r.nchunks - 1 + gzd::SCAN_WARPS - 1) / gzd::SCAN_WARPS;
+        gzd::gz_scan<<<g, gzd::SCAN_WARPS * 32, gzd::SCAN_SMEM, ctx->stream>>>(a);
+        CK(cudaGetLastError());
+        ctx->launches++;
+    }
+    if (f.debug) CK(cudaStreamSynchronize(ctx->stream));
+    auto t2 = GzClock::now();
+    gzd::gz_decode<<<(r.nchunks + gzd::DEC_THREADS - 1) / gzd::DEC_THREADS, gzd::DEC_THREADS, gzd::DEC_SMEM, ctx->stream>>>(a);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    gzl::Meta *meta = (gzl::Meta *)ctx->gz_hmeta.p;
+    CK(cudaMemcpyAsync(meta, ctx->gz_meta.p, (size_t)r.nchunks * sizeof(gzl::Meta), cudaMemcpyDeviceToHost, ctx->stream));
+    // While the lanes inflate, this thread reads the bytes the NEXT round will most likely ask
+    // for (every chunk accepted: its grid starts where this one's ends) and sends them to the
+    // other buffer on the copy stream.
+    double ms_prefetch = 0;
+    const auto tp0 = GzClock::now();
+    if (r.grid + (size_t)r.nchunks * chunk < file_n && r.nchunks == max_chunks) {
+        f.pre_off = r.grid + (size_t)r.nchunks * chunk;  // (the next round's grid starts here or, with smaller chunks, a little further on)
+        f.pre_end = std::min(file_n, f.pre_off + ((size_t)max_chunks + 2) * chunk);
+        rc = f.upload(f.cur ^ 1, f.pre_off, f.pre_end, ctx->copy_stream);
+        if (rc) return rc;
+        CK(cudaEventRecord(ctx->gz_pre, ctx->copy_stream));
+        f.pre_valid = true;
+        ms_prefetch = gz_ms(tp0, GzClock::now());
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    auto t3 = GzClock::now();
+    // ---- which chunks continue the stream
+    const gzc::Outcome o = st.chain(r, meta, symcap);
+    uint64_t text_len = o.text_off.back();
+    uint32_t text_crc = 0;
+    auto t4 = t3, t5 = t3;
+    if (o.accepted && text_len) {
+        const int go = f.sink.may_take(ctx, (size_t)text_len);
+        if (go < 0) return go;
+        if (go == 0) return TDG_STOP_ROUND;
+        const uint32_t pieces = (uint32_t)((text_len + gzd::PIECE - 1) / gzd::PIECE);
+        if ((rc = grow(ctx, ctx->gz_windows, ((size_t)o.accepted + 1) * (gzl::WIN * 4 + 1), false))) return rc;
+        if ((rc = grow(ctx, ctx->gz_lens, (size_t)o.accepted * 4, false))) return rc;
+        if ((rc = grow(ctx, ctx->gz_offs, ((size_t)o.accepted + 1) * 8, false))) return rc;
+        if ((rc = grow(ctx, ctx->gz_crc, ((size_t)pieces + pieces / 256 + 2) * 4 + 16, false))) return rc;
+        if ((rc = grow(ctx, ctx->gz_hcrc, ((size_t)pieces / 256 + 4) * 4 + 16, true))) return rc;
+        if ((rc = gz_text_room(ctx, f.carry, text_len))) return rc;
+        CK(cudaMemcpyAsync(ctx->gz_lens.p, o.lens.data(), o.lens.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+        // tokens -> symbols (accepted chunks only)
+        // the symbols: as many per chunk as the largest accepted chunk has
+        uint32_t stride = 64;
+        for (uint32_t len : o.lens) stride = std::max(stride, len);
+        stride = (stride + 63u) & ~63u;
+        if ((rc = grow(ctx, ctx->gz_sym2, (size_t)o.accepted * stride * 2, false))) return rc;
+        if ((rc = grow(ctx, ctx->gz_ntok, (size_t)o.accepted * 4, false))) return rc;
+        std::vector<uint32_t> ntok(o.accepted);
+        for (uint32_t k = 0; k < o.accepted; k++) ntok[k] = o.lens[k] ? meta[k].ntok : 0u;
+        for (const gzc::Repair &rp : o.repairs) ntok[rp.chunk] = 0;          // the host made these chunks' symbols
+        if ((rc = gz_expand_tokens(ctx, ntok, tokcap, stride))) return rc;
+        for (const gzc::Repair &rp : o.repairs)
+            if (!rp.syms.empty())
+                CK(cudaMemcpyAsync((uint16_t *)ctx->gz_sym2.p + (size_t)rp.chunk * stride, rp.syms.data(), rp.syms.size() * 2,
+                                   cudaMemcpyHostToDevice, ctx->stream));
+        if (f.debug) {
+            CK(cudaStreamSynchronize(ctx->stream));
+            fprintf(stderr, "gzdev expand: %.1f ms, %zu chunks made by the host\n", gz_ms(t3, GzClock::now()), o.repairs.size());
+        }
+        CK(cudaMemcpyAsync(ctx->gz_offs.p, o.text_off.data(), o.text_off.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+        gzd::WinArgs w;
+        w.syms = (const uint16_t *)ctx->gz_sym2.p;
+        w.symcap = stride;
+        w.out_len = (const uint32_t *)ctx->gz_lens.p;
+        w.accepted = o.accepted;
+        w.window_in = d_window;
+        w.ptrs = (uint32_t *)ctx->gz_windows.p;
+        w.done = (uint8_t *)ctx->gz_windows.p + ((size_t)o.accepted + 1) * gzl::WIN * 4;
+        w.window_out = d_window;
+        gzd::gz_ptr_init<<<o.accepted + 1, gzd::WIN_THREADS, 0, ctx->stream>>>(w);
+        CK(cudaGetLastError());
+        uint32_t passes = 1;
+        while ((1u << (passes - 1)) < o.accepted + 1) passes++;          // chains are at most accepted + 1 long
+        for (uint32_t ps = 0; ps < passes; ps++) gzd::gz_ptr_jump<<<o.accepted, gzd::WIN_THREADS, 0, ctx->stream>>>(w);
+        CK(cudaGetLastError());
+        ctx->launches += 1 + passes;
+        if (f.debug) {
+            CK(cudaStreamSynchronize(ctx->stream));
+            fprintf(stderr, "gzdev windows: %u passes, %.1f ms\n", passes, gz_ms(t3, GzClock::now()));
+        }
+        if ((rc = gz_resolve_text(ctx, stride, (const uint64_t *)ctx->gz_offs.p, o.accepted, f.carry, text_len, pieces))) return rc;
+        // the window behind the last accepted chunk opens the next round
+        gzd::gz_ptr_take<<<8, gzd::WIN_THREADS, 0, ctx->stream>>>(w);
+        CK(cudaGetLastError());
+        ctx->launches++;
+        // the pieces' raw CRCs: 256 full pieces fold into one on the device, the host folds the rest
+        uint32_t *d_flag = (uint32_t *)ctx->gz_crc.p + pieces;
+        const uint32_t nfull = (uint32_t)(text_len / gzd::PIECE), groups = (nfull + 255) / 256;
+        uint32_t *d_group = d_flag + 1;
+        if (groups) {
+            gzd::CrcFoldArgs fa;
+            fa.piece = (const uint32_t *)ctx->gz_crc.p;
+            fa.nfull = nfull;
+            fa.group = d_group;
+            for (int j = 0; j < 8; j++) fa.op[j] = (uint32_t)crc32_combine_gen((z_off_t)((uint64_t)gzd::PIECE << j));
+            gzd::gz_crc_fold<<<groups, 256, 0, ctx->stream>>>(fa);
+            CK(cudaGetLastError());
+            ctx->launches++;
+        }
+        // host copy: [0] the high-bit flag, [1 .. groups] the group CRCs, [groups + 1] the last (partial) piece's
+        uint32_t *hcrc = (uint32_t *)ctx->gz_hcrc.p;
+        CK(cudaMemcpyAsync(hcrc, d_flag, ((size_t)groups + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        if (pieces > nfull)
+            CK(cudaMemcpyAsync(hcrc + groups + 1, (uint32_t *)ctx->gz_crc.p + nfull, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        t4 = GzClock::now();
+        // CRC-32 of the round's text from the raw CRCs
+        uLong raw = 0;
+        if (groups) {
+            const uLong op_group = crc32_combine_gen((z_off_t)((uint64_t)gzd::PIECE * 256));
+            for (uint32_t g = 0; g + 1 < groups; g++) raw = crc32_combine_op(raw, hcrc[1 + g], op_group);
+            const uint64_t last_group = (uint64_t)(nfull - (groups - 1) * 256u) * gzd::PIECE;
+            raw = crc32_combine_op(raw, hcrc[groups], crc32_combine_gen((z_off_t)last_group));
+        }
+        if (pieces > nfull) raw = crc32_combine_op(raw, hcrc[groups + 1], crc32_combine_gen((z_off_t)(text_len - (uint64_t)nfull * gzd::PIECE)));
+        text_crc = (uint32_t)(raw ^ crc32_combine_op(0xFFFFFFFFul, 0, crc32_combine_gen((z_off_t)text_len)) ^ 0xFFFFFFFFul);
+        if ((rc = gz_check_utf8(f, hcrc[0], text_len))) return rc;
+        t5 = GzClock::now();
+    }
+    if (!st.advance(r, o, text_len, text_crc))
+        return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + f.path + ": incorrect data check");
+    if (o.accepted && text_len && (rc = f.to_sink(text_len))) return rc;
+    auto t6 = GzClock::now();
+    f.done = st.eof;
+    f.handover = st.handover;
+    f.stats.rounds++;
+    f.stats.chunks += r.nchunks;
+    f.stats.accepted += o.accepted;
+    f.stats.ms_upload += gz_ms(t0, t1);
+    f.stats.ms_scan += gz_ms(t1, t2);
+    f.stats.ms_decode += gz_ms(t2, t3);
+    f.stats.ms_host += gz_ms(t4, t5);
+    f.stats.ms_resolve += gz_ms(t3, t4);
+    f.stats.ms_sink += gz_ms(t5, t6);
+    if (f.debug)
+        fprintf(stderr, "gzdev round: %u chunks of %zu KiB, %u accepted, %llu bytes of text; upload %.1f%s scan %.1f decode %.1f "
+                        "(host read the next round's bytes meanwhile: %.1f) expand+windows+resolve %.1f crc/utf8 %.1f sink %.1f ms%s%s\n",
+                r.nchunks, chunk >> 10, o.accepted, (unsigned long long)text_len, gz_ms(t0, t1), prefetched ? " (prefetched)" : "", gz_ms(t1, t2),
+                gz_ms(t2, t3), ms_prefetch, gz_ms(t3, t4), gz_ms(t4, t5),
+                gz_ms(t5, t6), st.handover ? "  -> host reader: " : "", st.handover ? st.why : "");
+    return TDG_OK;
+}
+
+// Inflates `path` (an ordinary gzip file or BGZF) on the device round by round and hands every round's
 // text to `sink`.  handled = false: nothing was done (a header this feed does not take: the host
 // feeder starts from the beginning).  Otherwise the text went to the sink up to the end of the
 // file, or up to the place `ho` describes (ho.active), where the host feeder continues.
-int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, GzHandover &ho, size_t &carry, GzStats *stats,
+int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, GzHandover &ho, size_t &carry, GzStats &stats,
                    tdg::Utf8State *u8)
 {
     using namespace tdg;
     handled = false;
     ho = GzHandover();
-    GzMap map;
+    GzFeed f{ctx, path, sink, carry, stats, u8};
+    GzMap &map = f.map;
     map.fd = ::open(path, O_RDONLY);
     if (map.fd < 0) return TDG_OK;                       // the host feeder reports it
     struct stat sb;
@@ -402,332 +661,46 @@ int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, 
     void *mp = mmap(nullptr, map.n, PROT_READ, MAP_PRIVATE, map.fd, 0);
     if (mp == MAP_FAILED) return TDG_OK;
     map.p = (const uint8_t *)mp;
-    if (tdg::Feeder::is_bgzf(map.p, std::min<size_t>(map.n, 1024))) {
-        handled = true;
-        return gz_device_feed_bgzf(ctx, path, map, sink, ho, carry, stats, u8);
-    }
-    gzc::Stream st;
-    if (!st.open(map.p, map.n)) return TDG_OK;
+    const bool bgzf = Feeder::is_bgzf(map.p, std::min<size_t>(map.n, 1024));
+    if (!bgzf && !f.st.open(map.p, map.n)) return TDG_OK;
     int rc = gz_tables(ctx);
     if (rc) return rc;
     rc = ensure_slots(ctx);
     if (rc) return rc;
-
-    uint32_t max_chunks = (uint32_t)ctx->sm_count * gzd::DEC_THREADS;          // one lane per chunk, one CTA per SM
-    if (const char *e = getenv("TDG_GZDEV_MAXCHUNKS")) max_chunks = (uint32_t)std::max(1, atoi(e));
-    max_chunks = std::min<uint32_t>(max_chunks, 65000);             // gz_ptr_*: a chunk index has 16 bits
-    // Chunk size, chosen per round from what is left of the file: every lane gets work when there is enough of
-    // it, in steps of 16 KiB between 32 and 128 KiB (a chunk should hold a block start: zlib's blocks are
-    // 10 - 30 KB of compressed data).  What a lane may produce: symbols up to 8 x its chunk (and room for a
-    // large block), token slots up to 3 x its chunk (literal codes of 4 bits and more: two slots per compressed
-    // byte); a chunk that needs more ends the device feed (the host reader takes over).
-    size_t fixed_chunk = 0;
-    if (const char *e = getenv("TDG_GZDEV_CHUNK")) fixed_chunk = std::max<size_t>(4096, strtoull(e, nullptr, 10) / 16 * 16);
-    uint32_t fixed_cap = 0;
-    if (const char *e = getenv("TDG_GZDEV_SYMCAP")) fixed_cap = (uint32_t)std::max<unsigned long long>(1024, strtoull(e, nullptr, 10));
-    const bool debug = getenv("TDG_GZDEV_DEBUG") != nullptr;
-    const int threads = gz_io_threads();
-    uint8_t *d_tabs = (uint8_t *)ctx->gz_tabs.p;
-    uint8_t *d_window = d_tabs + 512 + 1024;
-    CK(cudaMemsetAsync(d_window, 0, gzl::WIN, ctx->stream));
+    f.max_chunks = (uint32_t)ctx->sm_count * gzd::DEC_THREADS;          // one lane per chunk (or member), one CTA per SM
+    if (const char *e = getenv("TDG_GZDEV_MAXCHUNKS")) f.max_chunks = (uint32_t)std::max(1, atoi(e));
+    if (const char *e = getenv("TDG_GZDEV_CHUNK")) f.fixed_chunk = std::max<size_t>(4096, strtoull(e, nullptr, 10) / 16 * 16);
+    if (const char *e = getenv("TDG_GZDEV_SYMCAP")) f.fixed_cap = (uint32_t)std::max<unsigned long long>(1024, strtoull(e, nullptr, 10));
+    f.debug = getenv("TDG_GZDEV_DEBUG") != nullptr;
+    f.threads = gz_io_threads();
+    uint8_t *d_window = (uint8_t *)ctx->gz_tabs.p + 512 + 1024;
+    if (!bgzf) CK(cudaMemsetAsync(d_window, 0, gzl::WIN, ctx->stream));      // a stream has no history in front of it
     handled = true;
     carry = 0;
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-        return std::chrono::duration<double, std::milli>(b - a).count();
-    };
 
-    int up_i = 0;
-    auto upload = [&](int which, size_t off, size_t end, cudaStream_t stream) -> int {
-        return gz_upload(ctx, map, path, threads, up_i, which, off, end, stream);
-    };
-    int cur = 0;                                             // which compressed buffer the round reads
-    bool pre_valid = false;                                  // the other one holds [pre_off, pre_end) of the file
-    size_t pre_off = 0, pre_end = 0;
-
-    // One round.  TDG_ERR_NOMEM from a buffer that cannot be had is not the file's fault: nothing of the round
-    // has been delivered then, and the host reader takes over at the state the round began in.  Not so once
-    // the sink has the round's text (st has moved past it): its failure ends the feed (sink_rc).
-    int round_no = 0, sink_rc = TDG_OK;
     const int oom_round = getenv("TDG_GZDEV_OOM_ROUND") ? atoi(getenv("TDG_GZDEV_OOM_ROUND")) : -1;      // test hook
-    auto one_round = [&]() -> int {
-        if (round_no++ == oom_round) return fail(ctx, TDG_ERR_NOMEM, "buffer of 0 bytes: simulated (TDG_GZDEV_OOM_ROUND)");
-        size_t chunk = fixed_chunk;
-        if (!chunk) {
-            const size_t left = map.n - (size_t)(st.pos_bit >> 3);
-            chunk = round_up((left + max_chunks - 1) / max_chunks, (size_t)16 << 10);
-            chunk = std::min<size_t>(std::max<size_t>(chunk, (size_t)32 << 10), (size_t)128 << 10);
-        }
-        const uint32_t symcap = fixed_cap ? fixed_cap : (uint32_t)std::max<size_t>(8 * chunk, (size_t)256 << 10);
-        const uint32_t tokcap = fixed_cap ? fixed_cap : (uint32_t)std::max<size_t>(3 * chunk, (size_t)128 << 10);
-        const gzc::Round r = st.plan(chunk, max_chunks);
-        const size_t nb = r.buf_end - r.buf_off;
-        const size_t nwords = (nb + 3) / 4;
-        // ---- the round's compressed bytes: file -> pinned pieces -> device (or already there: see below)
-        auto t0 = now();
-        const bool prefetched = pre_valid && pre_off <= r.buf_off && pre_end >= r.buf_end && (r.buf_off - pre_off) % 16 == 0;
-        size_t comp_skip = 0;                                // where the round's bytes begin in the buffer
-        if (prefetched) {
-            cur ^= 1;                                        // the bytes sit in the other buffer: wait for their copies
-            comp_skip = r.buf_off - pre_off;
-            CK(cudaStreamWaitEvent(ctx->stream, ctx->gz_pre, 0));
-        } else {
-            rc = upload(cur, r.buf_off, r.buf_end, ctx->stream);
-            if (rc) return rc;
-        }
-        pre_valid = false;
-        Buf &comp = cur ? ctx->gz_comp2 : ctx->gz_comp;
-        if ((rc = grow(ctx, ctx->gz_syms, (size_t)r.nchunks * tokcap * 2, false))) return rc;
-        if ((rc = grow(ctx, ctx->gz_meta, (size_t)r.nchunks * sizeof(gzl::Meta), false))) return rc;
-        if ((rc = grow(ctx, ctx->gz_cand, (size_t)r.nchunks * gzd::MAXC * 4, false))) return rc;
-        if ((rc = grow(ctx, ctx->gz_ncand, (size_t)r.nchunks * 4, false))) return rc;
-        if ((rc = grow(ctx, ctx->gz_hmeta, (size_t)r.nchunks * sizeof(gzl::Meta), true))) return rc;
-        if ((rc = grow(ctx, ctx->gz_cold, (size_t)(r.nchunks + 8) * gzl::COLD_U16 * 2, false))) return rc;
-        if (debug) CK(cudaStreamSynchronize(ctx->stream));
-        auto t1 = now();
-        // ---- scan + decode
-        gzd::RoundArgs a;
-        memset(&a, 0, sizeof(a));                            // (m_start / m_end stay null: this is one stream, not BGZF members)
-        a.in = (const uint32_t *)((const uint8_t *)comp.p + comp_skip);
-        a.nwords = nwords;
-        a.in_bits = (uint64_t)nb * 8;
-        a.nchunks = r.nchunks;
-        a.chunk_bytes = chunk;
-        a.file_left = map.n - r.grid;
-        a.pos_rel = r.pos_bit - (uint64_t)r.grid * 8;
-        a.base_bit = (uint64_t)r.grid * 8;
-        a.hist = r.hist;
-        a.symcap = symcap;
-        a.tokcap = tokcap;
-        a.cand = (uint32_t *)ctx->gz_cand.p;
-        a.ncand = (uint32_t *)ctx->gz_ncand.p;
-        a.syms = (uint16_t *)ctx->gz_syms.p;
-        a.meta = (gzl::Meta *)ctx->gz_meta.p;
-        a.kraft3 = d_tabs;
-        a.cold = (uint16_t *)ctx->gz_cold.p;
-        CK(cudaMemsetAsync(ctx->gz_ncand.p, 0, (size_t)r.nchunks * 4, ctx->stream));
-        if (r.nchunks > 1) {
-            const unsigned g = (r.nchunks - 1 + gzd::SCAN_WARPS - 1) / gzd::SCAN_WARPS;
-            gzd::gz_scan<<<g, gzd::SCAN_WARPS * 32, gzd::SCAN_SMEM, ctx->stream>>>(a);
-            CK(cudaGetLastError());
-            ctx->launches++;
-        }
-        if (debug) CK(cudaStreamSynchronize(ctx->stream));
-        auto t2 = now();
-        gzd::gz_decode<<<(r.nchunks + gzd::DEC_THREADS - 1) / gzd::DEC_THREADS, gzd::DEC_THREADS, gzd::DEC_SMEM, ctx->stream>>>(a);
-        CK(cudaGetLastError());
-        ctx->launches++;
-        gzl::Meta *meta = (gzl::Meta *)ctx->gz_hmeta.p;
-        CK(cudaMemcpyAsync(meta, ctx->gz_meta.p, (size_t)r.nchunks * sizeof(gzl::Meta), cudaMemcpyDeviceToHost, ctx->stream));
-        // While the lanes inflate, this thread reads the bytes the NEXT round will most likely ask
-        // for (every chunk accepted: its grid starts where this one's ends) and sends them to the
-        // other buffer on the copy stream.
-        double ms_prefetch = 0;
-        const auto tp0 = now();
-        if (r.grid + (size_t)r.nchunks * chunk < map.n && r.nchunks == max_chunks) {
-            pre_off = r.grid + (size_t)r.nchunks * chunk;    // (the next round's grid starts here or, with smaller chunks, a little further on)
-            pre_end = std::min(map.n, pre_off + ((size_t)max_chunks + 2) * chunk);
-            rc = upload(cur ^ 1, pre_off, pre_end, ctx->copy_stream);
-            if (rc) return rc;
-            CK(cudaEventRecord(ctx->gz_pre, ctx->copy_stream));
-            pre_valid = true;
-            ms_prefetch = ms(tp0, now());
-        }
-        CK(cudaStreamSynchronize(ctx->stream));
-        auto t3 = now();
-        // ---- which chunks continue the stream
-        const gzc::Outcome o = st.chain(r, meta, symcap);
-        uint64_t text_len = o.text_off.back();
-        if (o.accepted && text_len) {
-            const int go = sink.may_take(ctx, (size_t)text_len);
-            if (go < 0) return go;
-            if (go == 0) return TDG_STOP_ROUND;              // nothing of this round is used: the host feeder starts where it began
-        }
-        uint32_t text_crc = 0;
-        auto t4 = t3, t5 = t3;
-        if (o.accepted && text_len) {
-            const uint32_t pieces = (uint32_t)((text_len + gzd::PIECE - 1) / gzd::PIECE);
-            if ((rc = grow(ctx, ctx->gz_windows, ((size_t)o.accepted + 1) * (gzl::WIN * 4 + 1), false))) return rc;
-            if ((rc = grow(ctx, ctx->gz_lens, (size_t)o.accepted * 4, false))) return rc;
-            if ((rc = grow(ctx, ctx->gz_offs, ((size_t)o.accepted + 1) * 8, false))) return rc;
-            if ((rc = grow(ctx, ctx->gz_crc, ((size_t)pieces + pieces / 256 + 2) * 4 + 16, false))) return rc;
-            if ((rc = grow(ctx, ctx->gz_hcrc, ((size_t)pieces / 256 + 4) * 4 + 16, true))) return rc;
-            // the text buffer keeps the carried bytes in front
-            const size_t need = round_up(carry + text_len, TDG_TILE_BYTES) + TDG_HALO_BYTES + 64;
-            if (need > ctx->gz_text.cap) {
-                if (carry) {
-                    if ((rc = grow(ctx, ctx->gz_carry, carry, false))) return rc;
-                    CK(cudaMemcpyAsync(ctx->gz_carry.p, ctx->gz_text.p, carry, cudaMemcpyDeviceToDevice, ctx->stream));
-                }
-                if ((rc = grow(ctx, ctx->gz_text, need, false))) return rc;
-                if (carry) CK(cudaMemcpyAsync(ctx->gz_text.p, ctx->gz_carry.p, carry, cudaMemcpyDeviceToDevice, ctx->stream));
-            }
-            CK(cudaMemcpyAsync(ctx->gz_lens.p, o.lens.data(), o.lens.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-            // tokens -> symbols (accepted chunks only)
-            // the symbols: as many per chunk as the largest accepted chunk has
-            uint32_t stride = 64;
-            for (uint32_t len : o.lens) stride = std::max(stride, len);
-            stride = (stride + 63u) & ~63u;
-            if ((rc = grow(ctx, ctx->gz_sym2, (size_t)o.accepted * stride * 2, false))) return rc;
-            if ((rc = grow(ctx, ctx->gz_ntok, (size_t)o.accepted * 4, false))) return rc;
-            {
-                std::vector<uint32_t> ntok(o.accepted);
-                for (uint32_t k = 0; k < o.accepted; k++) ntok[k] = o.lens[k] ? meta[k].ntok : 0u;
-                for (const gzc::Repair &rp : o.repairs) ntok[rp.chunk] = 0;          // the host made these chunks' symbols
-                CK(cudaMemcpyAsync(ctx->gz_ntok.p, ntok.data(), ntok.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-                CK(cudaStreamSynchronize(ctx->stream));      // (ntok is a local)
-                gzd::ExpandArgs ea;
-                ea.tok = a.syms;
-                ea.syms = (uint16_t *)ctx->gz_sym2.p;
-                ea.tokcap = tokcap;
-                ea.symcap = stride;
-                ea.ntok = (const uint32_t *)ctx->gz_ntok.p;
-                ea.accepted = o.accepted;
-                gzd::gz_expand<<<(o.accepted + gzd::EXP_WARPS - 1) / gzd::EXP_WARPS, gzd::EXP_WARPS * 32, 0, ctx->stream>>>(ea);
-                CK(cudaGetLastError());
-                ctx->launches++;
-                for (const gzc::Repair &rp : o.repairs)
-                    if (!rp.syms.empty())
-                        CK(cudaMemcpyAsync((uint16_t *)ctx->gz_sym2.p + (size_t)rp.chunk * stride, rp.syms.data(), rp.syms.size() * 2,
-                                           cudaMemcpyHostToDevice, ctx->stream));
-                if (debug) {
-                    CK(cudaStreamSynchronize(ctx->stream));
-                    fprintf(stderr, "gzdev expand: %.1f ms, %zu chunks made by the host\n", ms(t3, now()), o.repairs.size());
-                }
-            }
-            CK(cudaMemcpyAsync(ctx->gz_offs.p, o.text_off.data(), o.text_off.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-            gzd::WinArgs w;
-            w.syms = (const uint16_t *)ctx->gz_sym2.p;
-            w.symcap = stride;
-            w.out_len = (const uint32_t *)ctx->gz_lens.p;
-            w.accepted = o.accepted;
-            w.window_in = d_window;
-            w.ptrs = (uint32_t *)ctx->gz_windows.p;
-            w.done = (uint8_t *)ctx->gz_windows.p + ((size_t)o.accepted + 1) * gzl::WIN * 4;
-            w.window_out = d_window;
-            gzd::gz_ptr_init<<<o.accepted + 1, gzd::WIN_THREADS, 0, ctx->stream>>>(w);
-            CK(cudaGetLastError());
-            uint32_t passes = 1;
-            while ((1u << (passes - 1)) < o.accepted + 1) passes++;          // chains are at most accepted + 1 long
-            for (uint32_t ps = 0; ps < passes; ps++) gzd::gz_ptr_jump<<<o.accepted, gzd::WIN_THREADS, 0, ctx->stream>>>(w);
-            CK(cudaGetLastError());
-            ctx->launches += 1 + passes;
-            if (debug) {
-                CK(cudaStreamSynchronize(ctx->stream));
-                fprintf(stderr, "gzdev windows: %u passes, %.1f ms\n", passes, ms(t3, now()));
-            }
-            uint32_t *d_flag = (uint32_t *)ctx->gz_crc.p + pieces;
-            CK(cudaMemsetAsync(d_flag, 0, 4, ctx->stream));
-            gzd::ResArgs ra;
-            ra.syms = (const uint16_t *)ctx->gz_sym2.p;
-            ra.symcap = stride;
-            ra.text_off = (const uint64_t *)ctx->gz_offs.p;
-            ra.accepted = o.accepted;
-            ra.ptrs = (const uint32_t *)ctx->gz_windows.p;
-            ra.text = (uint8_t *)ctx->gz_text.p + carry;
-            ra.text_len = text_len;
-            ra.crc = (uint32_t *)ctx->gz_crc.p;
-            ra.flag = d_flag;
-            ra.table = (const uint32_t *)(d_tabs + 512);
-            for (int j = 0; j < 8; j++) ra.op[j] = ctx->gz_op[j];
-            gzd::gz_resolve<<<pieces, gzd::RES_THREADS, 0, ctx->stream>>>(ra);
-            CK(cudaGetLastError());
-            // the window behind the last accepted chunk opens the next round
-            gzd::gz_ptr_take<<<8, gzd::WIN_THREADS, 0, ctx->stream>>>(w);
-            CK(cudaGetLastError());
-            ctx->launches += 2;
-            // the pieces' raw CRCs: 256 full pieces fold into one on the device, the host folds the rest
-            const uint32_t nfull = (uint32_t)(text_len / gzd::PIECE), groups = (nfull + 255) / 256;
-            uint32_t *d_group = d_flag + 1;
-            if (groups) {
-                gzd::CrcFoldArgs fa;
-                fa.piece = (const uint32_t *)ctx->gz_crc.p;
-                fa.nfull = nfull;
-                fa.group = d_group;
-                for (int j = 0; j < 8; j++) fa.op[j] = (uint32_t)crc32_combine_gen((z_off_t)((uint64_t)gzd::PIECE << j));
-                gzd::gz_crc_fold<<<groups, 256, 0, ctx->stream>>>(fa);
-                CK(cudaGetLastError());
-                ctx->launches++;
-            }
-            // host copy: [0] the high-bit flag, [1 .. groups] the group CRCs, [groups + 1] the last (partial) piece's
-            uint32_t *hcrc = (uint32_t *)ctx->gz_hcrc.p;
-            CK(cudaMemcpyAsync(hcrc, d_flag, ((size_t)groups + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-            if (pieces > nfull)
-                CK(cudaMemcpyAsync(hcrc + groups + 1, (uint32_t *)ctx->gz_crc.p + nfull, 4, cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaStreamSynchronize(ctx->stream));
-            t4 = now();
-            // CRC-32 of the round's text from the raw CRCs
-            uLong raw = 0;
-            if (groups) {
-                const uLong op_group = crc32_combine_gen((z_off_t)((uint64_t)gzd::PIECE * 256));
-                for (uint32_t g = 0; g + 1 < groups; g++) raw = crc32_combine_op(raw, hcrc[1 + g], op_group);
-                const uint64_t last_group = (uint64_t)(nfull - (groups - 1) * 256u) * gzd::PIECE;
-                raw = crc32_combine_op(raw, hcrc[groups], crc32_combine_gen((z_off_t)last_group));
-            }
-            if (pieces > nfull) raw = crc32_combine_op(raw, hcrc[groups + 1], crc32_combine_gen((z_off_t)(text_len - (uint64_t)nfull * gzd::PIECE)));
-            text_crc = (uint32_t)(raw ^ crc32_combine_op(0xFFFFFFFFul, 0, crc32_combine_gen((z_off_t)text_len)) ^ 0xFFFFFFFFul);
-            const uint32_t high_flag = hcrc[0];
-            // text mode: bytes >= 0x80 must form valid UTF-8 (open(f, 'rt'))
-            if (u8) {
-                if ((high_flag & 0x80u) || u8->need) {
-                    std::vector<uint8_t> host(text_len);
-                    CK(cudaMemcpy(host.data(), (uint8_t *)ctx->gz_text.p + carry, text_len, cudaMemcpyDeviceToHost));
-                    long long bad = tdg::utf8_feed(*u8, host.data(), host.size());
-                    if (bad >= 0) return fail(ctx, TDG_ERR_UTF8, "position " + std::to_string(bad) + ": invalid UTF-8 in " + path);
-                } else {
-                    u8->offset += text_len;
-                }
-            }
-            t5 = now();
-        }
-        if (!st.advance(r, o, text_len, text_crc))
-            return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + path + ": incorrect data check");
-        if (o.accepted && text_len) {
-            rc = sink.text(ctx, (uint8_t *)ctx->gz_text.p, carry, (size_t)text_len);
-            if (rc) return sink_rc = rc;
-        }
-        auto t6 = now();
-        if (stats) {
-            stats->rounds++;
-            stats->chunks += r.nchunks;
-            stats->accepted += o.accepted;
-            stats->ms_upload += ms(t0, t1);
-            stats->ms_scan += ms(t1, t2);
-            stats->ms_decode += ms(t2, t3);
-            stats->ms_host += ms(t3, t3) + ms(t4, t5);
-            stats->ms_resolve += ms(t3, t4);
-            stats->ms_sink += ms(t5, t6);
-        }
-        if (debug)
-            fprintf(stderr, "gzdev round: %u chunks of %zu KiB, %u accepted, %llu bytes of text; upload %.1f%s scan %.1f decode %.1f "
-                            "(host read the next round's bytes meanwhile: %.1f) expand+windows+resolve %.1f crc/utf8 %.1f sink %.1f ms%s%s\n",
-                    r.nchunks, chunk >> 10, o.accepted, (unsigned long long)text_len, ms(t0, t1), prefetched ? " (prefetched)" : "", ms(t1, t2),
-                    ms(t2, t3), ms_prefetch, ms(t3, t4), ms(t4, t5),
-                    ms(t5, t6), st.handover ? "  -> host reader: " : "", st.handover ? st.why : "");
-        return TDG_OK;
-    };
-    while (!st.eof && !st.handover) {
-        rc = one_round();
-        if (!sink_rc && (rc == TDG_ERR_NOMEM || rc == TDG_STOP_ROUND)) {
-            st.handover = true;
-            st.why = rc == TDG_ERR_NOMEM ? "device memory" : "read limit within reach";
-            pre_valid = false;
-            break;
-        }
-        if (rc) return rc;
+    int (*round)(GzFeed &) = bgzf ? gz_bgzf_round : gz_stream_round;
+    for (int round_no = 0; !f.done && !f.handover; round_no++) {
+        f.sunk = false;
+        rc = round_no == oom_round ? fail(ctx, TDG_ERR_NOMEM, "buffer of 0 bytes: simulated (TDG_GZDEV_OOM_ROUND)") : round(f);
+        if (!f.sunk && (rc == TDG_ERR_NOMEM || rc == TDG_STOP_ROUND)) f.handover = true;         // at the state the round began in
+        else if (rc) return rc;
     }
-    if (st.handover) {
+    if (f.handover) {
         ho.active = true;
-        ho.to_zlib = st.to_zlib;
-        ho.pos_bit = st.pos_bit;
-        ho.hist = st.hist;
-        ho.crc = st.crc;
-        ho.member_len = st.member_len;
-        ho.delivered = st.delivered;
-        ho.why = st.why;
-        ho.window.resize(gzl::WIN);
-        CK(cudaMemcpyAsync(ho.window.data(), d_window, gzl::WIN, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
+        ho.bgzf = bgzf;
+        ho.bgzf_off = f.off;
+        ho.to_zlib = f.st.to_zlib;
+        ho.pos_bit = f.st.pos_bit;
+        ho.hist = f.st.hist;
+        ho.crc = f.st.crc;
+        ho.member_len = f.st.member_len;
+        ho.delivered = bgzf ? f.delivered : f.st.delivered;
+        if (!bgzf) {
+            ho.window.resize(gzl::WIN);
+            CK(cudaMemcpyAsync(ho.window.data(), d_window, gzl::WIN, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+        }
     }
     return TDG_OK;
 }

@@ -11,6 +11,7 @@ import random
 import numpy as np
 import pytest
 
+from feed_check import bgzf_compress
 from tagdigger_b200 import _native, hostio, matchset, synth, trimming
 
 pytestmark = pytest.mark.gpu
@@ -38,6 +39,9 @@ class Inputs:
             fh.write(self.fq)
         with open(self.gz, "wb") as fh:
             fh.write(gzip.compress(self.fq, 6))
+        self.bgzf = str(tmp_path / ("reads%d.bgzf.gz" % big))
+        with open(self.bgzf, "wb") as fh:
+            fh.write(bgzf_compress(self.fq))
         barcut = hostio.combine_barcode_and_cutsite(self.barcodes, "TGCAG")
         self.split_bar = matchset.effective_set(barcut, len(barcut))
         with contextlib.redirect_stdout(io.StringIO()):
@@ -84,6 +88,11 @@ def _plain_file(eng, d):
 def _gzip_file(eng, d):
     _begin(eng, d)
     return _count(eng, d.gz)
+
+
+def _bgzf_file(eng, d):
+    _begin(eng, d)
+    return _count(eng, d.bgzf)
 
 
 def _released_gzip_file(eng, d):
@@ -142,7 +151,8 @@ def _match_batch(eng, d):
     return (row.tobytes(), col.tobytes()), None
 
 
-UNITS = [_tables, _submit, _plain_file, _gzip_file, _released_gzip_file, _timed, _trim, _split, _split_batch, _match_batch]
+GZIP_UNITS = (_gzip_file, _bgzf_file, _released_gzip_file)
+UNITS = [_tables, _submit, _plain_file, _gzip_file, _bgzf_file, _released_gzip_file, _timed, _trim, _split, _split_batch, _match_batch]
 
 
 def _sequence(eng, passes):
@@ -170,7 +180,7 @@ def test_allocation_failure_leaves_a_working_context(tmp_path, monkeypatch):
     want, want_feeds, failed = _sequence(eng, passes)
     eng.close()
     assert not failed
-    assert want_feeds[UNITS.index(_gzip_file)] == 0 and want_feeds[UNITS.index(_released_gzip_file)] == 0
+    assert all(want_feeds[UNITS.index(u)] == 0 for u in GZIP_UNITS)
 
     for k in range(1, BOUND + 1):
         monkeypatch.setenv("TDG_FAIL_ALLOC", str(k))
@@ -180,7 +190,7 @@ def test_allocation_failure_leaves_a_working_context(tmp_path, monkeypatch):
         for i, (a, b) in enumerate(zip(got, want)):
             assert a == b, "allocation %d: unit %s of pass %d" % (k, UNITS[i % len(UNITS)].__name__, i // len(UNITS))
         handed_over = [i for i, (f, w) in enumerate(zip(feeds, want_feeds)) if f != w]
-        assert all(UNITS[i % len(UNITS)] in (_gzip_file, _released_gzip_file) and feeds[i] == 1 for i in handed_over), (k, feeds)
+        assert all(UNITS[i % len(UNITS)] in GZIP_UNITS and feeds[i] == 1 for i in handed_over), (k, feeds)
         if not failed and not handed_over:
             break                                           # k is past the last allocation of the sequence
     else:
