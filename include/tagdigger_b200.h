@@ -242,8 +242,9 @@ int         tdg_memcpy_d2h(tdg_ctx *ctx, void *host, const void *dev, size_t n);
 uint64_t    tdg_launch_count(const tdg_ctx *ctx);
 /* Device time in milliseconds of the counting kernels launched between
  * tdg_timing_begin and tdg_timing_end (CUDA events on the context's stream,
- * one pair per kernel launch; at most 4096 launches), and of the BGZF writer's
- * kernels (one pair per deflate-scan-pack sequence).  tdg_timing_end
+ * one pair per kernel launch; at most 4096 launches), of the BGZF writer's
+ * kernels (one pair per deflate-scan-pack sequence) and of every
+ * tdg_split_count_block (one pair around its upload and kernels).  tdg_timing_end
  * synchronises; *nlaunch receives the number of kernels timed. */
 int         tdg_timing_begin(tdg_ctx *ctx);
 int         tdg_timing_end(tdg_ctx *ctx, double *kernel_ms, uint32_t *nlaunch);
@@ -302,6 +303,30 @@ int         tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int fi
                             uint64_t max_records, uint64_t *n_records, uint64_t *consumed,
                             int *needs_host, const uint8_t **out, const uint64_t **out_off,
                             const uint8_t **flags);
+
+/* Counting the streaming splitter's output instead of writing it: barcodeSplitter(f, barcodes,
+ * files, cutsite=S1, adapter=A) followed by find_tags_fastq(files[b], [''], tags, cutsite) for every
+ * barcode b, with barcode b's counts added to matrix row row_of_barcode[b] -- in one pass, without
+ * the files.  The stage-2 line of a record is t = sequence[slice1:slice2].strip() (upper case).
+ * tdg_split_count_begin: after tdg_set_tags, a matrix and tdg_split_begin (tdg_split_begin drops
+ * it again); loads the stage-2 barcode+cutsite table (blank barcode: the patterns, tag offsets and
+ * flags tdg_begin_file takes, without rows) and row_of_barcode[nbar], every row inside the matrix.
+ * The stage-1 table of tdg_begin_file stays as it is.
+ * tdg_split_count_block: as tdg_split_block for *n_records, *consumed and *needs_host; instead of
+ * output bytes, every record's tag hit is added to the matrix and totals[] receives the block's
+ * reads, reads with barcode and cut site, reads clipped on the 3' end and reads with a tag.  With
+ * *needs_host = 1 the matrix is untouched and totals[] are 0: the caller decides the records with
+ * tdg_split_batch, cuts t itself and counts it with tdg_split_count_batch.
+ * tdg_split_count_batch: n stage-2 lines t_i given as HOST buffers (stripped, upper case) with
+ * their stage-1 barcodes bar[i] (0 <= bar[i] < nbar); adds the hits to the matrix and returns
+ * col_out[i] = the tag column or -1.  Synchronous. */
+int         tdg_split_count_begin(tdg_ctx *ctx, const char *bases, const uint32_t *off, const uint32_t *tag_off,
+                                  uint32_t npat, uint32_t flags, const int32_t *row_of_barcode);
+int         tdg_split_count_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block,
+                                  uint64_t max_records, uint64_t *n_records, uint64_t *consumed,
+                                  int *needs_host, uint64_t totals[4]);
+int         tdg_split_count_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, const int32_t *bar,
+                                  uint32_t n, int32_t *col_out);
 
 /* BGZF output files for the streaming splitter (the reference writes plain text only).  Every
  * barcode's file is the series of gzip members bgzip writes: member k holds bytes

@@ -6,6 +6,12 @@ against the markers a keep-list leaves (tagdigger_script.py -k: :71-76, :123-133
 counting.count_files.  Reported: reads/s of each stage and of the flow; checked: the count rows of the
 first samples against the C oracle run over the split files, cell by cell.
 
+The fused leg counts the same library in one pass (count_files(..., adapter=...): split, trim and count
+on the GPU without the split files), alternating with the two-stage flow in the same process; its matrix
+must equal the two-stage matrix in every cell.  Reported for it: reads/s, the device time of its blocks
+(CUDA events around every block's upload and kernels), the time the host feed alone takes to read the
+input, and the GPU's name and power limit.
+
     python scripts/config5_flow.py [reads]
 """
 import contextlib
@@ -13,6 +19,7 @@ import io
 import json
 import os
 import random
+import subprocess
 import sys
 import tempfile
 import time
@@ -46,9 +53,33 @@ def make_reads(rng, barcodes, tags, adapter, n):
     return "".join(out)
 
 
+def gpu_name_and_power_limit():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                             stdout=subprocess.PIPE, universal_newlines=True, timeout=60).stdout
+        return out.splitlines()[0].strip()
+    except (OSError, IndexError, subprocess.SubprocessError):
+        return "unknown"
+
+
+def feed_seconds(_native, path):
+    """The host feed alone (splitter.BLOCK_BYTES per read, into pinned memory): what the fused pass reads through."""
+    from tagdigger_b200 import counting, splitter
+    eng = counting.get_engine()
+    buf = eng.host_alloc(splitter.BLOCK_BYTES)
+    feed = _native.Feed(path, False)
+    t0 = time.perf_counter()
+    while feed.read_into(buf, splitter.BLOCK_BYTES):
+        pass
+    t1 = time.perf_counter()
+    feed.close()
+    eng.host_free(buf)
+    return t1 - t0
+
+
 def main():
     from oracle import c_oracle
-    from tagdigger_b200 import counting, hostio, splitter, synth
+    from tagdigger_b200 import _native, counting, hostio, splitter, synth
     reads = int(sys.argv[1]) if len(sys.argv) > 1 else 8_000_000
     rng = random.Random(5)
     nrng = np.random.default_rng(5)
@@ -72,8 +103,13 @@ def main():
     res = {"config": "configs[4] as a flow: %d reads (150 bp), PstI-MspI-Hall adapters, 96-plex, %d tags of which a marker list keeps %d"
                      % (reads, len(tags), len(kept_tags)),
            "reads": reads, "input_MB": round(os.path.getsize(inp) / 1e6, 1), "host_cpus": os.cpu_count(), "runs": []}
+    fused_key = {inp: [list(barcodes), ["Sample%02d" % i for i in range(len(barcodes))]]}
+    res["gpu"] = gpu_name_and_power_limit()
+    res["feed_s"] = round(feed_seconds(_native, inp), 3)
+    res["fused_runs"] = []
     counts = None
-    for rep in range(2):
+    same = True
+    for rep in range(3):
         for o in outs:
             if os.path.exists(o):
                 os.remove(o)
@@ -87,6 +123,16 @@ def main():
         res["runs"].append({"split_s": round(t1 - t0, 3), "count_s": round(t2 - t1, 3),
                             "split_reads_per_s": round(reads / (t1 - t0), 1), "count_reads_per_s": round(reads / (t2 - t1), 1),
                             "flow_reads_per_s": round(reads / (t2 - t0), 1)})
+        eng = counting.get_engine()
+        t0 = time.perf_counter()
+        eng.timing_begin()
+        with contextlib.redirect_stdout(io.StringIO()):
+            _, fused = counting.count_files(fused_key, kept_tags, "TGCAG", as_array=True, adapter="PstI-MspI-Hall")
+        ms, blocks = eng.timing_end()
+        t1 = time.perf_counter()
+        same &= bool(np.array_equal(fused, counts))
+        res["fused_runs"].append({"fused_s": round(t1 - t0, 3), "fused_reads_per_s": round(reads / (t1 - t0), 1),
+                                  "block_device_ms": round(ms, 1), "blocks": blocks})
     res["split_output_MB"] = round(sum(os.path.getsize(o) for o in outs) / 1e6, 1)
     res["tag_hits"] = int(np.asarray(counts).sum())
     ok = True
@@ -95,6 +141,8 @@ def main():
             want, _ = c_oracle.Counter([""], kept_tags, "TGCAG").count(fh.read())
         ok &= bool((np.asarray(counts[i]) == want[0]).all())
     res["rows_equal_c_oracle_on_split_files"] = "ok (3 samples)" if ok else "FAILED"
+    res["fused_matrix_equals_two_stage"] = "ok (every cell)" if same else "FAILED"
+    ok &= same
     print(json.dumps(res))
     for p in outs + [inp]:
         os.remove(p)

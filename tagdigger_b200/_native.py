@@ -37,7 +37,8 @@ tdg_bind_matrix tdg_zero_matrix tdg_begin_file tdg_reset_file tdg_submit tdg_end
 tdg_count_lines_device tdg_count_file tdg_count_file2 tdg_last_file_info tdg_gz_inflate_host tdg_release_scratch tdg_sync tdg_file_totals tdg_read_matrix tdg_matrix_min tdg_comm_unique_id tdg_comm_init tdg_allreduce_matrix tdg_finish
 tdg_matrix_device_ptr tdg_stream tdg_stream_wait tdg_other_stream_wait tdg_host_alloc
 tdg_host_free tdg_device_alloc tdg_device_free tdg_memcpy_h2d tdg_memcpy_d2h tdg_launch_count
-tdg_timing_begin tdg_timing_end tdg_set_trim tdg_trim_batch tdg_split_batch tdg_split_begin tdg_split_block tdg_split_bgzf tdg_bgzf_append tdg_bgzf_finish tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
+tdg_timing_begin tdg_timing_end tdg_set_trim tdg_trim_batch tdg_split_batch tdg_split_begin tdg_split_block
+tdg_split_count_begin tdg_split_count_block tdg_split_count_batch tdg_split_bgzf tdg_bgzf_append tdg_bgzf_finish tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
 
 
 class TdgError(RuntimeError):
@@ -142,6 +143,9 @@ def lib():
         "tdg_split_begin": (i32, [vp, vp, vp, u32, u32]),
         "tdg_split_block": (i32, [vp, vp, sz, i32, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32),
                                   ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp)]),
+        "tdg_split_count_begin": (i32, [vp, vp, vp, vp, u32, u32, vp]),
+        "tdg_split_count_block": (i32, [vp, vp, sz, i32, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32), vp]),
+        "tdg_split_count_batch": (i32, [vp, vp, vp, vp, u32, vp]),
         "tdg_split_bgzf": (i32, [vp, i32]),
         "tdg_bgzf_append": (i32, [vp, vp, vp, ctypes.POINTER(vp), ctypes.POINTER(vp)]),
         "tdg_bgzf_finish": (i32, [vp, ctypes.POINTER(vp), ctypes.POINTER(vp)]),
@@ -525,6 +529,46 @@ class Engine(object):
         pieces = self._pieces(out, off)
         fl = np.ctypeslib.as_array(ctypes.cast(flags, ctypes.POINTER(ctypes.c_uint8)), shape=(max(nrec.value, 1),))[:nrec.value]
         return nrec.value, used.value, False, pieces, fl
+
+    def split_count_begin(self, patterns, tag_offs, rows, any_base=False):
+        """Count mode of the split started by split_begin (after set_tags and set_matrix): the
+        stage-2 barcode+cutsite table (blank barcode: matchset.plan([''], tags, cutsite).bar with
+        its tag offsets) and rows[b], the matrix row barcode b's reads are counted into."""
+        blob, off = _csr(patterns, np.uint32)
+        toff = np.asarray(list(tag_offs), dtype=np.uint32)
+        row = np.asarray(list(rows), dtype=np.int32)
+        if len(row) != self._split_nbar:
+            raise ValueError("one row per barcode: %d given, %d barcodes" % (len(row), self._split_nbar))
+        self._ck(self._L.tdg_split_count_begin(self._h, blob, off.ctypes.data, toff.ctypes.data, len(patterns),
+                                               TDG_ANY_BASE if any_base else 0, row.ctypes.data))
+
+    def split_count_block(self, ptr, n, final, max_records):
+        """split_block that counts the trimmed reads into the matrix instead of returning them.
+        Returns (records, consumed bytes, needs_host, totals): totals = [reads, with barcode and cut
+        site, clipped on the 3' end, with tag] of the block; None when needs_host (nothing counted)."""
+        u64 = ctypes.c_uint64
+        nrec, used, host = u64(0), u64(0), ctypes.c_int(0)
+        tot = np.zeros(4, dtype=np.uint64)
+        self._ck(self._L.tdg_split_count_block(self._h, ptr, n, 1 if final else 0, min(int(max_records), (1 << 64) - 1),
+                                               ctypes.byref(nrec), ctypes.byref(used), ctypes.byref(host), tot.ctypes.data))
+        if host.value:
+            return nrec.value, used.value, True, None
+        self.note_hits(int(tot[3]))
+        return nrec.value, used.value, False, [int(x) for x in tot]
+
+    def split_count_batch(self, seqs, bars):
+        """seqs: stage-2 lines t (stripped, upper case; bytes/str) of reads with barcode bars[i].
+        Counts them into the matrix; returns the tag column of each, -1 = no tag."""
+        raw = [x.encode("utf-8") if isinstance(x, str) else bytes(x) for x in seqs]
+        blob = b"".join(raw)
+        off = np.zeros(len(raw) + 1, dtype=np.uint64)
+        if raw:
+            np.cumsum([len(x) for x in raw], out=off[1:])
+        bar = np.asarray(list(bars), dtype=np.int32)
+        col = np.empty(len(raw), dtype=np.int32)
+        self._ck(self._L.tdg_split_count_batch(self._h, blob, off.ctypes.data, bar.ctypes.data, len(raw), col.ctypes.data))
+        self.note_hits(int(np.count_nonzero(col >= 0)))
+        return col
 
     def _pieces(self, out, off):
         """Per-barcode views of out[off[b] .. off[b+1]) (pinned memory of the context)."""

@@ -196,7 +196,7 @@ def global_rows(bckeys):
 
 
 def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0, world=1, reduce=None,
-                totals=None, as_array=False, gather=None):
+                totals=None, as_array=False, gather=None, adapter=None, split_cutsite=None, split_maxreads=500000000):
     """All files of a key (``readBarcodeKeyfile`` output) in one go: the batched
     form of the loop at tagdigger_script.py:123-128.  Every file counts straight
     into the GLOBAL sample rows of one device matrix, so the result equals
@@ -214,9 +214,22 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
     with ``as_array=True``, as one int32 ndarray (hostio.writeCounts / writeDiploidGeno format
     that with native threads; a 384 x 500,000 matrix is 768 MB as an array and several GB as
     Python integers).  ``totals`` (optional dict) receives ``{file: [reads, with barcode and
-    cut site, with tag]}`` for this rank's files."""
+    cut site, with tag]}`` for this rank's files.
+
+    With ``adapter`` (the name of an adapter set, a key of ``hostio.adapters``) every file is first
+    split and trimmed as ``barcodeSplitter(f, barcodes, files, cutsite=split_cutsite, adapter=...,
+    maxreads=split_maxreads)`` would, and each barcode's output is then counted as
+    ``find_tags_fastq(file, [''], tags, cutsite)`` into its sample's row -- in one pass per file on the
+    GPU, without writing the split files (:func:`splitter.count_trimmed_file`).  ``split_cutsite``
+    defaults to the cut site of the adapter set's enzyme, as barcode_splitter_script derives it.  Files
+    are dealt whole to the ranks.  ``totals`` then receives ``[reads, with barcode and cut site, clipped
+    on the 3' end, with tag]``."""
     files = sorted(bckeys.keys())
     samples, rows = global_rows(bckeys)
+    if adapter is not None:
+        eng = _count_trimmed_files(bckeys, files, rows, len(samples), tags, cutsite, maxreads, device, rank, world,
+                                   totals, adapter, split_cutsite, split_maxreads)
+        return _result(eng, samples, len(tags), world, reduce, as_array)
     limit = _native.limit_from_maxreads(maxreads)
     plans = {}
     tagplan = None
@@ -249,12 +262,49 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
         print("{0}: Reads: {1} With barcode and cut site: {2} With tag: {3}".format(f, tot[0], tot[1], tot[2]))
         if totals is not None:
             totals[f] = tot[:3]
+    return _result(eng, samples, ntags, world, reduce, as_array)
+
+
+def _result(eng, samples, ntags, world, reduce, as_array):
+    """count_files' return value: the matrix, summed over the ranks."""
     if world > 1:
         if reduce is None:
             raise ValueError("count_files with world > 1 needs a reduce callable (see nccl_reduce)")
         reduce(eng.matrix_ptr(), len(samples), ntags, eng)
     matrix = eng.read_matrix()
     return [samples, matrix if as_array else matrix.tolist()]
+
+
+def _count_trimmed_files(bckeys, files, rows, nrows, tags, cutsite, maxreads, device, rank, world, totals, adapter,
+                         split_cutsite, split_maxreads):
+    """count_files with ``adapter``: this rank's files through splitter.count_trimmed_file.  Returns the engine."""
+    from . import hostio, splitter
+    if not isinstance(adapter, str) or adapter not in hostio.adapters:
+        raise ValueError("unknown adapter set %r (one of %s)" % (adapter, ", ".join(sorted(hostio.adapters))))
+    if maxreads != 5e9:
+        raise ValueError("maxreads does not apply with adapter: a split file holds at most split_maxreads reads")
+    if split_maxreads is None or not float(split_maxreads) <= 5e9:
+        raise ValueError("split_maxreads must be at most 5e9, the number of reads the counter takes from a split file")
+    adapter_seqs = hostio.adapters[adapter]
+    if split_cutsite is None:
+        split_cutsite = hostio.enzymes[adapter[:adapter.find("-")]]
+    # set-up errors surface before any counting, in the order of the two-stage run: every file's split, then the count
+    for f in files:
+        splitter._check_args(split_cutsite, bckeys[f][0], adapter_seqs)
+        splitter._split_patterns(bckeys[f][0], split_cutsite)
+    plan = matchset.plan([""], tags, cutsite)
+    if plan.ntags == 0:
+        raise IndexError("list index out of range")
+    eng = get_engine(device)
+    eng.set_tags(plan.tags.patterns, plan.tags.index, any_base=plan.tags.any_base)
+    eng.set_matrix(nrows, plan.ntags)
+    for f in assign_files(files, rank, world):
+        tot = splitter.count_trimmed_file(eng, f, bckeys[f][0], rows[f], plan, cutsite=split_cutsite, adapter=adapter_seqs,
+                                          maxreads=split_maxreads)
+        print("{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}".format(f, *tot))
+        if totals is not None:
+            totals[f] = tot
+    return eng
 
 
 SHARD_MIN_BYTES = 1 << 20     # files smaller than this per rank are not worth cutting up

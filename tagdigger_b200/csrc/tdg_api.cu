@@ -1,7 +1,8 @@
 // C ABI of tagdigger_b200 (see include/tagdigger_b200.h): contexts, table
 // upload, chunk streaming with pinned buffers, zlib inflate on a host thread.
 // There is no CPU counting path in this file: every count comes from
-// count_kernel (tdg_kernel.cuh).
+// count_kernel (tdg_kernel.cuh), or from split_count / split_count_batch
+// (tdg_split.cuh) when the splitter's trimmed reads are counted.
 #include <cuda_runtime.h>
 #include <zlib.h>
 
@@ -241,6 +242,13 @@ struct tdg_ctx {
     Buf sp_hout, sp_hflags, sp_hbase;                                                          // pinned host
     uint32_t sp_nbar = 0, sp_cutlen = 0;
     bool have_split = false;
+
+    // counting the splitter's records instead of writing them (tdg_split_count_*): the stage-2 barcode
+    // table, the matrix row of every stage-1 barcode, and a block's totals [4] + complex flag
+    Buf sc_bar, sc_rows, sc_tot;         // device
+    Buf sc_htot;                         // pinned host
+    uint32_t sc_max_row = 0;
+    bool have_split_count = false;
 
     // BGZF output of the splitter (tdg_split_bgzf, tdg_bgzf.cuh): every barcode's pending tail
     // (< 65,280 bytes) waits in bz_tail between calls
@@ -759,6 +767,105 @@ int batch_run(tdg_ctx *ctx, const char *what, const char *seqs, const uint64_t *
     if (e != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
     if (e2 != cudaSuccess) return fail(ctx, TDG_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e2));
     return TDG_OK;
+}
+
+// The front tdg_split_block and tdg_split_count_block share: the block goes to the device, its line
+// ends are found and split_records takes the decisions for its first `nrec` whole records (nrec = 0:
+// there is none, and nothing ran past the line count).  prepare(nrec) grows the caller's own buffers
+// and sets w.complex_flag before split_records is launched.  last_end (the terminator of the last
+// record's last line) is valid once the caller has synchronised the stream.
+template <class Prepare>
+int split_front(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, uint64_t max_records, tdg::SplitWork &w,
+                uint64_t &nrec, uint32_t &last_end, Prepare prepare)
+{
+    cudaStream_t st = ctx->stream;
+    const uint32_t nbar = ctx->sp_nbar;
+    int rc;
+    nrec = 0;
+    last_end = 0;
+
+    // ---- the block, and its line ends
+    const uint32_t n_tiles = (uint32_t)((n + tdg::SPLIT_TILE_BYTES - 1) / tdg::SPLIT_TILE_BYTES);
+    if ((rc = grow(ctx, ctx->sp_in, round_up(n, 16) + 16, false))) return rc;
+    if ((rc = grow(ctx, ctx->sp_tiles, (size_t)(n_tiles + 2) * sizeof(uint32_t), false))) return rc;
+    CK(cudaMemcpyAsync(ctx->sp_in.p, bytes, n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync((uint8_t *)ctx->sp_in.p + n, 0, round_up(n, 16) + 16 - n, st));
+    memset(&w, 0, sizeof w);
+    w.b.bytes = (const uint8_t *)ctx->sp_in.p;
+    w.b.n = (uint32_t)n;
+    w.b.final_block = final_block ? 1u : 0u;
+    w.b.n_tiles = n_tiles;
+    w.b.tile_count = (uint32_t *)ctx->sp_tiles.p;
+    w.b.ends = nullptr;
+    w.b.ends_cap = 0;
+    tdg::lineend_count<<<n_tiles, 256, 0, st>>>(w.b);
+    tdg::tile_scan<<<1, 1024, 0, st>>>(w.b.tile_count, n_tiles);
+    ctx->launches += 2;
+    uint32_t lines = 0;
+    CK(cudaMemcpyAsync(&lines, w.b.tile_count + n_tiles, sizeof lines, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    // the text after the last line end is a line of its own when the file ends here
+    const uint8_t last = bytes[n - 1];
+    const bool open_tail = final_block && last != '\n' && last != '\r';
+    const uint64_t total_lines = (uint64_t)lines + (open_tail ? 1 : 0);
+    uint64_t records = total_lines / 4;
+    if (records > max_records) records = max_records;
+    if (records == 0) return TDG_OK;                 // the caller supplies more bytes (or stops at the end of the file)
+    if ((rc = grow(ctx, ctx->sp_ends, (size_t)(total_lines + 1) * sizeof(uint32_t), false))) return rc;
+    w.b.ends = (uint32_t *)ctx->sp_ends.p;
+    w.b.ends_cap = lines;
+    tdg::lineend_scatter<<<n_tiles, 256, 0, st>>>(w.b);
+    ctx->launches += 1;
+    if (open_tail) {
+        const uint32_t end = (uint32_t)n;
+        CK(cudaMemcpyAsync(w.b.ends + lines, &end, sizeof end, cudaMemcpyHostToDevice, st));
+    }
+    CK(cudaMemcpyAsync(&last_end, w.b.ends + (4 * records - 1), sizeof last_end, cudaMemcpyDeviceToHost, st));
+
+    // ---- decisions
+    if ((rc = grow(ctx, ctx->sp_rec, (size_t)records * sizeof(tdg::SplitRec), false))) return rc;
+    if ((rc = grow(ctx, ctx->sp_flags, (size_t)records + 16, false))) return rc;
+    if ((rc = prepare(records))) return rc;
+    w.n_rec = (uint32_t)records;
+    w.rec = (tdg::SplitRec *)ctx->sp_rec.p;
+    w.flags = (uint8_t *)ctx->sp_flags.p;
+    w.s.t = ctx->trim;
+    w.s.bar = (const tdg::BarTable *)ctx->d_bar.p;
+    w.bar_off = (const uint32_t *)ctx->sp_tabs.p;
+    w.s.bar_len = w.bar_off + nbar + 1;
+    w.barcodes = (const uint8_t *)(w.s.bar_len + nbar);
+    w.s.cutlen = ctx->sp_cutlen;
+    w.nbar = nbar;
+    CK(cudaMemsetAsync(w.complex_flag, 0, sizeof(unsigned long long), st));
+    tdg::split_records<<<(unsigned)((records + 7) / 8), 256, 0, st>>>(w);
+    ctx->launches += 1;
+    nrec = records;
+    return TDG_OK;
+}
+
+// tdg_split_count_block / tdg_split_count_batch: every table they read is loaded and fits the matrix
+int split_count_ready(tdg_ctx *ctx)
+{
+    if (!ctx->have_split_count || !ctx->have_split || !ctx->have_trim || !ctx->have_bar)
+        return fail(ctx, TDG_ERR_STATE, "tdg_split_count_begin has not been called");
+    if (!ctx->have_tags) return fail(ctx, TDG_ERR_STATE, "tdg_set_tags has not been called");
+    if (!ctx->d_matrix) return fail(ctx, TDG_ERR_STATE, "tdg_set_matrix / tdg_bind_matrix has not been called");
+    if (ctx->max_col >= ctx->cols) return fail(ctx, TDG_ERR_ARG, "a tag column lies outside the matrix");
+    if (ctx->sc_max_row >= ctx->rows) return fail(ctx, TDG_ERR_ARG, "a barcode row lies outside the matrix");
+    return TDG_OK;
+}
+
+tdg::SplitCountArgs split_count_args(tdg_ctx *ctx)
+{
+    tdg::SplitCountArgs c;
+    c.bar = (const tdg::BarTable *)ctx->sc_bar.p;
+    c.tags = ctx->tags.t;
+    c.tags.entries = (const tdg::TagEntry *)ctx->d_entries.p;
+    c.tags.ext = (const uint64_t *)ctx->d_ext.p;
+    c.row_of = (const int32_t *)ctx->sc_rows.p;
+    c.matrix = ctx->d_matrix;
+    c.cols = ctx->cols;
+    return c;
 }
 
 #include "tdg_gzfeed.cuh"      // the host side of the device gzip feed (part of this unit)
@@ -1770,6 +1877,7 @@ int tdg_split_begin(tdg_ctx *ctx, const char *barcodes, const uint32_t *bar_off,
     int rc = need_device(ctx);
     if (rc) return rc;
     ctx->have_split = false;
+    ctx->have_split_count = false;       // its rows are per barcode of this split
     if (!ctx->have_trim) return fail(ctx, TDG_ERR_STATE, "tdg_set_trim has not been called");
     if (!ctx->have_bar) return fail(ctx, TDG_ERR_STATE, "tdg_begin_file has not been called");
     if (!bar_off || (!barcodes && nbar && bar_off[nbar] != bar_off[0])) return fail(ctx, TDG_ERR_ARG, "null argument");
@@ -1816,77 +1924,31 @@ int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_bloc
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const uint32_t nbar = ctx->sp_nbar;
-
-    // ---- the block, and its line ends
-    const uint32_t n_tiles = (uint32_t)((n + tdg::SPLIT_TILE_BYTES - 1) / tdg::SPLIT_TILE_BYTES);
-    if ((rc = grow(ctx, ctx->sp_in, round_up(n, 16) + 16, false))) return rc;
-    if ((rc = grow(ctx, ctx->sp_tiles, (size_t)(n_tiles + 2) * sizeof(uint32_t), false))) return rc;
-    CK(cudaMemcpyAsync(ctx->sp_in.p, bytes, n, cudaMemcpyHostToDevice, st));
-    CK(cudaMemsetAsync((uint8_t *)ctx->sp_in.p + n, 0, round_up(n, 16) + 16 - n, st));
     tdg::SplitWork w;
-    memset(&w, 0, sizeof w);
-    w.b.bytes = (const uint8_t *)ctx->sp_in.p;
-    w.b.n = (uint32_t)n;
-    w.b.final_block = final_block ? 1u : 0u;
-    w.b.n_tiles = n_tiles;
-    w.b.tile_count = (uint32_t *)ctx->sp_tiles.p;
-    w.b.ends = nullptr;
-    w.b.ends_cap = 0;
-    tdg::lineend_count<<<n_tiles, 256, 0, st>>>(w.b);
-    tdg::tile_scan<<<1, 1024, 0, st>>>(w.b.tile_count, n_tiles);
-    ctx->launches += 2;
-    uint32_t lines = 0;
-    CK(cudaMemcpyAsync(&lines, w.b.tile_count + n_tiles, sizeof lines, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    // the text after the last line end is a line of its own when the file ends here
-    const uint8_t last = bytes[n - 1];
-    const bool open_tail = final_block && last != '\n' && last != '\r';
-    const uint64_t total_lines = (uint64_t)lines + (open_tail ? 1 : 0);
-    uint64_t nrec = total_lines / 4;
-    if (nrec > max_records) nrec = max_records;
-    if (nrec == 0) return TDG_OK;                    // the caller supplies more bytes (or stops at the end of the file)
-    if ((rc = grow(ctx, ctx->sp_ends, (size_t)(total_lines + 1) * sizeof(uint32_t), false))) return rc;
-    w.b.ends = (uint32_t *)ctx->sp_ends.p;
-    w.b.ends_cap = lines;
-    tdg::lineend_scatter<<<n_tiles, 256, 0, st>>>(w.b);
-    ctx->launches += 1;
-    if (open_tail) {
-        const uint32_t end = (uint32_t)n;
-        CK(cudaMemcpyAsync(w.b.ends + lines, &end, sizeof end, cudaMemcpyHostToDevice, st));
-    }
+    uint64_t nrec = 0;
     uint32_t last_end = 0;
-    CK(cudaMemcpyAsync(&last_end, w.b.ends + (4 * nrec - 1), sizeof last_end, cudaMemcpyDeviceToHost, st));
-
-    // ---- decisions
-    if ((rc = grow(ctx, ctx->sp_rec, (size_t)nrec * sizeof(tdg::SplitRec), false))) return rc;
-    if ((rc = grow(ctx, ctx->sp_flags, (size_t)nrec + 16, false))) return rc;
-    const uint32_t n_rtiles = (uint32_t)((nrec + tdg::SPLIT_REC_TILE - 1) / tdg::SPLIT_REC_TILE);
-    if ((rc = grow(ctx, ctx->sp_sums, (size_t)n_rtiles * nbar * sizeof(uint32_t), false))) return rc;
-    // bar_total [nbar], bar_base [nbar + 1], complex flag
-    if ((rc = grow(ctx, ctx->sp_base, (size_t)(2 * nbar + 2) * sizeof(unsigned long long), false))) return rc;
-    if ((rc = grow(ctx, ctx->sp_hbase, (size_t)(nbar + 2) * sizeof(unsigned long long), true))) return rc;
-    if ((rc = grow(ctx, ctx->sp_hflags, (size_t)nrec + 16, true))) return rc;
-    unsigned long long *bar_total = (unsigned long long *)ctx->sp_base.p;
-    w.n_rec = (uint32_t)nrec;
-    w.rec = (tdg::SplitRec *)ctx->sp_rec.p;
-    w.flags = (uint8_t *)ctx->sp_flags.p;
-    w.bar_base = bar_total + nbar;
-    w.complex_flag = (uint32_t *)(bar_total + 2 * nbar + 1);
-    w.s.t = ctx->trim;
-    w.s.bar = (const tdg::BarTable *)ctx->d_bar.p;
-    w.bar_off = (const uint32_t *)ctx->sp_tabs.p;
-    w.s.bar_len = w.bar_off + nbar + 1;
-    w.barcodes = (const uint8_t *)(w.s.bar_len + nbar);
-    w.s.cutlen = ctx->sp_cutlen;
-    w.nbar = nbar;
-    w.n_rtiles = n_rtiles;
-    w.tile_sums = (uint32_t *)ctx->sp_sums.p;
-    CK(cudaMemsetAsync(w.complex_flag, 0, sizeof(unsigned long long), st));
-    tdg::split_records<<<(unsigned)((nrec + 7) / 8), 256, 0, st>>>(w);
+    unsigned long long *bar_total = nullptr;
+    rc = split_front(ctx, bytes, n, final_block, max_records, w, nrec, last_end, [&](uint64_t records) {
+        const uint32_t n_rtiles = (uint32_t)((records + tdg::SPLIT_REC_TILE - 1) / tdg::SPLIT_REC_TILE);
+        int rc;
+        if ((rc = grow(ctx, ctx->sp_sums, (size_t)n_rtiles * nbar * sizeof(uint32_t), false))) return rc;
+        // bar_total [nbar], bar_base [nbar + 1], complex flag
+        if ((rc = grow(ctx, ctx->sp_base, (size_t)(2 * nbar + 2) * sizeof(unsigned long long), false))) return rc;
+        if ((rc = grow(ctx, ctx->sp_hbase, (size_t)(nbar + 2) * sizeof(unsigned long long), true))) return rc;
+        if ((rc = grow(ctx, ctx->sp_hflags, (size_t)records + 16, true))) return rc;
+        bar_total = (unsigned long long *)ctx->sp_base.p;
+        w.bar_base = bar_total + nbar;
+        w.complex_flag = (uint32_t *)(bar_total + 2 * nbar + 1);
+        w.n_rtiles = n_rtiles;
+        w.tile_sums = (uint32_t *)ctx->sp_sums.p;
+        return TDG_OK;
+    });
+    if (rc || nrec == 0) return rc;
+    const uint32_t n_rtiles = w.n_rtiles;
     tdg::bar_tile_sums<<<n_rtiles, tdg::SPLIT_REC_TILE, nbar * sizeof(uint32_t), st>>>(w);
     tdg::bar_tile_scan<<<(nbar + 255) / 256, 256, 0, st>>>(w, bar_total);
     tdg::bar_bases<<<1, 32, 0, st>>>(bar_total, w.bar_base, nbar);
-    ctx->launches += 4;
+    ctx->launches += 3;
     unsigned long long *hbase = (unsigned long long *)ctx->sp_hbase.p;
     CK(cudaMemcpyAsync(hbase, w.bar_base, (size_t)(nbar + 2) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -1919,6 +1981,106 @@ int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_bloc
     *out_off = (const uint64_t *)hbase;
     *flags = (const uint8_t *)ctx->sp_hflags.p;
     return TDG_OK;
+}
+
+int tdg_split_count_begin(tdg_ctx *ctx, const char *bases, const uint32_t *off, const uint32_t *tag_off, uint32_t npat,
+                          uint32_t flags, const int32_t *row_of_barcode)
+{
+    int rc = need_device(ctx);
+    if (rc) return rc;
+    ctx->have_split_count = false;
+    if (!ctx->have_tags) return fail(ctx, TDG_ERR_STATE, "tdg_set_tags has not been called");
+    if (!ctx->d_matrix) return fail(ctx, TDG_ERR_STATE, "tdg_set_matrix / tdg_bind_matrix has not been called");
+    if (!ctx->have_split) return fail(ctx, TDG_ERR_STATE, "tdg_split_begin has not been called");
+    if (!off || !tag_off || !row_of_barcode) return fail(ctx, TDG_ERR_ARG, "null argument");
+    const uint32_t nbar = ctx->sp_nbar;
+    uint32_t max_row = 0;
+    for (uint32_t b = 0; b < nbar; b++) {
+        if (row_of_barcode[b] < 0 || (uint32_t)row_of_barcode[b] >= ctx->rows)
+            return fail(ctx, TDG_ERR_ARG, "tdg_split_count_begin: a barcode row lies outside the matrix");
+        max_row = std::max(max_row, (uint32_t)row_of_barcode[b]);
+    }
+    // the table's own rows are never read: a hit goes to the row of the record's stage-1 barcode
+    const std::vector<int32_t> zero(npat, 0);
+    std::vector<uint8_t> blob;
+    std::string why = tdg::build_bar_table(bases, off, zero.data(), tag_off, npat, flags, blob);
+    if (!why.empty()) return fail(ctx, TDG_ERR_ARG, "tdg_split_count_begin: " + why);
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(ctx->stream));          // earlier kernels read the old tables
+    if ((rc = grow(ctx, ctx->sc_bar, round_up(blob.size(), 16), false)) || (rc = grow(ctx, ctx->sc_rows, nbar * sizeof(int32_t), false)) ||
+        (rc = grow_exact(ctx, ctx->sc_tot, 5 * sizeof(unsigned long long), false)) ||
+        (rc = grow_exact(ctx, ctx->sc_htot, 5 * sizeof(unsigned long long), true)))
+        return rc;
+    CK(cudaMemcpy(ctx->sc_bar.p, blob.data(), blob.size(), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(ctx->sc_rows.p, row_of_barcode, nbar * sizeof(int32_t), cudaMemcpyHostToDevice));
+    ctx->sc_max_row = max_row;
+    ctx->have_split_count = true;
+    return TDG_OK;
+}
+
+int tdg_split_count_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, uint64_t max_records,
+                          uint64_t *n_records, uint64_t *consumed, int *needs_host, uint64_t totals[4])
+{
+    int rc = need_device(ctx);
+    if (rc) return rc;
+    if ((rc = split_count_ready(ctx))) return rc;
+    if (!n_records || !consumed || !needs_host || !totals || (!bytes && n)) return fail(ctx, TDG_ERR_ARG, "null argument");
+    if (n > ((size_t)1 << 30)) return fail(ctx, TDG_ERR_ARG, "tdg_split_count_block: at most 1 GiB per block");
+    *n_records = 0;
+    *consumed = 0;
+    *needs_host = 0;
+    for (int k = 0; k < 4; k++) totals[k] = 0;
+    if (n == 0 || max_records == 0) return TDG_OK;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    unsigned long long *d_tot = (unsigned long long *)ctx->sc_tot.p;     // totals [4], complex flag
+    tdg::SplitWork w;
+    uint64_t nrec = 0;
+    uint32_t last_end = 0;
+    bool timed;                                      // tdg_timing_*: the block's upload and kernels as one
+    if ((rc = timed_start(ctx, timed))) return rc;
+    rc = split_front(ctx, bytes, n, final_block, max_records, w, nrec, last_end, [&](uint64_t) {
+        w.complex_flag = (uint32_t *)(d_tot + 4);
+        CK(cudaMemsetAsync(d_tot, 0, 4 * sizeof(unsigned long long), st));
+        return TDG_OK;
+    });
+    if (!rc && nrec) {
+        tdg::split_count<<<(unsigned)((nrec + 255) / 256), 256, 0, st>>>(w, split_count_args(ctx), d_tot);
+        ctx->launches += 1;
+    }
+    if (timed) CK(cudaEventRecord(ctx->tev[ctx->tev_used++], st));
+    if (rc || nrec == 0) return rc;
+    const unsigned long long *h = (const unsigned long long *)ctx->sc_htot.p;
+    CK(cudaMemcpyAsync(ctx->sc_htot.p, d_tot, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    *n_records = nrec;
+    *consumed = last_end >= n ? n : (uint64_t)last_end + 1;
+    if ((uint32_t)h[4] != 0) {                       // split_count left the matrix alone
+        *needs_host = 1;
+        return TDG_OK;
+    }
+    for (int k = 0; k < 4; k++) totals[k] = h[k];
+    return TDG_OK;
+}
+
+int tdg_split_count_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, const int32_t *bar, uint32_t n, int32_t *col_out)
+{
+    int rc = need_device(ctx);
+    if (rc) return rc;
+    if ((rc = split_count_ready(ctx))) return rc;
+    if (n == 0) return TDG_OK;
+    if (!off || !bar || !col_out || (!seqs && off[n] != off[0])) return fail(ctx, TDG_ERR_ARG, "null argument");
+    for (uint32_t i = 0; i < n; i++) {
+        if (bar[i] < 0 || (uint32_t)bar[i] >= ctx->sp_nbar) return fail(ctx, TDG_ERR_ARG, "barcode index out of range");
+        if (off[i + 1] < off[i]) return fail(ctx, TDG_ERR_ARG, "offsets must be non-decreasing");
+    }
+    CK(cudaSetDevice(ctx->device));
+    return batch_run(ctx, "tdg_split_count_batch", seqs, off, n, {{bar, nullptr, n * sizeof(int32_t)}, {nullptr, col_out, n * sizeof(int32_t)}},
+                     [&](const uint8_t *d, const unsigned long long *d_off, uint8_t *const *part) {
+                         tdg::split_count_batch<<<(n + 127) / 128, 128, 0, ctx->stream>>>(d, d_off, (const int32_t *)part[0], n,
+                                                                                         split_count_args(ctx), (int32_t *)part[1]);
+                     });
 }
 
 // ---------------------------------------------------------------------------

@@ -20,6 +20,13 @@
 //   bar_tile_scan   per barcode: exclusive prefix over the tiles, totals, barcode bases
 //   split_write     per tile: in-order offsets of its records inside their barcode's stream,
 //                   then the bytes
+//
+// Counting the trimmed reads without writing them (tdg_split_count_block): the same front up to
+// split_records, then
+//   split_count     one thread per record: find_tags_fastq's matcher (match_line, tdg_match.h) on
+//                   the stripped slice sequence[slice1:slice2] -- what the counter would read back
+//                   from the barcode's output file -- with the stage-2 table (blank barcode), the
+//                   hit added to the matrix row of the record's barcode; totals of the block
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -64,6 +71,15 @@ struct SplitWork {
     uint32_t *tile_sums;      // [n_rtiles][nbar] bytes, then exclusive prefix per barcode
     unsigned long long *bar_base;   // [nbar + 1] start of every barcode's stream in out
     uint8_t *out;
+};
+
+// The counter's side of split_count / split_count_batch
+struct SplitCountArgs {
+    const BarTable *bar;      // stage-2 barcode+cutsite table: find_tags_fastq(F_i, [''], tags, cutsite)
+    TagTable tags;
+    const int32_t *row_of;    // [nbar] matrix row of every stage-1 barcode
+    int32_t *matrix;
+    uint32_t cols;
 };
 
 #if defined(__CUDACC__)
@@ -407,6 +423,82 @@ __global__ void __launch_bounds__(SPLIT_REC_TILE) split_write(const SplitWork w)
         split_copy(dst, s + ql, ql_len, lane, false);               // quality[slice1:slice2]  (:1351)
         if (lane == 0) dst[ql_len] = '\n';
     }
+}
+
+// The counter's rule on one stage-2 line t (stripped): its tag column, or -1.  The window ends where t
+// ends, so a tag cannot reach past slice2.  Case is folded by the matcher (t.upper()).
+__device__ __forceinline__ int32_t split_count_col(const SplitCountArgs &c, const uint8_t *p, uint32_t len)
+{
+    GlobalBytes f;
+    f.p = p;
+    f.limit = len;
+    const BarEntry *bent = (const BarEntry *)((const uint8_t *)c.bar + sizeof(BarTable));
+    const MatchResult m = match_line(f, c.bar, bent, c.tags);
+    return m.row >= 0 ? m.col : -1;
+}
+
+// counts[row_of[bar]][col] += 1 for every lane that has a hit (bar >= 0, col >= 0); lanes on the same
+// cell add together, once.  Every lane of the warp must call it.
+__device__ __forceinline__ void split_count_add(const SplitCountArgs &c, int32_t bar, int32_t col)
+{
+    const bool hit = bar >= 0 && col >= 0;
+    // cells < 2^32 - 1 (tdg_set_matrix): the all-ones key is no cell
+    const uint32_t cell = hit ? (uint32_t)c.row_of[bar] * c.cols + (uint32_t)col : 0xFFFFFFFFu;
+    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
+    if (hit && (threadIdx.x & 31u) == (uint32_t)__ffs(peers) - 1u) atomicAdd(c.matrix + cell, (int)__popc(peers));
+}
+
+// One thread per record of the block (after split_records): the trimmed sequence slice, stripped,
+// through the counter's matcher into the matrix.  totals[0..3] gain the block's reads, reads with
+// barcode and cut site, reads clipped on the 3' end and reads with a tag.  A block split_records left
+// to the host (complex flag) is not counted at all: the host counts its records itself.
+__global__ void __launch_bounds__(256) split_count(const SplitWork w, const SplitCountArgs c, unsigned long long *totals)
+{
+    if (*w.complex_flag) return;
+    __shared__ uint32_t part[4][8];
+    const uint32_t r = blockIdx.x * 256u + threadIdx.x;
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    int32_t bar = -1, col = -1;
+    uint32_t clipped = 0;
+    if (r < w.n_rec) {
+        const SplitRec rec = w.rec[r];
+        bar = rec.bar;
+        if (bar >= 0) {
+            clipped = (w.flags[r] & SPLIT_FLAG_CLIP) ? 1u : 0u;
+            // t = s[slice1:slice2].strip(): blanks can surface inside the slice when the cut site is empty
+            uint32_t lo = rec.seq, hi = rec.seq + rec.seq_len;
+            split_strip(w.b.bytes, lo, hi);
+            col = split_count_col(c, w.b.bytes + lo, hi - lo);
+        }
+    }
+    split_count_add(c, bar, col);
+    const uint32_t v[4] = {r < w.n_rec ? 1u : 0u, bar >= 0 ? 1u : 0u, clipped, col >= 0 ? 1u : 0u};
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const uint32_t s = __reduce_add_sync(0xFFFFFFFFu, v[k]);
+        if (lane == 0) part[k][warp] = s;
+    }
+    __syncthreads();
+    if (threadIdx.x < 4) {
+        uint32_t s = 0;
+        for (int i = 0; i < 8; i++) s += part[threadIdx.x][i];
+        if (s) atomicAdd(totals + threadIdx.x, (unsigned long long)s);
+    }
+}
+
+// The same count for stage-2 lines the host cut itself (blocks left to the host):
+// t_i = seqs[off[i] .. off[i+1]), stripped and upper-cased by Python; bar[i] >= 0 its stage-1 barcode.
+__global__ void __launch_bounds__(128) split_count_batch(const uint8_t *seqs, const unsigned long long *off, const int32_t *bar,
+                                                         uint32_t n, const SplitCountArgs c, int32_t *col_out)
+{
+    const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    int32_t b = -1, col = -1;
+    if (r < n) {
+        b = bar[r];
+        col = split_count_col(c, seqs + off[r], (uint32_t)(off[r + 1] - off[r]));
+        col_out[r] = col;
+    }
+    split_count_add(c, b, col);
 }
 
 #endif  // __CUDACC__

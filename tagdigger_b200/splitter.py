@@ -16,6 +16,10 @@ With ``bgzf=True`` every output file is BGZF (what bgzip writes) instead of plai
 both paths go to the device encoder (``tdg_split_bgzf``, csrc/tdg_bgzf.cuh), which cuts each file's
 stream into 65,280-byte members whatever the blocks were, and decompressed each file equals the plain
 one byte for byte.
+
+``count_trimmed_file`` runs the same block loop and the same device front, but counts instead of
+writing: every barcode's trimmed reads go through find_tags_fastq's matcher with a blank barcode
+(``tdg_split_count_block``), as counting the output files would -- without the files.
 """
 
 import csv
@@ -80,26 +84,15 @@ class _Progress:
         c[0] += n
 
 
-def _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress):
-    """Complete records of ``text`` (universal newlines), decided in blocks on the GPU and
-    written by Python: the path for text the device does not slice itself."""
-    def flush(block):
-        seqs = [rec[1] for rec in block]
-        raws = [s.encode("utf-8") for s in seqs]
+def _decided_blocks(eng, text, barlen, cutlen):
+    """Complete records of ``text`` (universal newlines), decided in blocks of BLOCK_READS on the
+    GPU: the path for text the device does not slice itself.  Yields lists of (comment1, sequence,
+    comment2, quality, barcode index or -1, slice2 in characters or None for no 3' trim)."""
+    def decide(block):
+        raws = [rec[1].encode("utf-8") for rec in block]
         bars, cuts = eng.split_batch(raws, barlen, cutlen)
-        for (comment1, sequence, comment2, quality), raw, b, cut in zip(block, raws, bars.tolist(), cuts.tolist()):
-            clipped = 0
-            if b > -1:
-                slice1 = barlen[b]
-                if cut == 999:
-                    slice2 = len(sequence)
-                else:
-                    slice2 = _byte_to_char_index(sequence, raw, cut)
-                    clipped = 1
-                head = comment1 + barcodes[b] + "\n"
-                rec = head + sequence[slice1:slice2] + "\n" + ("+\n" if comment2 == "+" else head) + quality[slice1:slice2] + "\n"
-                outcons[b].write(rec.encode("utf-8"))
-            progress.one(1 if b > -1 else 0, clipped)
+        return [rec + (b, None if cut == 999 else _byte_to_char_index(rec[1], raw, cut))
+                for rec, raw, b, cut in zip(block, raws, bars.tolist(), cuts.tolist())]
 
     block = []
     comment1 = sequence = comment2 = ""
@@ -114,57 +107,80 @@ def _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress):
         else:
             block.append((comment1, sequence, comment2, line.strip()))
             if len(block) >= BLOCK_READS:
-                flush(block)
+                yield decide(block)
                 block = []
     if block:
-        flush(block)
+        yield decide(block)
 
 
-def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=hostio.adapters["PstI-MspI-Hall"],
-                    maxreads=500000000, device=None, bgzf=False):
+def _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress):
+    """Complete records of ``text``, decided on the GPU and written by Python."""
+    for block in _decided_blocks(eng, text, barlen, cutlen):
+        for comment1, sequence, comment2, quality, b, cut in block:
+            clipped = 0
+            if b > -1:
+                slice1 = barlen[b]
+                if cut is None:
+                    slice2 = len(sequence)
+                else:
+                    slice2 = cut
+                    clipped = 1
+                head = comment1 + barcodes[b] + "\n"
+                rec = head + sequence[slice1:slice2] + "\n" + ("+\n" if comment2 == "+" else head) + quality[slice1:slice2] + "\n"
+                outcons[b].write(rec.encode("utf-8"))
+            progress.one(1 if b > -1 else 0, clipped)
+
+
+def _check_args(cutsite, barcodes, adapter):
+    """barcodeSplitter's asserts (:1288-1293)."""
     assert set(cutsite) <= hostio.BASES, "Only ACGT cut sites allowed."
     assert all([set(bc) <= hostio.BASES for bc in barcodes]), "Found non-ACGT barcodes."
     assert len(adapter) == 2
     assert all([set(a[0]) <= set("ACGT^") for a in adapter])
     assert set(adapter[0][1]) <= hostio.BASES
     assert set(adapter[1][1]) <= set("[barcode]ACGT")
-    if bgzf:
-        # the counters (counting.py, the reference's find_tags_fastq) take a file for gzip by the last
-        # two characters of its name: a BGZF file under another name would be read as text
-        plain = [name for name in outputFiles if name[-2:].lower() != "gz"]
-        if plain:
-            raise ValueError("BGZF output needs file names ending in 'gz': %s" % ", ".join(plain))
 
-    print("Building indices for rapid searching...")
-    barlen = [len(bc) for bc in barcodes]
+
+def _split_patterns(barcodes, cutsite):
     barcut = hostio.combine_barcode_and_cutsite(barcodes, cutsite)
-    patterns = matchset.effective_set(barcut, len(barcut))          # raises like build_sequence_tree
-    eng = get_engine(device)
-    tables = trimming.trim_tables(adapter, barcodes)                 # prints the reference's overlap messages
+    return matchset.effective_set(barcut, len(barcut))               # raises like build_sequence_tree
+
+
+def _load_split(eng, patterns, barcodes, cutsite, adapter):
+    """The splitter's tables on the device: barcode+cutsite lookup, trim tables (printing the
+    reference's overlap messages), barcode strings."""
+    tables = trimming.trim_tables(adapter, barcodes)
     eng.begin_file(patterns.patterns, patterns.index, [len(p) for p in patterns.patterns], any_base=patterns.any_base)
     eng.set_trim(tables[0], tables[1], tables[2], tables[3], tables[4])
-    cutlen = len(cutsite)
-    eng.split_begin(barcodes, cutlen)
-    if bgzf:
-        eng.split_bgzf(True)
-    print("Done with indexing setup.")
-    print(inputFile)
+    eng.split_begin(barcodes, len(cutsite))
 
+
+def _open_input(inputFile):
     open(inputFile, "rb").close()                                    # the reference's OSError for a missing file
     try:
-        feed = _native.Feed(inputFile, inputFile[-2:].lower() == "gz")
+        return _native.Feed(inputFile, inputFile[-2:].lower() == "gz")
     except _native.TdgError as e:
         raise _gzip_exception(e.message) if e.code == _native.TDG_ERR_GZIP else OSError(e.message)
-    outcons = [open(name, mode="wb") for name in outputFiles]
-    progress = _Progress(inputFile)
+
+
+def _feed_error(e):
+    """The exception the reference's reading raises for a TdgError of the block loop."""
+    if e.code == _native.TDG_ERR_GZIP:
+        return _gzip_exception(e.message)
+    if e.code == _native.TDG_ERR_IO:
+        return OSError(e.message)
+    return e
+
+
+def _block_loop(eng, feed, maxreads, device_block, host_block):
+    """The splitter's loop over one input: blocks of up to BLOCK_BYTES from ``feed`` in pinned memory,
+    the unconsumed tail carried to the front of the next block, the buffer doubled for a record longer
+    than it.  ``device_block(buf, fill, eof, left)`` runs one block on the device and returns (records,
+    consumed bytes, needs_host); ``host_block(text)`` takes the records of a block the device left to
+    the host."""
     left = _native.limit_from_maxreads(maxreads)
     cap = 2 * BLOCK_BYTES
     buf = eng.host_alloc(cap)
-    pool = ThreadPoolExecutor(max_workers=8)
-
-    def write(pieces):
-        list(pool.map(lambda t: t[0].write(t[1]), [(o, p) for o, p in zip(outcons, pieces) if len(p)]))
-
     try:
         fill, eof = 0, False
         while left > 0:
@@ -172,7 +188,7 @@ def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=h
                 got = feed.read_into(buf + fill, min(BLOCK_BYTES, cap - fill))
                 eof = got == 0
                 fill += got
-            nrec, used, needs_host, pieces, flags = eng.split_block(buf, fill, eof, left)
+            nrec, used, needs_host = device_block(buf, fill, eof, left)
             if nrec == 0:
                 if eof:
                     break                                    # what is left is not a whole record
@@ -183,35 +199,120 @@ def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=h
                     buf, cap = bigger, 2 * cap
                 continue
             if needs_host:
-                text = ctypes.string_at(buf, used).decode("utf-8")
-                if bgzf:
-                    parts = [io.BytesIO() for _ in outcons]
-                    _host_records(eng, text, barcodes, barlen, cutlen, parts, progress)
-                    write(eng.bgzf_append([p.getvalue() for p in parts]))
-                else:
-                    _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress)
-            else:
-                write(pieces)
-                progress.many(flags)
+                host_block(ctypes.string_at(buf, used).decode("utf-8"))
             left -= nrec
             fill -= used
             if fill:
                 ctypes.memmove(buf, buf + used, fill)
+    finally:
+        eng.host_free(buf)
+
+
+def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=hostio.adapters["PstI-MspI-Hall"],
+                    maxreads=500000000, device=None, bgzf=False):
+    _check_args(cutsite, barcodes, adapter)
+    if bgzf:
+        # the counters (counting.py, the reference's find_tags_fastq) take a file for gzip by the last
+        # two characters of its name: a BGZF file under another name would be read as text
+        plain = [name for name in outputFiles if name[-2:].lower() != "gz"]
+        if plain:
+            raise ValueError("BGZF output needs file names ending in 'gz': %s" % ", ".join(plain))
+
+    print("Building indices for rapid searching...")
+    barlen = [len(bc) for bc in barcodes]
+    patterns = _split_patterns(barcodes, cutsite)
+    eng = get_engine(device)
+    _load_split(eng, patterns, barcodes, cutsite, adapter)
+    cutlen = len(cutsite)
+    if bgzf:
+        eng.split_bgzf(True)
+    print("Done with indexing setup.")
+    print(inputFile)
+
+    feed = _open_input(inputFile)
+    outcons = [open(name, mode="wb") for name in outputFiles]
+    progress = _Progress(inputFile)
+    pool = ThreadPoolExecutor(max_workers=8)
+
+    def write(pieces):
+        list(pool.map(lambda t: t[0].write(t[1]), [(o, p) for o, p in zip(outcons, pieces) if len(p)]))
+
+    def device_block(buf, fill, eof, left):
+        nrec, used, needs_host, pieces, flags = eng.split_block(buf, fill, eof, left)
+        if nrec and not needs_host:
+            write(pieces)
+            progress.many(flags)
+        return nrec, used, needs_host
+
+    def host_block(text):
+        if bgzf:
+            parts = [io.BytesIO() for _ in outcons]
+            _host_records(eng, text, barcodes, barlen, cutlen, parts, progress)
+            write(eng.bgzf_append([p.getvalue() for p in parts]))
+        else:
+            _host_records(eng, text, barcodes, barlen, cutlen, outcons, progress)
+
+    try:
+        _block_loop(eng, feed, maxreads, device_block, host_block)
         if bgzf:
             write(eng.bgzf_finish())
     except _native.TdgError as e:
-        if e.code == _native.TDG_ERR_GZIP:
-            raise _gzip_exception(e.message)
-        if e.code == _native.TDG_ERR_IO:
-            raise OSError(e.message)
-        raise
+        raise _feed_error(e)
     finally:
         pool.shutdown()
-        eng.host_free(buf)
         feed.close()
         for o in outcons:
             o.close()
     return None
+
+
+def count_trimmed_file(eng, inputFile, barcodes, rows, plan, cutsite="TGCAG", adapter=hostio.adapters["PstI-MspI-Hall"],
+                       maxreads=500000000):
+    """barcodeSplitter(inputFile, barcodes, files, cutsite, adapter, maxreads), then
+    find_tags_fastq(files[b], [''], tags, stage-2 cut site) added into matrix row ``rows[b]`` for every
+    barcode b -- without the files: the splitter's device front decides every record, and the
+    counter's matcher runs on the slice the file would hold (``tdg_split_count_block``).  ``plan`` is
+    ``matchset.plan([''], tags, stage-2 cut site)``; the engine must hold its tags (``set_tags``) and
+    the matrix.  Blocks with non-ASCII sequence or quality lines are cut by Python, as
+    barcodeSplitter writes them, and counted on the GPU (``tdg_split_count_batch``).
+
+    Returns [reads, reads with barcode and cut site, reads clipped on the 3' end, reads with tag]."""
+    _check_args(cutsite, barcodes, adapter)
+    barlen = [len(bc) for bc in barcodes]
+    cutlen = len(cutsite)
+    _load_split(eng, _split_patterns(barcodes, cutsite), barcodes, cutsite, adapter)
+    eng.split_count_begin(plan.bar.patterns, plan.bar_tag_off, rows, any_base=plan.bar.any_base)
+    feed = _open_input(inputFile)
+    tot = [0, 0, 0, 0]
+
+    def device_block(buf, fill, eof, left):
+        nrec, used, needs_host, t = eng.split_count_block(buf, fill, eof, left)
+        if nrec and not needs_host:
+            for k in range(4):
+                tot[k] += t[k]
+        return nrec, used, needs_host
+
+    def host_block(text):
+        for block in _decided_blocks(eng, text, barlen, cutlen):
+            seqs, bars = [], []
+            for _c1, sequence, _c2, _q, b, cut in block:
+                tot[0] += 1
+                if b > -1:
+                    tot[1] += 1
+                    tot[2] += cut is not None
+                    # the line find_tags_fastq reads back from barcode b's file: line.strip().upper()
+                    seqs.append(sequence[barlen[b]:len(sequence) if cut is None else cut].strip().upper())
+                    bars.append(b)
+            if seqs:
+                tot[3] += int(np.count_nonzero(eng.split_count_batch(seqs, bars) >= 0))
+
+    try:
+        _block_loop(eng, feed, maxreads, device_block, host_block)
+    except _native.TdgError as e:
+        raise _feed_error(e)
+    finally:
+        feed.close()
+    return tot
 
 
 def writeMD5sums(filelist, outfile):

@@ -4,6 +4,11 @@ tagdigger_script.py (/root/reference/tagdigger_script.py:10-35) on the GPU path.
 
     python -m tagdigger_b200.tagdigger_script -e PstI --MergedTags tags.csv -b key.csv -o counts.csv [-g geno.csv]
     torchrun --nproc-per-node 8 -m tagdigger_b200.tagdigger_script ...      # files dealt to 8 GPUs, one all-reduce
+    python -m tagdigger_b200.tagdigger_script -e PstI --MergedTags tags.csv -b key.csv -o counts.csv --adapter PstI-MspI-Hall
+
+With --adapter the key lists the raw library files (File, Barcode, Sample): every file is split by
+barcode and trimmed as barcode_splitter_script -a would, and the trimmed reads are counted with a blank
+barcode -- the two-stage run in one pass on the GPU, without the split files.
 
 The flow is the reference's (:37-133): resolve the cut site, change directory,
 read the tags in exactly one format, sanitise them, read the key file, sniff
@@ -42,6 +47,9 @@ def build_parser():
     p.add_argument("-b", "--barcodefile", help="Name of barcode key file", required=True)
     p.add_argument("-o", "--outputcounts", help="Output file name for read counts", required=True)
     p.add_argument("-g", "--outputgen", help="Output file name for numeric genotypes")
+    p.add_argument("--adapter", help="Name of an adapter set: split and trim every FASTQ file by barcode as "
+                   "barcode_splitter_script -a would (its cut site from the set's enzyme) and count the trimmed reads, "
+                   "without writing the split files", choices=sorted(tdf.adapters.keys()))
     return p
 
 
@@ -135,7 +143,7 @@ def main(argv=None):
         reduce = engine_reduce                      # one ncclAllReduce on the counting stream
         gather = dist_gather
     samples, counts = tdf.count_files(bckeys, tags[1], cutsite=cutsite, rank=rank, world=world, reduce=reduce,
-                                      gather=gather, as_array=True)
+                                      gather=gather, as_array=True, adapter=args.adapter)
     if rank == 0:
         tdf.writeCounts(args.outputcounts, counts, samples, tags[0])
         if args.outputgen is not None:
