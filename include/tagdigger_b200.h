@@ -327,6 +327,16 @@ int         tdg_split_count_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, 
                                   int *needs_host, uint64_t totals[4]);
 int         tdg_split_count_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, const int32_t *bar,
                                   uint32_t n, int32_t *col_out);
+/* tdg_split_count_device: tdg_split_count_block on bytes already in DEVICE memory (no alignment or
+ * padding asked of dev_bytes; the block is copied device to device into the context's own padded
+ * buffer, so there is no host-to-device copy).  Same arguments, limits (at most 1 GiB per call: a
+ * longer text is walked in calls that each start at the previous call's *consumed) and results; with
+ * *needs_host = 1 the caller copies dev_bytes[0 .. consumed) to the host and handles those records as
+ * it would for tdg_split_count_block.  Used to count one rank's byte range of a file that is sharded
+ * across GPUs after the range was loaded and its lines counted on the device. */
+int         tdg_split_count_device(tdg_ctx *ctx, const void *dev_bytes, size_t n, int final_block,
+                                   uint64_t max_records, uint64_t *n_records, uint64_t *consumed,
+                                   int *needs_host, uint64_t totals[4]);
 
 /* BGZF output files for the streaming splitter (the reference writes plain text only).  Every
  * barcode's file is the series of gzip members bgzip writes: member k holds bytes

@@ -38,7 +38,7 @@ tdg_count_lines_device tdg_count_file tdg_count_file2 tdg_last_file_info tdg_gz_
 tdg_matrix_device_ptr tdg_stream tdg_stream_wait tdg_other_stream_wait tdg_host_alloc
 tdg_host_free tdg_device_alloc tdg_device_free tdg_memcpy_h2d tdg_memcpy_d2h tdg_launch_count
 tdg_timing_begin tdg_timing_end tdg_set_trim tdg_trim_batch tdg_split_batch tdg_split_begin tdg_split_block
-tdg_split_count_begin tdg_split_count_block tdg_split_count_batch tdg_split_bgzf tdg_bgzf_append tdg_bgzf_finish tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
+tdg_split_count_begin tdg_split_count_block tdg_split_count_device tdg_split_count_batch tdg_split_bgzf tdg_bgzf_append tdg_bgzf_finish tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
 
 
 class TdgError(RuntimeError):
@@ -145,6 +145,7 @@ def lib():
                                   ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp)]),
         "tdg_split_count_begin": (i32, [vp, vp, vp, vp, u32, u32, vp]),
         "tdg_split_count_block": (i32, [vp, vp, sz, i32, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32), vp]),
+        "tdg_split_count_device": (i32, [vp, vp, sz, i32, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32), vp]),
         "tdg_split_count_batch": (i32, [vp, vp, vp, vp, u32, vp]),
         "tdg_split_bgzf": (i32, [vp, i32]),
         "tdg_bgzf_append": (i32, [vp, vp, vp, ctypes.POINTER(vp), ctypes.POINTER(vp)]),
@@ -546,11 +547,19 @@ class Engine(object):
         """split_block that counts the trimmed reads into the matrix instead of returning them.
         Returns (records, consumed bytes, needs_host, totals): totals = [reads, with barcode and cut
         site, clipped on the 3' end, with tag] of the block; None when needs_host (nothing counted)."""
+        return self._split_count(self._L.tdg_split_count_block, ptr, n, final, max_records)
+
+    def split_count_device(self, dev_ptr, n, final, max_records):
+        """split_count_block on ``n`` bytes already in device memory at ``dev_ptr`` (any alignment;
+        at most 1 GiB per call).  Same return value."""
+        return self._split_count(self._L.tdg_split_count_device, dev_ptr, n, final, max_records)
+
+    def _split_count(self, fn, ptr, n, final, max_records):
         u64 = ctypes.c_uint64
         nrec, used, host = u64(0), u64(0), ctypes.c_int(0)
         tot = np.zeros(4, dtype=np.uint64)
-        self._ck(self._L.tdg_split_count_block(self._h, ptr, n, 1 if final else 0, min(int(max_records), (1 << 64) - 1),
-                                               ctypes.byref(nrec), ctypes.byref(used), ctypes.byref(host), tot.ctypes.data))
+        self._ck(fn(self._h, ptr, n, 1 if final else 0, min(int(max_records), (1 << 64) - 1),
+                    ctypes.byref(nrec), ctypes.byref(used), ctypes.byref(host), tot.ctypes.data))
         if host.value:
             return nrec.value, used.value, True, None
         self.note_hits(int(tot[3]))

@@ -9,6 +9,7 @@ reads on the CPU.
 import ctypes
 import gzip
 import os
+import re
 import zlib
 
 import numpy as np
@@ -222,13 +223,15 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
     ``find_tags_fastq(file, [''], tags, cutsite)`` into its sample's row -- in one pass per file on the
     GPU, without writing the split files (:func:`splitter.count_trimmed_file`).  ``split_cutsite``
     defaults to the cut site of the adapter set's enzyme, as barcode_splitter_script derives it.  Files
-    are dealt whole to the ranks.  ``totals`` then receives ``[reads, with barcode and cut site, clipped
-    on the 3' end, with tag]``."""
+    are dealt to the ranks, or sharded by byte range as above (:func:`count_trimmed_range`, which lines
+    the ranges up on record boundaries); sharded files are counted first.  ``totals`` then receives
+    ``[reads, with barcode and cut site, clipped on the 3' end, with tag]``, for a sharded file on every
+    rank and summed over the ranks."""
     files = sorted(bckeys.keys())
     samples, rows = global_rows(bckeys)
     if adapter is not None:
         eng = _count_trimmed_files(bckeys, files, rows, len(samples), tags, cutsite, maxreads, device, rank, world,
-                                   totals, adapter, split_cutsite, split_maxreads)
+                                   totals, adapter, split_cutsite, split_maxreads, gather)
         return _result(eng, samples, len(tags), world, reduce, as_array)
     limit = _native.limit_from_maxreads(maxreads)
     plans = {}
@@ -246,9 +249,7 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
     first = plans[files[0]]
     eng.set_tags(first.tags.patterns, first.tags.index, any_base=first.tags.any_base)
     eng.set_matrix(len(samples), ntags)
-    # Fewer files than GPUs: a plain (uncompressed) file is cut into one byte range per rank
-    # (cut at line ends); otherwise whole files are dealt to the ranks.
-    split = [f for f in files if world > 1 and len(files) < world and not _is_gz(f) and shardable(f, world)]
+    split = shard_files(files, world)
     for f in split:
         load_plan(eng, plans[f], row_of=rows[f], set_tags=False)
         tot = count_file_range(eng, f, rank, world, limit, gather)
@@ -276,7 +277,7 @@ def _result(eng, samples, ntags, world, reduce, as_array):
 
 
 def _count_trimmed_files(bckeys, files, rows, nrows, tags, cutsite, maxreads, device, rank, world, totals, adapter,
-                         split_cutsite, split_maxreads):
+                         split_cutsite, split_maxreads, gather):
     """count_files with ``adapter``: this rank's files through splitter.count_trimmed_file.  Returns the engine."""
     from . import hostio, splitter
     if not isinstance(adapter, str) or adapter not in hostio.adapters:
@@ -298,7 +299,13 @@ def _count_trimmed_files(bckeys, files, rows, nrows, tags, cutsite, maxreads, de
     eng = get_engine(device)
     eng.set_tags(plan.tags.patterns, plan.tags.index, any_base=plan.tags.any_base)
     eng.set_matrix(nrows, plan.ntags)
-    for f in assign_files(files, rank, world):
+    split = shard_files(files, world)
+    for f in split:
+        tot = count_trimmed_range(eng, f, rank, world, gather, bckeys[f][0], rows[f], plan, split_cutsite, adapter_seqs,
+                                  split_maxreads)
+        if tot is not None and totals is not None:
+            totals[f] = tot
+    for f in assign_files([f for f in files if f not in split], rank, world):
         tot = splitter.count_trimmed_file(eng, f, bckeys[f][0], rows[f], plan, cutsite=split_cutsite, adapter=adapter_seqs,
                                           maxreads=split_maxreads)
         print("{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}".format(f, *tot))
@@ -308,6 +315,15 @@ def _count_trimmed_files(bckeys, files, rows, nrows, tags, cutsite, maxreads, de
 
 
 SHARD_MIN_BYTES = 1 << 20     # files smaller than this per rank are not worth cutting up
+
+
+def shard_files(files, world):
+    """The files of a key that count_files cuts into one byte range per rank (both counting modes):
+    with fewer files than ranks, every plain (uncompressed) file that is large enough.  The other
+    files are dealt whole to the ranks."""
+    if world <= 1 or len(files) >= world:
+        return []
+    return [f for f in files if not _is_gz(f) and shardable(f, world)]
 
 
 def shardable(f, world):
@@ -369,7 +385,25 @@ def count_file_range(eng, path, rank, world, limit, gather):
         return tot
     lo, hi = bounds[rank], bounds[rank + 1]
     n = hi - lo
-    cap = (n + _native.TDG_TILE_BYTES - 1) // _native.TDG_TILE_BYTES * _native.TDG_TILE_BYTES + _native.TDG_HALO_BYTES
+    dev = _load_range(eng, path, lo, n)
+    try:
+        lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
+        every = gather([lines])
+        base = sum(x[0] for x in every[:rank])
+        eng.reset_file()
+        eng.count_device(dev, n, base, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF, limit)
+        tot = eng.file_totals()
+    finally:
+        eng.device_free(dev)
+    print("{0} [bytes {1}-{2}]: Reads: {3} With barcode and cut site: {4} With tag: {5}".format(path, lo, hi, *tot[:3]))
+    return tot
+
+
+def _load_range(eng, path, lo, n, extra=0):
+    """Bytes [lo, lo + n) of ``path`` in a fresh device allocation padded as tdg_count_device asks, with
+    ``extra`` more bytes of room behind them; read with pread through one pinned buffer of at most
+    256 MiB.  Returns the device pointer (free with device_free)."""
+    cap = (n + extra + _native.TDG_TILE_BYTES - 1) // _native.TDG_TILE_BYTES * _native.TDG_TILE_BYTES + _native.TDG_HALO_BYTES
     dev = eng.device_alloc(cap)
     try:
         piece = 256 << 20
@@ -387,15 +421,139 @@ def count_file_range(eng, path, rank, world, limit, gather):
                     done += got
         finally:
             eng.host_free(host)
-        lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
-        every = gather([lines])
-        base = sum(x[0] for x in every[:rank])
-        eng.reset_file()
-        eng.count_device(dev, n, base, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF, limit)
-        tot = eng.file_totals()
-    finally:
+    except BaseException:
         eng.device_free(dev)
-    print("{0} [bytes {1}-{2}]: Reads: {3} With barcode and cut site: {4} With tag: {5}".format(path, lo, hi, *tot[:3]))
+        raise
+    return dev
+
+
+HEAD_CAP = 1 << 20            # a range whose first three lines are longer than this is not sharded
+_TERMINATOR = re.compile(rb"\r\n|\r|\n")
+
+
+def line_ends(data, k, whole=True):
+    """Offsets just past the first ``k`` line terminators of ``data`` (universal newlines: '\\n', '\\r\\n'
+    or a lone '\\r'); fewer when there are fewer.  A '\\r' that is the last byte ends a line only when
+    ``whole`` (nothing follows data that could make it '\\r\\n')."""
+    ends = []
+    for m in _TERMINATOR.finditer(data):
+        if len(ends) == k or (m.end() == len(data) and m.group() == b"\r" and not whole):
+            break
+        ends.append(m.end())
+    return ends
+
+
+def range_head(path, lo, hi):
+    """The head of the range [lo, hi) of ``path``: its bytes up to and including its third line
+    terminator, or all of them when it has fewer.  None when that is longer than HEAD_CAP."""
+    with open(path, "rb") as fh:
+        fh.seek(lo)
+        data = fh.read(min(hi - lo, HEAD_CAP + 1))
+    whole = len(data) == hi - lo
+    ends = line_ends(data, 3, whole)
+    if len(ends) == 3:
+        data = data[:ends[2]]
+    elif not whole:
+        return None
+    return data if len(data) <= HEAD_CAP else None
+
+
+def plan_trimmed_shards(lines, heads, limit):
+    """Lines up the byte ranges of a sharded file on record boundaries, from every range's line starts
+    ``lines[k]`` and head ``heads[k]`` (:func:`range_head`).  Records are groups of four lines counted
+    from the start of the file, so range k has base_k = sum(lines[:k]) lines before it, and its first
+    skip_k = (4 - base_k % 4) % 4 lines finish a record that began before it.  Range k owns its text
+    from its first whole record on, plus the first skip_{k+1} lines of range k + 1 (from that range's
+    head): whole records, except at the end of the file.
+
+    Returns, per range, (start, tail, first, max_records): the owned text is range[start:] + tail, its
+    first record is record ``first`` of the file, and at most max_records = max(0, limit - first) of its
+    records are taken (``limit``: the file's record limit, limit_from_maxreads).  None when some range
+    holds fewer than skip_k + 1 line starts, or its head fewer than skip_k line ends."""
+    skips, firsts, base = [], [], 0
+    for k, n in enumerate(lines):
+        skip = (4 - base % 4) % 4
+        if n < skip + 1 or len(line_ends(heads[k], skip)) < skip:
+            return None
+        skips.append(skip)
+        firsts.append((base + skip) // 4)
+        base += n
+    out = []
+    for k in range(len(lines)):
+        start = line_ends(heads[k], skips[k])[-1] if skips[k] else 0
+        tail = heads[k + 1][:line_ends(heads[k + 1], skips[k + 1])[-1]] if k + 1 < len(lines) and skips[k + 1] else b""
+        out.append((start, tail, firsts[k], max(0, limit - firsts[k])))
+    return out
+
+
+def count_trimmed_range(eng, path, rank, world, gather, barcodes, rows, plan, cutsite, adapter, maxreads):
+    """One rank's share of a plain file that count_files(..., adapter=...) shards across ``world`` GPUs.
+    The file is cut at line ends (:func:`range_bounds`), but the splitter's front needs text that
+    begins at a RECORD start, and ``maxreads`` counts records from the start of the file.  So:
+
+    1. every rank loads its range into device memory, counts its lines there
+       (``tdg_count_lines_device``) and reads its head (:func:`range_head`);
+    2. one ``gather`` of [ok, lines, head] tells every rank where every range's first whole record
+       starts (:func:`plan_trimmed_shards`); rank k appends the lines of range k + 1 that complete its
+       last record, from that range's head;
+    3. if any rank cannot take part (no line end near a cut, an allocation failure, a head longer
+       than HEAD_CAP, a range with too few lines), rank 0 counts the whole file with
+       :func:`splitter.count_trimmed_file`, exactly as when files are dealt whole;
+    4. otherwise every rank counts its owned text on the device (:func:`splitter.count_trimmed_resident`);
+    5. a second ``gather`` sums the four totals, and rank 0 prints the file's line.  A rank that failed
+       in step 4 raises its own exception after that gather, the others a RuntimeError naming it.
+
+    Returns the file's [reads, with barcode and cut site, clipped on the 3' end, with tag], or None on
+    the ranks other than 0 when rank 0 counted the file whole."""
+    from . import splitter
+    if gather is None:
+        raise ValueError("sharding a file across ranks needs a gather callable (see dist_gather)")
+    dev, lines, head, n = None, 0, b"", 0
+    try:
+        bounds = range_bounds(path, world)
+        if bounds is not None:
+            lo, hi = bounds[rank], bounds[rank + 1]
+            n = hi - lo
+            head = range_head(path, lo, hi)
+            if head is not None:
+                dev = _load_range(eng, path, lo, n, extra=HEAD_CAP)
+                lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
+    except (OSError, _native.TdgError):
+        if dev is not None:
+            eng.device_free(dev)
+            dev = None                          # this rank votes for counting the file whole
+    every = gather([1, lines, len(head)] + list(head) if dev is not None else [0, 0, 0])
+    shards = None
+    if all(x[0] for x in every):
+        shards = plan_trimmed_shards([x[1] for x in every], [bytes(x[3:3 + x[2]]) for x in every],
+                                     _native.limit_from_maxreads(maxreads))
+    if shards is None:
+        if dev is not None:
+            eng.device_free(dev)
+        if rank != 0:
+            return None
+        tot = splitter.count_trimmed_file(eng, path, barcodes, rows, plan, cutsite=cutsite, adapter=adapter, maxreads=maxreads)
+    else:
+        start, tail, _first, max_records = shards[rank]
+        tot, err = [0, 0, 0, 0], None
+        try:
+            if tail:
+                eng.memcpy_h2d(dev + n, np.frombuffer(tail, dtype=np.uint8).ctypes.data, len(tail))
+            tot = splitter.count_trimmed_resident(eng, dev + start, n - start + len(tail), barcodes, rows, plan, cutsite,
+                                                  adapter, max_records)
+        except Exception as e:                  # every rank still takes part in the second gather
+            err = e
+        finally:
+            eng.device_free(dev)
+        every = gather([0 if err is None else 1] + [int(t) for t in tot])
+        if err is not None:
+            raise err
+        failed = [k for k, x in enumerate(every) if x[0]]
+        if failed:
+            raise RuntimeError("%s: rank %d failed while counting its byte range" % (path, failed[0]))
+        tot = [sum(x[1 + k] for x in every) for k in range(4)]
+    if rank == 0:
+        print("{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}".format(path, *tot))
     return tot
 
 

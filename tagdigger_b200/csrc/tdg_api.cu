@@ -769,14 +769,15 @@ int batch_run(tdg_ctx *ctx, const char *what, const char *seqs, const uint64_t *
     return TDG_OK;
 }
 
-// The front tdg_split_block and tdg_split_count_block share: the block goes to the device, its line
-// ends are found and split_records takes the decisions for its first `nrec` whole records (nrec = 0:
-// there is none, and nothing ran past the line count).  prepare(nrec) grows the caller's own buffers
-// and sets w.complex_flag before split_records is launched.  last_end (the terminator of the last
-// record's last line) is valid once the caller has synchronised the stream.
+// The front tdg_split_block, tdg_split_count_block and tdg_split_count_device share: the block goes to
+// sp_in (`kind` says whether `bytes` is host or device memory; either way sp_in carries the zero padding
+// the kernels read past n), its line ends are found and split_records takes the decisions for its first
+// `nrec` whole records (nrec = 0: there is none, and nothing ran past the line count).  prepare(nrec)
+// grows the caller's own buffers and sets w.complex_flag before split_records is launched.  last_end
+// (the terminator of the last record's last line) is valid once the caller has synchronised the stream.
 template <class Prepare>
-int split_front(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, uint64_t max_records, tdg::SplitWork &w,
-                uint64_t &nrec, uint32_t &last_end, Prepare prepare)
+int split_front(tdg_ctx *ctx, const uint8_t *bytes, cudaMemcpyKind kind, size_t n, int final_block, uint64_t max_records,
+                tdg::SplitWork &w, uint64_t &nrec, uint32_t &last_end, Prepare prepare)
 {
     cudaStream_t st = ctx->stream;
     const uint32_t nbar = ctx->sp_nbar;
@@ -788,7 +789,7 @@ int split_front(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, u
     const uint32_t n_tiles = (uint32_t)((n + tdg::SPLIT_TILE_BYTES - 1) / tdg::SPLIT_TILE_BYTES);
     if ((rc = grow(ctx, ctx->sp_in, round_up(n, 16) + 16, false))) return rc;
     if ((rc = grow(ctx, ctx->sp_tiles, (size_t)(n_tiles + 2) * sizeof(uint32_t), false))) return rc;
-    CK(cudaMemcpyAsync(ctx->sp_in.p, bytes, n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(ctx->sp_in.p, bytes, n, kind, st));
     CK(cudaMemsetAsync((uint8_t *)ctx->sp_in.p + n, 0, round_up(n, 16) + 16 - n, st));
     memset(&w, 0, sizeof w);
     w.b.bytes = (const uint8_t *)ctx->sp_in.p;
@@ -802,10 +803,12 @@ int split_front(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, u
     tdg::tile_scan<<<1, 1024, 0, st>>>(w.b.tile_count, n_tiles);
     ctx->launches += 2;
     uint32_t lines = 0;
+    uint8_t last = 0;
     CK(cudaMemcpyAsync(&lines, w.b.tile_count + n_tiles, sizeof lines, cudaMemcpyDeviceToHost, st));
+    if (kind == cudaMemcpyDeviceToDevice) CK(cudaMemcpyAsync(&last, (const uint8_t *)ctx->sp_in.p + n - 1, 1, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
+    if (kind == cudaMemcpyHostToDevice) last = bytes[n - 1];
     // the text after the last line end is a line of its own when the file ends here
-    const uint8_t last = bytes[n - 1];
     const bool open_tail = final_block && last != '\n' && last != '\r';
     const uint64_t total_lines = (uint64_t)lines + (open_tail ? 1 : 0);
     uint64_t records = total_lines / 4;
@@ -1928,7 +1931,7 @@ int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_bloc
     uint64_t nrec = 0;
     uint32_t last_end = 0;
     unsigned long long *bar_total = nullptr;
-    rc = split_front(ctx, bytes, n, final_block, max_records, w, nrec, last_end, [&](uint64_t records) {
+    rc = split_front(ctx, bytes, cudaMemcpyHostToDevice, n, final_block, max_records, w, nrec, last_end, [&](uint64_t records) {
         const uint32_t n_rtiles = (uint32_t)((records + tdg::SPLIT_REC_TILE - 1) / tdg::SPLIT_REC_TILE);
         int rc;
         if ((rc = grow(ctx, ctx->sp_sums, (size_t)n_rtiles * nbar * sizeof(uint32_t), false))) return rc;
@@ -2018,14 +2021,17 @@ int tdg_split_count_begin(tdg_ctx *ctx, const char *bases, const uint32_t *off, 
     return TDG_OK;
 }
 
-int tdg_split_count_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, uint64_t max_records,
-                          uint64_t *n_records, uint64_t *consumed, int *needs_host, uint64_t totals[4])
+// tdg_split_count_block (host bytes) and tdg_split_count_device (device bytes): one block through
+// split_front and split_count.
+static int split_count_run(tdg_ctx *ctx, const char *what, const uint8_t *bytes, cudaMemcpyKind kind, size_t n,
+                           int final_block, uint64_t max_records, uint64_t *n_records, uint64_t *consumed, int *needs_host,
+                           uint64_t totals[4])
 {
     int rc = need_device(ctx);
     if (rc) return rc;
     if ((rc = split_count_ready(ctx))) return rc;
     if (!n_records || !consumed || !needs_host || !totals || (!bytes && n)) return fail(ctx, TDG_ERR_ARG, "null argument");
-    if (n > ((size_t)1 << 30)) return fail(ctx, TDG_ERR_ARG, "tdg_split_count_block: at most 1 GiB per block");
+    if (n > ((size_t)1 << 30)) return fail(ctx, TDG_ERR_ARG, std::string(what) + ": at most 1 GiB per block");
     *n_records = 0;
     *consumed = 0;
     *needs_host = 0;
@@ -2039,7 +2045,7 @@ int tdg_split_count_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int fina
     uint32_t last_end = 0;
     bool timed;                                      // tdg_timing_*: the block's upload and kernels as one
     if ((rc = timed_start(ctx, timed))) return rc;
-    rc = split_front(ctx, bytes, n, final_block, max_records, w, nrec, last_end, [&](uint64_t) {
+    rc = split_front(ctx, bytes, kind, n, final_block, max_records, w, nrec, last_end, [&](uint64_t) {
         w.complex_flag = (uint32_t *)(d_tot + 4);
         CK(cudaMemsetAsync(d_tot, 0, 4 * sizeof(unsigned long long), st));
         return TDG_OK;
@@ -2062,6 +2068,20 @@ int tdg_split_count_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int fina
     }
     for (int k = 0; k < 4; k++) totals[k] = h[k];
     return TDG_OK;
+}
+
+int tdg_split_count_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, uint64_t max_records,
+                          uint64_t *n_records, uint64_t *consumed, int *needs_host, uint64_t totals[4])
+{
+    return split_count_run(ctx, "tdg_split_count_block", bytes, cudaMemcpyHostToDevice, n, final_block, max_records, n_records,
+                           consumed, needs_host, totals);
+}
+
+int tdg_split_count_device(tdg_ctx *ctx, const void *dev_bytes, size_t n, int final_block, uint64_t max_records,
+                           uint64_t *n_records, uint64_t *consumed, int *needs_host, uint64_t totals[4])
+{
+    return split_count_run(ctx, "tdg_split_count_device", (const uint8_t *)dev_bytes, cudaMemcpyDeviceToDevice, n, final_block,
+                           max_records, n_records, consumed, needs_host, totals);
 }
 
 int tdg_split_count_batch(tdg_ctx *ctx, const char *seqs, const uint64_t *off, const int32_t *bar, uint32_t n, int32_t *col_out)

@@ -20,6 +20,8 @@ one byte for byte.
 ``count_trimmed_file`` runs the same block loop and the same device front, but counts instead of
 writing: every barcode's trimmed reads go through find_tags_fastq's matcher with a blank barcode
 (``tdg_split_count_block``), as counting the output files would -- without the files.
+``count_trimmed_resident`` counts the same way on text that is already in device memory
+(``tdg_split_count_device``): one rank's share of a file sharded across GPUs.
 """
 
 import csv
@@ -266,27 +268,22 @@ def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=h
     return None
 
 
-def count_trimmed_file(eng, inputFile, barcodes, rows, plan, cutsite="TGCAG", adapter=hostio.adapters["PstI-MspI-Hall"],
-                       maxreads=500000000):
-    """barcodeSplitter(inputFile, barcodes, files, cutsite, adapter, maxreads), then
-    find_tags_fastq(files[b], [''], tags, stage-2 cut site) added into matrix row ``rows[b]`` for every
-    barcode b -- without the files: the splitter's device front decides every record, and the
-    counter's matcher runs on the slice the file would hold (``tdg_split_count_block``).  ``plan`` is
-    ``matchset.plan([''], tags, stage-2 cut site)``; the engine must hold its tags (``set_tags``) and
-    the matrix.  Blocks with non-ASCII sequence or quality lines are cut by Python, as
-    barcodeSplitter writes them, and counted on the GPU (``tdg_split_count_batch``).
-
-    Returns [reads, reads with barcode and cut site, reads clipped on the 3' end, reads with tag]."""
+def _trimmed_counter(eng, barcodes, rows, plan, cutsite, adapter):
+    """The set-up of a one-pass count (split tables, stage-2 table) and the two block handlers that
+    count_trimmed_file and count_trimmed_resident share.  Returns (tot, device_result, host_block):
+    ``tot`` = [reads, with barcode and cut site, clipped on the 3' end, with tag] so far;
+    ``device_result(r)`` adds the totals of a split_count_block / split_count_device result r and
+    returns (records, consumed, needs_host); ``host_block(text)`` cuts and counts the records of a
+    block the device left to the host."""
     _check_args(cutsite, barcodes, adapter)
     barlen = [len(bc) for bc in barcodes]
     cutlen = len(cutsite)
     _load_split(eng, _split_patterns(barcodes, cutsite), barcodes, cutsite, adapter)
     eng.split_count_begin(plan.bar.patterns, plan.bar_tag_off, rows, any_base=plan.bar.any_base)
-    feed = _open_input(inputFile)
     tot = [0, 0, 0, 0]
 
-    def device_block(buf, fill, eof, left):
-        nrec, used, needs_host, t = eng.split_count_block(buf, fill, eof, left)
+    def device_result(r):
+        nrec, used, needs_host, t = r
         if nrec and not needs_host:
             for k in range(4):
                 tot[k] += t[k]
@@ -306,12 +303,62 @@ def count_trimmed_file(eng, inputFile, barcodes, rows, plan, cutsite="TGCAG", ad
             if seqs:
                 tot[3] += int(np.count_nonzero(eng.split_count_batch(seqs, bars) >= 0))
 
+    return tot, device_result, host_block
+
+
+def count_trimmed_file(eng, inputFile, barcodes, rows, plan, cutsite="TGCAG", adapter=hostio.adapters["PstI-MspI-Hall"],
+                       maxreads=500000000):
+    """barcodeSplitter(inputFile, barcodes, files, cutsite, adapter, maxreads), then
+    find_tags_fastq(files[b], [''], tags, stage-2 cut site) added into matrix row ``rows[b]`` for every
+    barcode b -- without the files: the splitter's device front decides every record, and the
+    counter's matcher runs on the slice the file would hold (``tdg_split_count_block``).  ``plan`` is
+    ``matchset.plan([''], tags, stage-2 cut site)``; the engine must hold its tags (``set_tags``) and
+    the matrix.  Blocks with non-ASCII sequence or quality lines are cut by Python, as
+    barcodeSplitter writes them, and counted on the GPU (``tdg_split_count_batch``).
+
+    Returns [reads, reads with barcode and cut site, reads clipped on the 3' end, reads with tag]."""
+    tot, device_result, host_block = _trimmed_counter(eng, barcodes, rows, plan, cutsite, adapter)
+    feed = _open_input(inputFile)
+
+    def device_block(buf, fill, eof, left):
+        return device_result(eng.split_count_block(buf, fill, eof, left))
+
     try:
         _block_loop(eng, feed, maxreads, device_block, host_block)
     except _native.TdgError as e:
         raise _feed_error(e)
     finally:
         feed.close()
+    return tot
+
+
+RESIDENT_CALL_BYTES = 1 << 30     # the split kernels' 32-bit offsets: at most 1 GiB per tdg_split_count_device call
+
+
+def count_trimmed_resident(eng, dev, n, barcodes, rows, plan, cutsite, adapter, max_records):
+    """count_trimmed_file on text already in device memory: ``n`` bytes at ``dev`` that begin at a record
+    start and end at a record boundary or at the end of the file, of which at most ``max_records``
+    records are taken.  The text is walked in calls of at most RESIDENT_CALL_BYTES
+    (``tdg_split_count_device``), each starting where the previous one stopped; the last call is final.
+    A call that needs the host copies its bytes back and goes through count_trimmed_file's host path.
+    Returns the same four totals."""
+    tot, device_result, host_block = _trimmed_counter(eng, barcodes, rows, plan, cutsite, adapter)
+    pos = done = 0
+    while pos < n and done < max_records:
+        size = min(RESIDENT_CALL_BYTES, n - pos)
+        final = pos + size == n
+        nrec, used, needs_host = device_result(eng.split_count_device(dev + pos, size, final, max_records - done))
+        if nrec == 0:
+            if final:
+                break                                        # what is left is not a whole record
+            raise _native.TdgError(_native.TDG_ERR_ARG, "count_trimmed_resident: a record longer than %d bytes"
+                                   % RESIDENT_CALL_BYTES)
+        if needs_host:
+            raw = np.empty(used, dtype=np.uint8)
+            eng.memcpy_d2h(raw.ctypes.data, dev + pos, used)
+            host_block(raw.tobytes().decode("utf-8"))
+        done += nrec
+        pos += used
     return tot
 
 
