@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """One config-5 library file counted in one pass (count_files(..., adapter=...)) at world 1 and sharded
-across W ranks (count_trimmed_range): every cell of the W-rank matrix must equal the world-1 matrix.
+across W ranks (counting._count_sharded): every cell of the W-rank matrix must equal the world-1 matrix.
 
 The input is the config-5 shape of scripts/config5_flow.py (150 bp reads in /dev/shm, 96-plex,
 PstI-MspI-Hall, 2,000 of 4,000 tags kept).  W is the number of GPUs present, at least 2: with one GPU

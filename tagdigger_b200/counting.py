@@ -58,6 +58,23 @@ def _is_gz(name):
     return name[-2:].lower() == "gz"            # tagdigger_fun.py:240
 
 
+def _reference_error(e, opening=False):
+    """The exception the reference's open() / gzip.open(...).read() raises (tagdigger_fun.py:240-243) for
+    the defect a library call reported as TdgError ``e``: gzip's for a gzip defect, OSError for an I/O
+    error, UnicodeDecodeError for invalid UTF-8 (open(f, 'r') / gzip.open(f, 'rt') decode the file; of
+    the library's calls only tdg_count_file checks it).  Other codes (CUDA, allocation, state) have no
+    counterpart there and stay ``e`` -- except when ``opening`` a file: the feed's open fails as
+    open() does, with an OSError."""
+    if e.code == _native.TDG_ERR_GZIP:
+        return _gzip_exception(e.message)
+    if e.code == _native.TDG_ERR_IO or opening:
+        return OSError(e.message)
+    if e.code == _native.TDG_ERR_UTF8:
+        pos = int(e.message.split()[1].rstrip(":")) if e.message.startswith("position ") else 0
+        return UnicodeDecodeError("utf-8", b"\xff", 0, 1, "invalid UTF-8 at byte %d (%s)" % (pos, e.message))
+    return e
+
+
 def _run_file(eng, fqfile, limit, next_file=None):
     """Stream one file; map library errors to the exceptions the reference's
     open()/gzip.open() would raise.  ``next_file``: the file that will be counted next (the
@@ -68,15 +85,7 @@ def _run_file(eng, fqfile, limit, next_file=None):
         return eng.count_file(fqfile, _is_gz(fqfile), limit, next_path=next_file,
                               next_gz=_is_gz(next_file) if next_file else False)
     except _native.TdgError as e:
-        if e.code == _native.TDG_ERR_GZIP:
-            raise _gzip_exception(e.message)
-        if e.code == _native.TDG_ERR_IO:
-            raise OSError(e.message)
-        if e.code == _native.TDG_ERR_UTF8:
-            # open(f, 'r') / gzip.open(f, 'rt') decode the file as UTF-8 (tagdigger_fun.py:240-243)
-            pos = int(e.message.split()[1].rstrip(":")) if e.message.startswith("position ") else 0
-            raise UnicodeDecodeError("utf-8", b"\xff", 0, 1, "invalid UTF-8 at byte %d (%s)" % (pos, e.message))
-        raise
+        raise _reference_error(e)
 
 
 def find_tags_fastq(fqfile, barcodes, tags, cutsite="TGCAG", maxreads=5e9, tassel_tagcount=False,
@@ -208,14 +217,17 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
     size (largest first, to the least loaded rank) and ``reduce(ptr, rows, cols,
     engine)`` must sum the per-rank matrices in place (one NCCL all-reduce, see
     :func:`nccl_reduce`); integer sums make the result independent of ``world``.  When there are
-    fewer files than ranks, plain files are sharded by byte range instead (:func:`count_file_range`),
-    which needs ``gather(list_of_ints) -> list of every rank's list`` (:func:`dist_gather`).
+    fewer files than ranks, plain files are sharded by byte range instead and counted first
+    (:func:`_count_sharded`, which needs ``gather(list_of_ints) -> list of every rank's list``,
+    :func:`dist_gather`).  Results, rank 0's output and exceptions stay those of a one-rank run.
 
     Returns ``[sample names, count rows]`` -- rows as lists of int like combineReadCounts, or,
     with ``as_array=True``, as one int32 ndarray (hostio.writeCounts / writeDiploidGeno format
     that with native threads; a 384 x 500,000 matrix is 768 MB as an array and several GB as
-    Python integers).  ``totals`` (optional dict) receives ``{file: [reads, with barcode and
-    cut site, with tag]}`` for this rank's files.
+    Python integers).  Each file prints one line with its totals, on the rank that counted it (rank 0
+    for a sharded file), and ``totals`` (optional dict) receives ``{file: [reads, with barcode and
+    cut site, with tag]}`` for this rank's files; a sharded file's totals are summed over the ranks
+    and go to every rank (to rank 0 alone when it counted the file whole).
 
     With ``adapter`` (the name of an adapter set, a key of ``hostio.adapters``) every file is first
     split and trimmed as ``barcodeSplitter(f, barcodes, files, cutsite=split_cutsite, adapter=...,
@@ -223,47 +235,31 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
     ``find_tags_fastq(file, [''], tags, cutsite)`` into its sample's row -- in one pass per file on the
     GPU, without writing the split files (:func:`splitter.count_trimmed_file`).  ``split_cutsite``
     defaults to the cut site of the adapter set's enzyme, as barcode_splitter_script derives it.  Files
-    are dealt to the ranks, or sharded by byte range as above (:func:`count_trimmed_range`, which lines
-    the ranges up on record boundaries); sharded files are counted first.  ``totals`` then receives
-    ``[reads, with barcode and cut site, clipped on the 3' end, with tag]``, for a sharded file on every
-    rank and summed over the ranks."""
+    are dealt or sharded as above.  ``totals`` then receives ``[reads, with barcode and cut site,
+    clipped on the 3' end, with tag]``."""
     files = sorted(bckeys.keys())
     samples, rows = global_rows(bckeys)
-    if adapter is not None:
-        eng = _count_trimmed_files(bckeys, files, rows, len(samples), tags, cutsite, maxreads, device, rank, world,
-                                   totals, adapter, split_cutsite, split_maxreads, gather)
-        return _result(eng, samples, len(tags), world, reduce, as_array)
-    limit = _native.limit_from_maxreads(maxreads)
-    plans = {}
-    tagplan = None
-    for f in files:                               # set-up errors surface before any counting, file by file
-        if tagplan is None:
-            plans[f] = matchset.plan(bckeys[f][0], tags, cutsite)
-            tagplan = matchset.plan_tags(tags, cutsite)       # shared by the other files of the key
-        else:
-            plans[f] = matchset.plan(bckeys[f][0], tags, cutsite, tagplan=tagplan)
-        if plans[f].barnum == 0 or plans[f].ntags == 0:
-            raise IndexError("list index out of range")
-    ntags = len(tags)
+    if adapter is None:
+        mode = _PlainCount(bckeys, files, rows, tags, cutsite, maxreads)
+    else:
+        mode = _TrimmedCount(bckeys, files, rows, tags, cutsite, maxreads, adapter, split_cutsite, split_maxreads)
     eng = get_engine(device)
-    first = plans[files[0]]
-    eng.set_tags(first.tags.patterns, first.tags.index, any_base=first.tags.any_base)
-    eng.set_matrix(len(samples), ntags)
+    eng.set_tags(mode.tags.patterns, mode.tags.index, any_base=mode.tags.any_base)
+    eng.set_matrix(len(samples), len(tags))
     split = shard_files(files, world)
-    for f in split:
-        load_plan(eng, plans[f], row_of=rows[f], set_tags=False)
-        tot = count_file_range(eng, f, rank, world, limit, gather)
+    todo = split + assign_files([f for f in files if f not in split], rank, world)
+    for i, f in enumerate(todo):
+        if f in split:
+            tot = _count_sharded(eng, mode, f, rank, world, gather)
+            if tot is None:
+                continue                          # rank 0 counted the file whole
+        else:
+            tot = mode.whole(eng, f, next_file=todo[i + 1] if i + 1 < len(todo) else None)
+        if rank == 0 or f not in split:
+            print(mode.line.format(f, *tot))
         if totals is not None:
-            totals[f] = tot[:3]
-    mine = assign_files([f for f in files if f not in split], rank, world)
-    for i, f in enumerate(mine):
-        p = plans[f]
-        load_plan(eng, p, row_of=rows[f], set_tags=False)
-        tot = _run_file(eng, f, limit, next_file=mine[i + 1] if i + 1 < len(mine) else None)
-        print("{0}: Reads: {1} With barcode and cut site: {2} With tag: {3}".format(f, tot[0], tot[1], tot[2]))
-        if totals is not None:
-            totals[f] = tot[:3]
-    return _result(eng, samples, ntags, world, reduce, as_array)
+            totals[f] = tot
+    return _result(eng, samples, len(tags), world, reduce, as_array)
 
 
 def _result(eng, samples, ntags, world, reduce, as_array):
@@ -276,42 +272,100 @@ def _result(eng, samples, ntags, world, reduce, as_array):
     return [samples, matrix if as_array else matrix.tolist()]
 
 
-def _count_trimmed_files(bckeys, files, rows, nrows, tags, cutsite, maxreads, device, rank, world, totals, adapter,
-                         split_cutsite, split_maxreads, gather):
-    """count_files with ``adapter``: this rank's files through splitter.count_trimmed_file.  Returns the engine."""
-    from . import hostio, splitter
-    if not isinstance(adapter, str) or adapter not in hostio.adapters:
-        raise ValueError("unknown adapter set %r (one of %s)" % (adapter, ", ".join(sorted(hostio.adapters))))
-    if maxreads != 5e9:
-        raise ValueError("maxreads does not apply with adapter: a split file holds at most split_maxreads reads")
-    if split_maxreads is None or not float(split_maxreads) <= 5e9:
-        raise ValueError("split_maxreads must be at most 5e9, the number of reads the counter takes from a split file")
-    adapter_seqs = hostio.adapters[adapter]
-    if split_cutsite is None:
-        split_cutsite = hostio.enzymes[adapter[:adapter.find("-")]]
-    # set-up errors surface before any counting, in the order of the two-stage run: every file's split, then the count
-    for f in files:
-        splitter._check_args(split_cutsite, bckeys[f][0], adapter_seqs)
-        splitter._split_patterns(bckeys[f][0], split_cutsite)
-    plan = matchset.plan([""], tags, cutsite)
-    if plan.ntags == 0:
-        raise IndexError("list index out of range")
-    eng = get_engine(device)
-    eng.set_tags(plan.tags.patterns, plan.tags.index, any_base=plan.tags.any_base)
-    eng.set_matrix(nrows, plan.ntags)
-    split = shard_files(files, world)
-    for f in split:
-        tot = count_trimmed_range(eng, f, rank, world, gather, bckeys[f][0], rows[f], plan, split_cutsite, adapter_seqs,
-                                  split_maxreads)
-        if tot is not None and totals is not None:
-            totals[f] = tot
-    for f in assign_files([f for f in files if f not in split], rank, world):
-        tot = splitter.count_trimmed_file(eng, f, bckeys[f][0], rows[f], plan, cutsite=split_cutsite, adapter=adapter_seqs,
-                                          maxreads=split_maxreads)
-        print("{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}".format(f, *tot))
-        if totals is not None:
-            totals[f] = tot
-    return eng
+class _PlainCount:
+    """count_files' plain mode: every file counted as find_tags_fastq counts it.  Construction runs the
+    set-up checks, file by file, before anything is counted.  What the mode supplies to count_files and
+    :func:`_count_sharded`: ``tags`` (the tag plan), ``line`` (the format of a file's output line),
+    ``whole`` (count a whole file), ``payload`` / ``extra`` / ``place`` (what a rank adds to the
+    first gather, the room it needs behind its range, and where its range lies in the file) and ``own``
+    (count its range)."""
+    line = "{0}: Reads: {1} With barcode and cut site: {2} With tag: {3}"
+    extra = 0
+
+    def __init__(self, bckeys, files, rows, tags, cutsite, maxreads):
+        self.limit = _native.limit_from_maxreads(maxreads)
+        self.rows = rows
+        self.plans = {}
+        tagplan = None
+        for f in files:
+            if tagplan is None:
+                self.plans[f] = matchset.plan(bckeys[f][0], tags, cutsite)
+                tagplan = matchset.plan_tags(tags, cutsite)       # shared by the other files of the key
+            else:
+                self.plans[f] = matchset.plan(bckeys[f][0], tags, cutsite, tagplan=tagplan)
+            if self.plans[f].barnum == 0 or self.plans[f].ntags == 0:
+                raise IndexError("list index out of range")
+        self.tags = self.plans[files[0]].tags
+
+    def whole(self, eng, f, next_file=None):
+        """[reads, with barcode and cut site, with tag] of file ``f``."""
+        load_plan(eng, self.plans[f], row_of=self.rows[f], set_tags=False)
+        return _run_file(eng, f, self.limit, next_file)[:3]
+
+    def payload(self, f, lo, hi):
+        return []
+
+    def place(self, lines, payloads, rank):
+        """The range's first line index in the file: read indices, and so ``maxreads``, stay global."""
+        return sum(lines[:rank])
+
+    def own(self, eng, f, rank, dev, n, base):
+        load_plan(eng, self.plans[f], row_of=self.rows[f], set_tags=False)   # a fresh line state, too
+        eng.count_device(dev, n, base, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF, self.limit)
+        return eng.file_totals()[:3]
+
+
+class _TrimmedCount:
+    """count_files' one-pass split-trim-count mode (``adapter``), with the members of :class:`_PlainCount`.
+    Set-up errors surface in the order of the two-stage run: every file's split, then the count."""
+    line = "{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}"
+
+    def __init__(self, bckeys, files, rows, tags, cutsite, maxreads, adapter, split_cutsite, split_maxreads):
+        from . import hostio, splitter
+        if not isinstance(adapter, str) or adapter not in hostio.adapters:
+            raise ValueError("unknown adapter set %r (one of %s)" % (adapter, ", ".join(sorted(hostio.adapters))))
+        if maxreads != 5e9:
+            raise ValueError("maxreads does not apply with adapter: a split file holds at most split_maxreads reads")
+        if split_maxreads is None or not float(split_maxreads) <= 5e9:
+            raise ValueError("split_maxreads must be at most 5e9, the number of reads the counter takes from a split file")
+        self.adapter = hostio.adapters[adapter]
+        self.cutsite = hostio.enzymes[adapter[:adapter.find("-")]] if split_cutsite is None else split_cutsite
+        for f in files:
+            splitter._check_args(self.cutsite, bckeys[f][0], self.adapter)
+            splitter._split_patterns(bckeys[f][0], self.cutsite)
+        self.plan = matchset.plan([""], tags, cutsite)
+        if self.plan.ntags == 0:
+            raise IndexError("list index out of range")
+        self.tags = self.plan.tags
+        self.bckeys, self.rows, self.maxreads = bckeys, rows, split_maxreads
+
+    @property
+    def extra(self):
+        return HEAD_CAP           # room for the lines of the next range that complete the last record
+
+    def whole(self, eng, f, next_file=None):
+        """[reads, with barcode and cut site, clipped on the 3' end, with tag] of file ``f``."""
+        from . import splitter
+        return splitter.count_trimmed_file(eng, f, self.bckeys[f][0], self.rows[f], self.plan, cutsite=self.cutsite,
+                                           adapter=self.adapter, maxreads=self.maxreads)
+
+    def payload(self, f, lo, hi):
+        """The range's head (:func:`range_head`), or None when it is too long to send."""
+        head = range_head(f, lo, hi)
+        return None if head is None else list(head)
+
+    def place(self, lines, payloads, rank):
+        """The range's owned text and record budget (:func:`plan_trimmed_shards`); None to count the file whole."""
+        shards = plan_trimmed_shards(lines, [bytes(p) for p in payloads], _native.limit_from_maxreads(self.maxreads))
+        return None if shards is None else shards[rank]
+
+    def own(self, eng, f, rank, dev, n, shard):
+        from . import splitter
+        start, tail, _first, max_records = shard
+        if tail:
+            eng.memcpy_h2d(dev + n, np.frombuffer(tail, dtype=np.uint8).ctypes.data, len(tail))
+        return splitter.count_trimmed_resident(eng, dev + start, n - start + len(tail), self.bckeys[f][0], self.rows[f],
+                                               self.plan, self.cutsite, self.adapter, max_records)
 
 
 SHARD_MIN_BYTES = 1 << 20     # files smaller than this per rank are not worth cutting up
@@ -361,42 +415,6 @@ def range_bounds(path, world):
             bounds.append(min(found, size))
     bounds.append(size)
     return bounds
-
-
-def count_file_range(eng, path, rank, world, limit, gather):
-    """One rank's share of a plain FASTQ file that is sharded across ``world`` GPUs.
-
-    The file is cut at line ends into one byte range per rank.  Which lines are sequence lines
-    depends on the line index from the start of the FILE (tagdigger_fun.py:250-254), so every
-    rank first counts the lines of its range on its GPU (``tdg_count_lines_device``: the scan
-    half of the kernel), the counts are exchanged (``gather``), and the range is then counted
-    with its true first line index (``tdg_count_device``).  ``maxreads`` works unchanged: read
-    indices are global.  Returns this rank's [reads, with barcode and cut site, with tag]."""
-    if gather is None:
-        raise ValueError("sharding a file across ranks needs a gather callable (see dist_gather)")
-    bounds = range_bounds(path, world)
-    ok = gather([0 if bounds is None else 1])
-    if not all(x[0] for x in ok):                       # every rank must take the same decision
-        bounds = None
-    if bounds is None:
-        tot = [0, 0, 0, 0]
-        if rank == 0:
-            tot = _run_file(eng, path, limit)
-        return tot
-    lo, hi = bounds[rank], bounds[rank + 1]
-    n = hi - lo
-    dev = _load_range(eng, path, lo, n)
-    try:
-        lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
-        every = gather([lines])
-        base = sum(x[0] for x in every[:rank])
-        eng.reset_file()
-        eng.count_device(dev, n, base, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF, limit)
-        tot = eng.file_totals()
-    finally:
-        eng.device_free(dev)
-    print("{0} [bytes {1}-{2}]: Reads: {3} With barcode and cut site: {4} With tag: {5}".format(path, lo, hi, *tot[:3]))
-    return tot
 
 
 def _load_range(eng, path, lo, n, extra=0):
@@ -486,75 +504,61 @@ def plan_trimmed_shards(lines, heads, limit):
     return out
 
 
-def count_trimmed_range(eng, path, rank, world, gather, barcodes, rows, plan, cutsite, adapter, maxreads):
-    """One rank's share of a plain file that count_files(..., adapter=...) shards across ``world`` GPUs.
-    The file is cut at line ends (:func:`range_bounds`), but the splitter's front needs text that
-    begins at a RECORD start, and ``maxreads`` counts records from the start of the file.  So:
+def _count_sharded(eng, mode, path, rank, world, gather):
+    """One file that count_files cuts into one byte range per rank (:func:`shard_files`), in either counting
+    mode (``mode``: :class:`_PlainCount` or :class:`_TrimmedCount`).  Lines, reads and records are numbered
+    from the start of the FILE (tagdigger_fun.py:250-254), so a range cannot be counted on its own:
 
-    1. every rank loads its range into device memory, counts its lines there
-       (``tdg_count_lines_device``) and reads its head (:func:`range_head`);
-    2. one ``gather`` of [ok, lines, head] tells every rank where every range's first whole record
-       starts (:func:`plan_trimmed_shards`); rank k appends the lines of range k + 1 that complete its
-       last record, from that range's head;
-    3. if any rank cannot take part (no line end near a cut, an allocation failure, a head longer
-       than HEAD_CAP, a range with too few lines), rank 0 counts the whole file with
-       :func:`splitter.count_trimmed_file`, exactly as when files are dealt whole;
-    4. otherwise every rank counts its owned text on the device (:func:`splitter.count_trimmed_resident`);
-    5. a second ``gather`` sums the four totals, and rank 0 prints the file's line.  A rank that failed
-       in step 4 raises its own exception after that gather, the others a RuntimeError naming it.
+    1. every rank loads its range of :func:`range_bounds` into device memory (:func:`_load_range`), with
+       ``mode.extra`` bytes of room behind it, and counts its line starts there (``tdg_count_lines_device``);
+    2. one ``gather`` of [ok, line starts, ``mode.payload``] tells every rank where its range lies in the
+       file (``mode.place``);
+    3. if some rank cannot take part (no cut point or an empty range, a failed load, no payload) or
+       ``mode.place`` refuses, rank 0 counts the file whole (``mode.whole``), exactly as a file dealt whole:
+       nothing has touched the matrix yet;
+    4. otherwise every rank counts its range (``mode.own``);
+    5. a second ``gather`` of [failed, totals] sums the totals.  A rank that failed in step 4 raises its
+       own exception after that gather, the others a RuntimeError naming it.
 
-    Returns the file's [reads, with barcode and cut site, clipped on the 3' end, with tag], or None on
-    the ranks other than 0 when rank 0 counted the file whole."""
-    from . import splitter
+    Returns the file's totals, or None on the ranks other than 0 when rank 0 counted the file whole."""
     if gather is None:
         raise ValueError("sharding a file across ranks needs a gather callable (see dist_gather)")
-    dev, lines, head, n = None, 0, b"", 0
+    dev, n, lines, payload = None, 0, 0, None
     try:
         bounds = range_bounds(path, world)
-        if bounds is not None:
+        if bounds is not None and bounds[rank] < bounds[rank + 1]:
             lo, hi = bounds[rank], bounds[rank + 1]
             n = hi - lo
-            head = range_head(path, lo, hi)
-            if head is not None:
-                dev = _load_range(eng, path, lo, n, extra=HEAD_CAP)
+            payload = mode.payload(path, lo, hi)
+            if payload is not None:
+                dev = _load_range(eng, path, lo, n, extra=mode.extra)
                 lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
     except (OSError, _native.TdgError):
         if dev is not None:
             eng.device_free(dev)
             dev = None                          # this rank votes for counting the file whole
-    every = gather([1, lines, len(head)] + list(head) if dev is not None else [0, 0, 0])
-    shards = None
+    every = gather([0] if dev is None else [1, lines] + payload)
+    share = None
     if all(x[0] for x in every):
-        shards = plan_trimmed_shards([x[1] for x in every], [bytes(x[3:3 + x[2]]) for x in every],
-                                     _native.limit_from_maxreads(maxreads))
-    if shards is None:
+        share = mode.place([x[1] for x in every], [x[2:] for x in every], rank)
+    if share is None:
         if dev is not None:
             eng.device_free(dev)
-        if rank != 0:
-            return None
-        tot = splitter.count_trimmed_file(eng, path, barcodes, rows, plan, cutsite=cutsite, adapter=adapter, maxreads=maxreads)
-    else:
-        start, tail, _first, max_records = shards[rank]
-        tot, err = [0, 0, 0, 0], None
-        try:
-            if tail:
-                eng.memcpy_h2d(dev + n, np.frombuffer(tail, dtype=np.uint8).ctypes.data, len(tail))
-            tot = splitter.count_trimmed_resident(eng, dev + start, n - start + len(tail), barcodes, rows, plan, cutsite,
-                                                  adapter, max_records)
-        except Exception as e:                  # every rank still takes part in the second gather
-            err = e
-        finally:
-            eng.device_free(dev)
-        every = gather([0 if err is None else 1] + [int(t) for t in tot])
-        if err is not None:
-            raise err
-        failed = [k for k, x in enumerate(every) if x[0]]
-        if failed:
-            raise RuntimeError("%s: rank %d failed while counting its byte range" % (path, failed[0]))
-        tot = [sum(x[1 + k] for x in every) for k in range(4)]
-    if rank == 0:
-        print("{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}".format(path, *tot))
-    return tot
+        return mode.whole(eng, path) if rank == 0 else None
+    tot, err = [], None
+    try:
+        tot = mode.own(eng, path, rank, dev, n, share)
+    except Exception as e:                      # every rank still takes part in the second gather
+        err = e
+    finally:
+        eng.device_free(dev)
+    every = gather([0 if err is None else 1] + [int(t) for t in tot])
+    if err is not None:
+        raise err
+    failed = [k for k, x in enumerate(every) if x[0]]
+    if failed:
+        raise RuntimeError("%s: rank %d failed while counting its byte range" % (path, failed[0]))
+    return [sum(t) for t in zip(*(x[1:] for x in every))]
 
 
 def dist_gather(values):

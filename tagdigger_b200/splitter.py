@@ -33,7 +33,7 @@ from concurrent.futures import ThreadPoolExecutor
 import numpy as np
 
 from . import _native, hostio, matchset, trimming
-from .counting import _gzip_exception, get_engine
+from .counting import _reference_error, get_engine
 
 BLOCK_READS = 200000          # reads decided per GPU call on the host path
 BLOCK_BYTES = 64 << 20        # bytes streamed through the device per call
@@ -162,16 +162,7 @@ def _open_input(inputFile):
     try:
         return _native.Feed(inputFile, inputFile[-2:].lower() == "gz")
     except _native.TdgError as e:
-        raise _gzip_exception(e.message) if e.code == _native.TDG_ERR_GZIP else OSError(e.message)
-
-
-def _feed_error(e):
-    """The exception the reference's reading raises for a TdgError of the block loop."""
-    if e.code == _native.TDG_ERR_GZIP:
-        return _gzip_exception(e.message)
-    if e.code == _native.TDG_ERR_IO:
-        return OSError(e.message)
-    return e
+        raise _reference_error(e, opening=True)
 
 
 def _block_loop(eng, feed, maxreads, device_block, host_block):
@@ -259,7 +250,7 @@ def barcodeSplitter(inputFile, barcodes, outputFiles, cutsite="TGCAG", adapter=h
         if bgzf:
             write(eng.bgzf_finish())
     except _native.TdgError as e:
-        raise _feed_error(e)
+        raise _reference_error(e)
     finally:
         pool.shutdown()
         feed.close()
@@ -326,7 +317,7 @@ def count_trimmed_file(eng, inputFile, barcodes, rows, plan, cutsite="TGCAG", ad
     try:
         _block_loop(eng, feed, maxreads, device_block, host_block)
     except _native.TdgError as e:
-        raise _feed_error(e)
+        raise _reference_error(e)
     finally:
         feed.close()
     return tot

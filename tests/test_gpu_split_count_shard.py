@@ -1,7 +1,8 @@
-"""One library file sharded across ranks in the one-pass split-and-count mode: tdg_split_count_device
-against tdg_split_count_block on the same bytes, and count_files(..., adapter=...) at world 2 and 3
-(torch.multiprocessing ranks sharing device 0, gloo for the gathers and for the matrix sum) against the
-world-1 run in this process: samples, matrix, totals, rank 0's output and exceptions."""
+"""One library file sharded across ranks: tdg_split_count_device against tdg_split_count_block on the
+same bytes, and count_files at world 2 and 3, in the plain mode and in the one-pass split-and-count mode
+(``adapter=...``), with torch.multiprocessing ranks sharing device 0 and gloo for the gathers and for the
+matrix sum, against the world-1 run in this process: samples, matrix, totals, rank 0's output and
+exceptions, also when rank 1 fails to load or to count its range."""
 
 import contextlib
 import gzip
@@ -146,21 +147,25 @@ def _write(path, text, raw=None):
 
 
 def _cases(root, library):
-    """{name: (directory, key, tags, cutsite, adapter name, split_maxreads, resident call bytes)}."""
+    """{name: (directory, key, tags, cutsite, adapter name, maxreads / split_maxreads, resident call bytes,
+    failure injected on rank 1)}."""
     rng, tags, text = library
     recs = _records(text)
     cases = {}
 
     def add(name, files, key=None, tags_=tags, cutsite="TGCAG", adapter="PstI-MspI-Hall", maxreads=500000000,
-            call_bytes=None):
+            call_bytes=None, inject=None):
         d = os.path.join(root, name.replace(" ", "_"))
         os.makedirs(d)
         for f, t in files.items():
             _write(os.path.join(d, f), t if isinstance(t, str) else None, raw=t if isinstance(t, bytes) else None)
-        cases[name] = (d, key or {f: [BARCODES, SAMPLES] for f in files}, tags_, cutsite, adapter, maxreads, call_bytes)
+        cases[name] = (d, key or {f: [BARCODES, SAMPLES] for f in files}, tags_, cutsite, adapter, maxreads, call_bytes,
+                       inject)
 
     add("lf", {"lib.fq": text})
     add("lf, calls of 40 kB", {"lib.fq": text}, call_bytes=40000)
+    add("load fails on rank 1", {"lib.fq": text}, inject="load")
+    add("count fails on rank 1", {"lib.fq": text}, inject="count")
     add("crlf", {"lib.fq": text.replace("\n", "\r\n")}, call_bytes=40000)
     data = text.encode("utf-8")
     shifted = bytearray(data)
@@ -174,8 +179,8 @@ def _cases(root, library):
     for w in (2, 3):                                           # the limit inside rank 1's range and at its start
         first = _first_record(path, w, 1)
         for m in (first, first + 5):
-            add("split_maxreads %d" % m, {"lib.fq": text}, maxreads=m)
-    add("split_maxreads 7", {"lib.fq": text}, maxreads=7)
+            add("maxreads %d" % m, {"lib.fq": text}, maxreads=m)
+    add("maxreads 7", {"lib.fq": text}, maxreads=7)
     half = len(recs) // 2
     mixed = list(recs)
     for i in range(half + 50, len(mixed), 97):                 # non-ASCII sequence lines in the later ranges
@@ -211,15 +216,18 @@ def _first_record(path, world, rank):
     return counting.plan_trimmed_shards(lines, heads, 1 << 40)[rank][2]
 
 
-def _run(key, tags, cutsite, adapter, maxreads, **kw):
-    """count_files(..., adapter=...) with its output captured: (result, output, exception)."""
+MODES = ("plain", "adapter")
+
+
+def _run(mode, key, tags, cutsite, adapter, maxreads, **kw):
+    """count_files in the plain mode or with ``adapter``, its output captured: (result, output, exception)."""
     out = io.StringIO()
     tot = {}
     res = err = None
+    args = dict(maxreads=maxreads) if mode == "plain" else dict(adapter=adapter, split_maxreads=maxreads)
     try:
         with contextlib.redirect_stdout(out):
-            s, m = counting.count_files(key, tags, cutsite, adapter=adapter, split_maxreads=maxreads, totals=tot,
-                                        as_array=True, device=0, **kw)
+            s, m = counting.count_files(key, tags, cutsite, totals=tot, as_array=True, device=0, **args, **kw)
         res = (s, m.tolist(), tot)
     except Exception as e:  # noqa: BLE001
         err = (type(e).__name__, str(e))
@@ -241,12 +249,21 @@ def _rank_main(rank, world, port, cases, out_dir):
         a = np.ascontiguousarray(t.numpy())
         eng.memcpy_h2d(ptr, a.ctypes.data, a.nbytes)
 
+    def fail(*args, **kw):
+        raise _native.TdgError(_native.TDG_ERR_NOMEM, "injected failure")
+
     results = {}
-    for name, (d, key, tags, cutsite, adapter, maxreads, call_bytes) in sorted(cases.items()):
+    for (name, mode), (d, key, tags, cutsite, adapter, maxreads, call_bytes, inject) in sorted(cases.items()):
         os.chdir(d)
         splitter.RESIDENT_CALL_BYTES = call_bytes or (1 << 30)
-        results[name] = _run(key, tags, cutsite, adapter, maxreads, rank=rank, world=world, reduce=cpu_reduce,
-                             gather=counting.dist_gather)
+        with pytest.MonkeyPatch.context() as mp:
+            if rank == 1 and inject == "load":
+                mp.setattr(counting, "_load_range", fail)
+            if rank == 1 and inject == "count":                 # the own-range count of either mode
+                mp.setattr(_native.Engine, "count_device", fail)
+                mp.setattr(splitter, "count_trimmed_resident", fail)
+            results[name, mode] = _run(mode, key, tags, cutsite, adapter, maxreads, rank=rank, world=world,
+                                       reduce=cpu_reduce, gather=counting.dist_gather)
     with open(os.path.join(out_dir, "rank%d.pkl" % rank), "wb") as fh:
         pickle.dump(results, fh)
     dist.barrier()
@@ -262,13 +279,15 @@ def _free_port():
 @pytest.mark.parametrize("world", [2, 3])
 def test_sharded_count_equals_one_rank(world, tmp_path, library):
     import torch.multiprocessing as mp
-    cases = _cases(str(tmp_path), library)
+    # the plain mode does not check UTF-8 in a sharded range (DESIGN §7), so that case is the adapter mode's
+    cases = {(name, mode): c for name, c in _cases(str(tmp_path), library).items() for mode in MODES
+             if mode == "adapter" or name != "invalid utf-8"}
     want = {}
     old = os.getcwd()
     try:
-        for name, (d, key, tags, cutsite, adapter, maxreads, _cb) in cases.items():
+        for (name, mode), (d, key, tags, cutsite, adapter, maxreads, _cb, _inject) in cases.items():
             os.chdir(d)
-            want[name] = _run(key, tags, cutsite, adapter, maxreads)
+            want[name, mode] = _run(mode, key, tags, cutsite, adapter, maxreads)
     finally:
         os.chdir(old)
     ctx = mp.get_context("spawn")
@@ -289,28 +308,35 @@ def test_sharded_count_equals_one_rank(world, tmp_path, library):
     for r in range(world):
         with open(str(tmp_path / ("rank%d.pkl" % r)), "rb") as fh:
             got.append(pickle.load(fh))
-    for name, (res, out, err) in sorted(want.items()):
+    for case, (res, out, err) in sorted(want.items()):
+        name, mode = case
+        kinds = [g[case][2] for g in got]
         if name == "invalid utf-8":
             assert res is None and err[0] == "UnicodeDecodeError", err
-            kinds = [g[name][2] for g in got]
             assert kinds[1][0] == "UnicodeDecodeError", kinds
+        if name == "count fails on rank 1":
+            assert err is None, err
+            assert kinds[1][0] == "TdgError" and "injected" in kinds[1][1], kinds
+        if name in ("invalid utf-8", "count fails on rank 1"):      # rank 1 raises its own error, the others name it
             assert all(k[0] == "RuntimeError" and "rank 1 " in k[1] for i, k in enumerate(kinds) if i != 1), kinds
             continue
-        assert err is None, (name, err)
+        assert err is None, (case, err)
         for r in range(world):
-            g_res, g_out, g_err = got[r][name]
-            assert g_err is None, (name, r, g_err)
-            assert g_res[0] == res[0] and g_res[1] == res[1], (name, r)
+            g_res, g_out, g_err = got[r][case]
+            assert g_err is None, (case, r, g_err)
+            assert g_res[0] == res[0] and g_res[1] == res[1], (case, r)
             for f, t in g_res[2].items():
-                assert t == res[2][f], (name, r, f)
-        holders = [sorted(got[r][name][0][2]) for r in range(world)]
-        if name in ("lone cr", "giant lines"):                 # counted whole on rank 0
-            assert holders == [["lib.fq"]] + [[]] * (world - 1), name
+                assert t == res[2][f], (case, r, f)
+        holders = [sorted(got[r][case][0][2]) for r in range(world)]
+        # counted whole on rank 0: no cut point, a failed load, and (in the adapter mode, which sends every
+        # range's first lines to the other ranks) lines longer than HEAD_CAP
+        if name in ("lone cr", "load fails on rank 1") or (name, mode) == ("giant lines", "adapter"):
+            assert holders == [["lib.fq"]] + [[]] * (world - 1), case
         elif name != "plain and gzip":                         # sharded: every rank has the file's totals
-            assert holders == [["lib.fq"]] * world, name
+            assert holders == [["lib.fq"]] * world, case
         if name == "plain and gzip" and world == 2:            # two files, two ranks: dealt whole
-            assert sorted(got[0][name][1].splitlines() + got[1][name][1].splitlines()) == sorted(out.splitlines())
+            assert sorted(got[0][case][1].splitlines() + got[1][case][1].splitlines()) == sorted(out.splitlines())
         else:
-            assert got[0][name][1] == out, name
+            assert got[0][case][1] == out, case
         if name == "plain and gzip" and world == 3:
             assert all("a.fq" in h for h in holders), holders
