@@ -187,6 +187,26 @@ int         tdg_release_scratch(tdg_ctx *ctx);
 int         tdg_gz_inflate_host(tdg_ctx *ctx, const char *path, void *dst, size_t cap, uint64_t *n,
                                 int64_t info[4], double ms[6]);
 
+/* The member chain of a BGZF file (what bgzip writes), walked on the host without inflating: *n
+ * receives the number of members, and off[k] / isize[k] the file offset and uncompressed length of
+ * member k when `cap` holds them all.  cap = 0 (off and isize may be NULL) asks for *n only; a
+ * non-zero cap below *n is TDG_ERR_ARG.  TDG_ERR_GZIP: the file is not a clean BGZF chain -- some
+ * member from offset 0 on has no BGZF header, holds more than 65,536 bytes, or runs past the end
+ * of the file, or the file is empty (an empty member, such as the end-of-file marker, is an
+ * ordinary member).  TDG_ERR_IO: the file cannot be opened.  No context; errors via
+ * tdg_last_error(NULL).  Costs 12 bytes of output per member (per 64 KiB of text). */
+int         tdg_bgzf_index(const char *path, uint64_t *off, uint32_t *isize, size_t cap, size_t *n);
+
+/* The complete BGZF members in the file range [c_lo, c_hi) of `path` (member offsets of
+ * tdg_bgzf_index; c_hi may be the file size), inflated ON THE DEVICE into dst[0 .. cap) (device
+ * memory of the caller, any alignment), CRC and length checked against every member's trailer.
+ * *n receives the number of bytes written, *high = 1 when one of them is >= 0x80.  Never falls back to
+ * the host: a member header that is not BGZF, a chain that runs past c_hi or a corrupt member is
+ * TDG_ERR_GZIP, a working buffer that cannot be had is TDG_ERR_NOMEM, a text longer than cap is
+ * TDG_ERR_ARG.  Synchronises.  Used to shard one BGZF file across GPUs by member ranges. */
+int         tdg_bgzf_inflate_device(tdg_ctx *ctx, const char *path, uint64_t c_lo, uint64_t c_hi,
+                                    void *dst, size_t cap, uint64_t *n, int *high);
+
 /* Wait for all submitted work. */
 int         tdg_sync(tdg_ctx *ctx);
 /* Running totals since the last tdg_begin_file (synchronises): reads, reads with

@@ -10,7 +10,13 @@ all-reduce when every rank has a GPU of its own, a CPU all-reduce over gloo othe
 rank: the seconds of the range load, the line count, the gathers, the one-pass count of the owned
 text and the reduce; with the GPU's name and power limit.
 
-    python scripts/split_count_shard_e2e.py [reads] [out.json]
+With --bgzf the library is bgzipped (members of 65,280 bytes of text, as bgzip writes them) and counted in
+both modes: the plain mode with a config-2 tag table (40,000 tags) and the adapter mode as above.  Each is
+counted at world 1 (the device gzip feed inflates the file whole) and sharded by member ranges at world W;
+reported per rank in addition: the seconds of the member index (tdg_bgzf_index), of the device inflate
+(tdg_bgzf_inflate_device), of the plain mode's count (tdg_count_device), and the sum of rank 0's matrix.
+
+    python scripts/split_count_shard_e2e.py [--bgzf] [reads] [out.json]
 """
 import contextlib
 import io
@@ -41,7 +47,21 @@ def timed(times, key, fn):
     return run
 
 
-def rank_main(rank, world, port, ngpu, key, tags, out_dir):
+def bgzip(src, dst):
+    """``src`` as BGZF (one member per 65,280 bytes, compressed by a pool of processes, then the EOF marker)."""
+    import multiprocessing
+    from feed_check import bgzf_block
+    with open(src, "rb") as fh:
+        data = fh.read()
+    pieces = [data[i:i + 65280] for i in range(0, len(data), 65280)]
+    with multiprocessing.Pool() as pool:
+        blocks = pool.starmap(bgzf_block, [(p, 1) for p in pieces], chunksize=256)
+    with open(dst, "wb") as fh:
+        fh.writelines(blocks)
+        fh.write(bgzf_block(b""))
+
+
+def rank_main(rank, world, port, ngpu, key, tags, out_dir, adapter="PstI-MspI-Hall", tag="x"):
     import torch
     import torch.distributed as dist
     from tagdigger_b200 import _native, counting, splitter
@@ -62,18 +82,24 @@ def rank_main(rank, world, port, ngpu, key, tags, out_dir):
 
     times = {}
     counting._load_range = timed(times, "load_s", counting._load_range)
+    counting._load_bgzf_share = timed(times, "load_s", counting._load_bgzf_share)
+    _native.bgzf_index = timed(times, "index_s", _native.bgzf_index)
+    _native.Engine.bgzf_inflate_device = timed(times, "inflate_s", _native.Engine.bgzf_inflate_device)
     _native.Engine.count_lines_device = timed(times, "line_count_s", _native.Engine.count_lines_device)
+    _native.Engine.count_device = timed(times, "count_s", _native.Engine.count_device)
     splitter.count_trimmed_resident = timed(times, "split_count_s", splitter.count_trimmed_resident)
     gather = timed(times, "gathers_s", counting.dist_gather)
+    totals = {}
     reduce = timed(times, "reduce_s", counting.engine_reduce if own_gpu else cpu_reduce)
     dist.barrier()
     t0 = time.perf_counter()
     with contextlib.redirect_stdout(io.StringIO()):
         _, matrix = counting.count_files(key, tags, "TGCAG", device=device, rank=rank, world=world, reduce=reduce,
-                                         gather=gather, as_array=True, adapter="PstI-MspI-Hall")
+                                         gather=gather, as_array=True, adapter=adapter, totals=totals)
     times["count_files_s"] = time.perf_counter() - t0
-    res = {"rank": rank, "device": device, **{k: round(v, 4) for k, v in times.items()}}
-    with open(os.path.join(out_dir, "rank%d.pkl" % rank), "wb") as fh:
+    res = {"rank": rank, "device": device, **{k: round(v, 4) for k, v in times.items()},
+           "holds_file": bool(totals), "matrix_sum": int(matrix.sum())}
+    with open(os.path.join(out_dir, "rank%d_%s.pkl" % (rank, tag)), "wb") as fh:
         pickle.dump((res, matrix if rank == 0 else None), fh)
     dist.barrier()
     dist.destroy_process_group()
@@ -83,8 +109,10 @@ def main():
     import torch
     import torch.multiprocessing as mp
     from tagdigger_b200 import counting, hostio, synth
-    reads = int(sys.argv[1]) if len(sys.argv) > 1 else 8_000_000
-    out_json = sys.argv[2] if len(sys.argv) > 2 else os.path.join(REPO, "profiles", "r03_split_count_shard_e2e.json")
+    args = [a for a in sys.argv[1:] if a != "--bgzf"]
+    use_bgzf = "--bgzf" in sys.argv[1:]
+    reads = int(args[0]) if args else 8_000_000
+    out_json = args[1] if len(args) > 1 else os.path.join(REPO, "profiles", "r03_split_count_shard_e2e.json")
     ngpu = torch.cuda.device_count()
     if ngpu < 1:
         raise SystemExit("needs a GPU")
@@ -106,6 +134,9 @@ def main():
         for _ in range(max(1, reads // unit)):
             fh.write(text)
     reads = max(1, reads // unit) * unit
+    if use_bgzf:
+        sys.path.insert(0, os.path.join(REPO, "tests"))
+        return bgzf_legs(inp, tmp, reads, barcodes, tags, kept_tags, ngpu, world, out_json)
     key = {inp: [list(barcodes), ["Sample%02d" % i for i in range(len(barcodes))]]}
     res = {"config": "config 5 shape: %d reads (150 bp), PstI-MspI-Hall adapters, 96-plex, %d tags of which %d kept"
                      % (reads, len(tags), len(kept_tags)),
@@ -124,7 +155,7 @@ def main():
     ranks = []
     got = None
     for r in range(world):
-        with open(os.path.join(tmp, "rank%d.pkl" % r), "rb") as fh:
+        with open(os.path.join(tmp, "rank%d_x.pkl" % r), "rb") as fh:
             info, m = pickle.load(fh)
         ranks.append(info)
         if r == 0:
@@ -143,6 +174,67 @@ def main():
         os.remove(os.path.join(tmp, f))
     os.rmdir(tmp)
     return 0 if np.array_equal(got, want) else 1
+
+
+def bgzf_legs(inp, tmp, reads, barcodes, tags, kept_tags, ngpu, world, out_json):
+    import torch.multiprocessing as mp
+    from tagdigger_b200 import counting, synth
+    gz = inp + ".gz"
+    t0 = time.perf_counter()
+    bgzip(inp, gz)
+    bgzip_s = time.perf_counter() - t0
+    text_mb = os.path.getsize(inp) / 1e6
+    os.remove(inp)
+    names, _, seqs = synth.make_marker_pairs(18000, np.random.default_rng(7))
+    config2_tags = list(tags) + [s for p in seqs for s in p]            # 4,000 + 36,000 tags
+    key = {gz: [list(barcodes), ["Sample%02d" % i for i in range(len(barcodes))]]}
+    res = {"config": "%d reads (150 bp, the config-5 generator), 96-plex, bgzipped; plain mode with %d tags (config-2 "
+                     "table), adapter mode (PstI-MspI-Hall) with %d kept tags" % (reads, len(config2_tags), len(kept_tags)),
+           "text_MB": round(text_mb, 1), "bgzf_MB": round(os.path.getsize(gz) / 1e6, 1), "bgzip_s": round(bgzip_s, 1),
+           "gpu": gpu_name_and_power_limit(), "gpus": ngpu, "world": world, "host_cpus": os.cpu_count(),
+           "ranks_share_one_gpu": world > ngpu}
+    if world > ngpu:
+        res["note"] = "ranks share one GPU: a correctness run; whole-box speed-up not measured"
+    ok = True
+    for leg, adapter, leg_tags in (("plain", None, config2_tags), ("adapter", "PstI-MspI-Hall", kept_tags)):
+        out = {}
+        with contextlib.redirect_stdout(io.StringIO()):
+            counting.count_files(key, leg_tags, "TGCAG", as_array=True, adapter=adapter)          # warm-up
+            t0 = time.perf_counter()
+            _, want = counting.count_files(key, leg_tags, "TGCAG", as_array=True, adapter=adapter)
+            out["world1_s"] = round(time.perf_counter() - t0, 3)
+        with socket.socket() as s:
+            s.bind(("127.0.0.1", 0))
+            port = s.getsockname()[1]
+        t0 = time.perf_counter()
+        mp.spawn(rank_main, args=(world, port, ngpu, key, leg_tags, tmp, adapter, leg), nprocs=world, join=True)
+        out["worldW_spawn_to_end_s"] = round(time.perf_counter() - t0, 3)
+        ranks = []
+        for r in range(world):
+            with open(os.path.join(tmp, "rank%d_%s.pkl" % (r, leg)), "rb") as fh:
+                info, m = pickle.load(fh)
+            ranks.append(info)
+            if r == 0:
+                got = m
+        out["ranks"] = ranks
+        out["worldW_count_files_s"] = max(r["count_files_s"] for r in ranks)
+        out["speedup_count_files"] = round(out["world1_s"] / out["worldW_count_files_s"], 3)
+        out["world1_reads_per_s"] = round(reads / out["world1_s"])
+        out["cells"] = int(want.size)
+        out["matrix_sum_world1"] = int(want.sum())
+        out["matrix_equals_world1"] = "ok (every cell)" if np.array_equal(got, want) else "FAILED"
+        out["sharded"] = all(r["holds_file"] for r in ranks)
+        ok = ok and np.array_equal(got, want)
+        res[leg] = out
+    line = json.dumps(res)
+    print(line)
+    os.makedirs(os.path.dirname(os.path.abspath(out_json)), exist_ok=True)
+    with open(out_json, "w") as fh:
+        fh.write(line + "\n")
+    for f in os.listdir(tmp):
+        os.remove(os.path.join(tmp, f))
+    os.rmdir(tmp)
+    return 0 if ok else 1
 
 
 if __name__ == "__main__":

@@ -34,7 +34,7 @@ NO_LIMIT = (1 << 63)
 
 EXPORTS = """tdg_abi_version tdg_create tdg_destroy tdg_last_error tdg_set_tags tdg_set_matrix
 tdg_bind_matrix tdg_zero_matrix tdg_begin_file tdg_reset_file tdg_submit tdg_end_file tdg_count_device
-tdg_count_lines_device tdg_count_file tdg_count_file2 tdg_last_file_info tdg_gz_inflate_host tdg_release_scratch tdg_sync tdg_file_totals tdg_read_matrix tdg_matrix_min tdg_comm_unique_id tdg_comm_init tdg_allreduce_matrix tdg_finish
+tdg_count_lines_device tdg_count_file tdg_count_file2 tdg_last_file_info tdg_gz_inflate_host tdg_bgzf_index tdg_bgzf_inflate_device tdg_release_scratch tdg_sync tdg_file_totals tdg_read_matrix tdg_matrix_min tdg_comm_unique_id tdg_comm_init tdg_allreduce_matrix tdg_finish
 tdg_matrix_device_ptr tdg_stream tdg_stream_wait tdg_other_stream_wait tdg_host_alloc
 tdg_host_free tdg_device_alloc tdg_device_free tdg_memcpy_h2d tdg_memcpy_d2h tdg_launch_count
 tdg_timing_begin tdg_timing_end tdg_set_trim tdg_trim_batch tdg_split_batch tdg_split_begin tdg_split_block
@@ -114,6 +114,8 @@ def lib():
         "tdg_count_file": (i32, [vp, ctypes.c_char_p, i32, u64, vp]),
         "tdg_count_file2": (i32, [vp, ctypes.c_char_p, i32, u64, vp, ctypes.c_char_p, i32]),
         "tdg_gz_inflate_host": (i32, [vp, ctypes.c_char_p, vp, sz, vp, vp, vp]),
+        "tdg_bgzf_index": (i32, [ctypes.c_char_p, vp, vp, sz, ctypes.POINTER(sz)]),
+        "tdg_bgzf_inflate_device": (i32, [vp, ctypes.c_char_p, u64, u64, vp, sz, ctypes.POINTER(u64), ctypes.POINTER(i32)]),
         "tdg_last_file_info": (i32, [vp, vp]),
         "tdg_release_scratch": (i32, [vp]),
         "tdg_sync": (i32, [vp]),
@@ -222,6 +224,24 @@ def write_counts_csv(path, matrix, samnames, tagnames, threads=8):
                                 header, len(header), blob, off.ctypes.data, threads)
     if rc != TDG_OK:
         raise OSError(L.tdg_last_error(None).decode())
+
+
+def bgzf_index(path):
+    """The member chain of a BGZF file (tdg_bgzf_index): (offsets uint64, ISIZEs uint32), one entry per member,
+    or None when ``path`` is not a clean BGZF chain from offset 0 to its end.  TdgError when it cannot be read."""
+    L = lib()
+    n = ctypes.c_size_t(0)
+    off = isize = np.empty(0, dtype=np.uint64)
+    for cap in (0, None):                    # the number of members, then the members
+        if cap is None:
+            cap = n.value
+            off, isize = np.empty(cap, dtype=np.uint64), np.empty(cap, dtype=np.uint32)
+        rc = L.tdg_bgzf_index(os.fsencode(path), off.ctypes.data, isize.ctypes.data, cap, ctypes.byref(n))
+        if rc == TDG_ERR_GZIP:
+            return None
+        if rc != TDG_OK:
+            raise TdgError(rc, L.tdg_last_error(None).decode())
+    return off[:n.value], isize[:n.value]
 
 
 def write_geno_csv(path, matrix, samnames, markers, col0, col1, threads=8):
@@ -348,6 +368,15 @@ class Engine(object):
         keys = ("upload", "scan", "decode", "resolve", "crc", "copy")
         return (out[:n.value].tobytes(), {"rounds": int(info[0]), "chunks": int(info[1]), "accepted": int(info[2]), "mode": int(info[3])},
                 dict(zip(keys, (round(float(x), 2) for x in ms))))
+
+    def bgzf_inflate_device(self, path, c_lo, c_hi, dev_ptr, cap):
+        """The BGZF members in the file range [c_lo, c_hi) of ``path``, inflated on the device into
+        dev_ptr[0 .. cap) (tdg_bgzf_inflate_device).  Returns (bytes written, whether one is >= 0x80)."""
+        n = ctypes.c_uint64(0)
+        high = ctypes.c_int(0)
+        self._ck(self._L.tdg_bgzf_inflate_device(self._h, os.fsencode(path), int(c_lo), int(c_hi), dev_ptr, cap, ctypes.byref(n),
+                                                 ctypes.byref(high)))
+        return n.value, bool(high.value)
 
     def last_file_info(self):
         """How the last count_file fed its file: {rounds, accepted, mode} (mode 0 device, 1 host took over, -1 host only)."""

@@ -217,7 +217,8 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
     size (largest first, to the least loaded rank) and ``reduce(ptr, rows, cols,
     engine)`` must sum the per-rank matrices in place (one NCCL all-reduce, see
     :func:`nccl_reduce`); integer sums make the result independent of ``world``.  When there are
-    fewer files than ranks, plain files are sharded by byte range instead and counted first
+    fewer files than ranks, plain files are sharded by byte range, and BGZF files by member range,
+    instead and counted first
     (:func:`_count_sharded`, which needs ``gather(list_of_ints) -> list of every rank's list``,
     :func:`dist_gather`).  Results, rank 0's output and exceptions stay those of a one-rank run.
 
@@ -247,10 +248,10 @@ def count_files(bckeys, tags, cutsite="TGCAG", maxreads=5e9, device=None, rank=0
     eng.set_tags(mode.tags.patterns, mode.tags.index, any_base=mode.tags.any_base)
     eng.set_matrix(len(samples), len(tags))
     split = shard_files(files, world)
-    todo = split + assign_files([f for f in files if f not in split], rank, world)
+    todo = list(split) + assign_files([f for f in files if f not in split], rank, world)
     for i, f in enumerate(todo):
         if f in split:
-            tot = _count_sharded(eng, mode, f, rank, world, gather)
+            tot = _count_sharded(eng, mode, f, rank, world, gather, split[f])
             if tot is None:
                 continue                          # rank 0 counted the file whole
         else:
@@ -277,10 +278,11 @@ class _PlainCount:
     set-up checks, file by file, before anything is counted.  What the mode supplies to count_files and
     :func:`_count_sharded`: ``tags`` (the tag plan), ``line`` (the format of a file's output line),
     ``whole`` (count a whole file), ``payload`` / ``extra`` / ``place`` (what a rank adds to the
-    first gather, the room it needs behind its range, and where its range lies in the file) and ``own``
-    (count its range)."""
+    first gather, the room it needs behind its range, and where its range lies in the file), ``own``
+    (count its range) and ``ascii_only`` (a range of a BGZF file with a byte >= 0x80 is not sharded)."""
     line = "{0}: Reads: {1} With barcode and cut site: {2} With tag: {3}"
     extra = 0
+    ascii_only = True         # tdg_count_device does not check UTF-8 (DESIGN §7): sharded BGZF text stays ASCII
 
     def __init__(self, bckeys, files, rows, tags, cutsite, maxreads):
         self.limit = _native.limit_from_maxreads(maxreads)
@@ -302,7 +304,7 @@ class _PlainCount:
         load_plan(eng, self.plans[f], row_of=self.rows[f], set_tags=False)
         return _run_file(eng, f, self.limit, next_file)[:3]
 
-    def payload(self, f, lo, hi):
+    def payload(self, head):
         return []
 
     def place(self, lines, payloads, rank):
@@ -319,6 +321,7 @@ class _TrimmedCount:
     """count_files' one-pass split-trim-count mode (``adapter``), with the members of :class:`_PlainCount`.
     Set-up errors surface in the order of the two-stage run: every file's split, then the count."""
     line = "{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}"
+    ascii_only = False        # non-ASCII records go to the host (tdg_split_count_device's needs_host)
 
     def __init__(self, bckeys, files, rows, tags, cutsite, maxreads, adapter, split_cutsite, split_maxreads):
         from . import hostio, splitter
@@ -349,10 +352,11 @@ class _TrimmedCount:
         return splitter.count_trimmed_file(eng, f, self.bckeys[f][0], self.rows[f], self.plan, cutsite=self.cutsite,
                                            adapter=self.adapter, maxreads=self.maxreads)
 
-    def payload(self, f, lo, hi):
-        """The range's head (:func:`range_head`), or None when it is too long to send."""
-        head = range_head(f, lo, hi)
-        return None if head is None else list(head)
+    def payload(self, head):
+        """The range's head (``head()``: :func:`range_head` for a plain file, the loaded text's for a BGZF
+        file), or None when it is too long to send."""
+        h = head()
+        return None if h is None else list(h)
 
     def place(self, lines, payloads, rank):
         """The range's owned text and record budget (:func:`plan_trimmed_shards`); None to count the file whole."""
@@ -372,12 +376,36 @@ SHARD_MIN_BYTES = 1 << 20     # files smaller than this per rank are not worth c
 
 
 def shard_files(files, world):
-    """The files of a key that count_files cuts into one byte range per rank (both counting modes):
-    with fewer files than ranks, every plain (uncompressed) file that is large enough.  The other
-    files are dealt whole to the ranks."""
+    """The files of a key that count_files cuts into one range per rank (both counting modes), each with
+    its BGZF member index (None for a plain file): with fewer files than ranks, every file that is large
+    enough and either plain (uncompressed: cut by byte ranges) or a clean BGZF member chain
+    (``_native.bgzf_index``: cut by member ranges, which are inflated on the device, so not with
+    TDG_GZDEV=0).  The other files are dealt whole to the ranks."""
     if world <= 1 or len(files) >= world:
-        return []
-    return [f for f in files if not _is_gz(f) and shardable(f, world)]
+        return {}
+    out = {}
+    for f in files:
+        if not shardable(f, world):
+            continue
+        if not _is_gz(f):
+            out[f] = None
+        elif not _host_inflate_only():
+            try:
+                index = _native.bgzf_index(f)
+            except _native.TdgError:
+                index = None
+            if index is not None:
+                out[f] = index
+    return out
+
+
+def _host_inflate_only():
+    """TDG_GZDEV=0, read as the library reads it (atoi): gzip files are inflated on the host."""
+    e = os.environ.get("TDG_GZDEV")
+    if e is None:
+        return False
+    m = re.match(r"\s*([+-]?\d+)", e)
+    return m is None or int(m.group(1)) == 0
 
 
 def shardable(f, world):
@@ -417,12 +445,16 @@ def range_bounds(path, world):
     return bounds
 
 
+def _device_room(n):
+    """The allocation tdg_count_device asks for behind a device image of ``n`` bytes."""
+    return (n + _native.TDG_TILE_BYTES - 1) // _native.TDG_TILE_BYTES * _native.TDG_TILE_BYTES + _native.TDG_HALO_BYTES
+
+
 def _load_range(eng, path, lo, n, extra=0):
     """Bytes [lo, lo + n) of ``path`` in a fresh device allocation padded as tdg_count_device asks, with
     ``extra`` more bytes of room behind them; read with pread through one pinned buffer of at most
     256 MiB.  Returns the device pointer (free with device_free)."""
-    cap = (n + extra + _native.TDG_TILE_BYTES - 1) // _native.TDG_TILE_BYTES * _native.TDG_TILE_BYTES + _native.TDG_HALO_BYTES
-    dev = eng.device_alloc(cap)
+    dev = eng.device_alloc(_device_room(n + extra))
     try:
         piece = 256 << 20
         host = eng.host_alloc(min(piece, max(n, 1)))
@@ -467,7 +499,20 @@ def range_head(path, lo, hi):
     with open(path, "rb") as fh:
         fh.seek(lo)
         data = fh.read(min(hi - lo, HEAD_CAP + 1))
-    whole = len(data) == hi - lo
+    return _head(data, len(data) == hi - lo)
+
+
+def _device_head(eng, dev, n):
+    """:func:`range_head` of the ``n`` bytes of text at device address ``dev``."""
+    k = min(n, HEAD_CAP + 1)
+    buf = np.empty(k, dtype=np.uint8)
+    if k:
+        eng.memcpy_d2h(buf.ctypes.data, dev, k)
+    return _head(buf.tobytes(), k == n)
+
+
+def _head(data, whole):
+    """The head of a range that begins with ``data`` (all of it when ``whole``)."""
     ends = line_ends(data, 3, whole)
     if len(ends) == 3:
         data = data[:ends[2]]
@@ -504,16 +549,159 @@ def plan_trimmed_shards(lines, heads, limit):
     return out
 
 
-def _count_sharded(eng, mode, path, rank, world, gather):
-    """One file that count_files cuts into one byte range per rank (:func:`shard_files`), in either counting
-    mode (``mode``: :class:`_PlainCount` or :class:`_TrimmedCount`).  Lines, reads and records are numbered
-    from the start of the FILE (tagdigger_fun.py:250-254), so a range cannot be counted on its own:
+LOOKAHEAD_CAP = 16 << 20     # as range_bounds: a cut followed by no '\n' within this much text is not sharded
 
-    1. every rank loads its range of :func:`range_bounds` into device memory (:func:`_load_range`), with
-       ``mode.extra`` bytes of room behind it, and counts its line starts there (``tdg_count_lines_device``);
+
+def plan_bgzf_share(off, isize, size, rank, world, text_of, cap=None):
+    """The text rank ``rank`` of ``world`` owns of a BGZF file of ``size`` bytes whose members start at file
+    offsets ``off`` and hold ``isize`` bytes of text each (``_native.bgzf_index``): :func:`range_bounds` in
+    text coordinates.  The file is cut at members: c[r] is the first member that starts at or after
+    size * r // world (c[0] = 0, c[world] = the end), a function of the file alone, so every rank finds the same
+    cuts.  T_r is the text of members [c[r], c[r+1]).  Rank r > 0 owns text from just after the first '\n' of
+    T_r; rank r < world - 1 owns text up to just after the first '\n' of T_{r+1}, which it finds by looking
+    ahead, member after member, at most ``cap`` bytes of text (LOOKAHEAD_CAP) into T_{r+1}.  So every range
+    starts at a line start, and the ranges of all ranks put together are the whole text.
+
+    ``text_of(k0, k1)`` returns the text of members [k0, k1).  Returns (lo, hi, k_first, k_last, front, back):
+    the owned text is text[lo:hi] = front + the text of members [k_first, k_last) + back.  None (count the
+    file whole) when T_r has no '\n' within ``cap`` bytes (r > 0), the look-ahead finds none within ``cap``
+    bytes, or the owned text is empty."""
+    cap = LOOKAHEAD_CAP if cap is None else cap
+    m = len(off)
+    t = np.zeros(m + 1, dtype=np.int64)
+    np.cumsum(np.asarray(isize, dtype=np.int64), out=t[1:])
+    starts = np.asarray(off, dtype=np.int64)
+    c = [0] + [int(np.searchsorted(starts, size * r // world, side="left")) for r in range(1, world)] + [m]
+
+    def first_lf(k, stop):
+        """(text of members [k, j), the position of its first '\n') for the first j that holds one; members
+        are taken one, two, four ... at a time.  None when members [k, stop) hold none within ``cap`` bytes."""
+        got, n, step = [], 0, 1
+        while k < stop and n < cap:
+            j = min(stop, k + step)
+            piece = text_of(k, j)
+            at = piece.find(b"\n")
+            if at >= 0:
+                return (b"".join(got) + piece, n + at, j) if n + at < cap else None
+            got.append(piece)
+            n += len(piece)
+            k, step = j, step * 2
+        return None
+
+    lo, k_first, front = 0, 0, b""
+    if rank > 0:
+        found = first_lf(c[rank], c[rank + 1])
+        if found is None:
+            return None
+        data, at, k_first = found
+        lo, front = int(t[c[rank]]) + at + 1, data[at + 1:]
+    hi, k_last, back = int(t[m]), m, b""
+    if rank < world - 1:
+        found = first_lf(c[rank + 1], m)
+        if found is None:
+            return None
+        data, at, _ = found
+        hi, k_last, back = int(t[c[rank + 1]]) + at + 1, c[rank + 1], data[:at + 1]
+    return (lo, hi, k_first, k_last, front, back) if lo < hi else None
+
+
+def _load_bgzf_share(eng, path, index, rank, world, extra, ascii_only):
+    """The owned text of a BGZF file (:func:`plan_bgzf_share`) in a fresh device allocation padded as
+    tdg_count_device asks, with ``extra`` bytes of room behind it: the members in between are inflated on the
+    device straight into it (``tdg_bgzf_inflate_device``), the partial members at its two ends, which the
+    plan inflated to find the cuts, are copied there from the host.  Returns (device pointer, length), or
+    None when the plan refuses, or ``ascii_only`` and a byte of the text is >= 0x80."""
+    off, isize = index
+    size = os.path.getsize(path)
+    t = np.zeros(len(off) + 1, dtype=np.int64)
+    np.cumsum(np.asarray(isize, dtype=np.int64), out=t[1:])
+
+    def at(k):
+        return int(off[k]) if k < len(off) else size
+
+    def text_of(k0, k1):
+        n = int(t[k1] - t[k0])
+        if not n:
+            return b""
+        dev = eng.device_alloc(n)
+        try:
+            got, _high = eng.bgzf_inflate_device(path, at(k0), at(k1), dev, n)
+            buf = np.empty(got, dtype=np.uint8)
+            eng.memcpy_d2h(buf.ctypes.data, dev, got)
+        finally:
+            eng.device_free(dev)
+        return buf.tobytes()
+
+    share = plan_bgzf_share(off, isize, size, rank, world, text_of)
+    if share is None:
+        return None
+    lo, hi, k_first, k_last, front, back = share
+    if ascii_only and not (front.isascii() and back.isascii()):
+        return None
+    n = hi - lo
+    mid = n - len(front) - len(back)
+    dev = eng.device_alloc(_device_room(n + extra))
+    try:
+        if front:
+            eng.memcpy_h2d(dev, np.frombuffer(front, dtype=np.uint8).ctypes.data, len(front))
+        if mid:
+            got, high = eng.bgzf_inflate_device(path, at(k_first), at(k_last), dev + len(front), mid)
+            if got != mid:
+                raise _native.TdgError(_native.TDG_ERR_GZIP, "%s: %d bytes of text where the index has %d" % (path, got, mid))
+            if ascii_only and high:
+                eng.device_free(dev)
+                return None
+        if back:
+            eng.memcpy_h2d(dev + n - len(back), np.frombuffer(back, dtype=np.uint8).ctypes.data, len(back))
+    except BaseException:
+        eng.device_free(dev)
+        raise
+    return dev, n
+
+
+def _load_share(eng, mode, path, rank, world, index):
+    """Step 1 of :func:`_count_sharded` up to the line count: this rank's text of ``path`` in device memory, with
+    ``mode.extra`` bytes of room behind it -- its byte range of a plain file (``index`` None: :func:`range_bounds`,
+    :func:`_load_range`) or its owned text of a BGZF file (``index``: :func:`_load_bgzf_share`) -- and
+    ``mode.payload`` of its head.  Returns (device pointer, length, payload), or None: the rank votes for
+    counting the file whole."""
+    if index is None:
+        bounds = range_bounds(path, world)
+        if bounds is None or bounds[rank] >= bounds[rank + 1]:
+            return None
+        lo, hi = bounds[rank], bounds[rank + 1]
+        payload = mode.payload(lambda: range_head(path, lo, hi))
+        if payload is None:
+            return None
+        return _load_range(eng, path, lo, hi - lo, extra=mode.extra), hi - lo, payload
+    loaded = _load_bgzf_share(eng, path, index, rank, world, mode.extra, mode.ascii_only)
+    if loaded is None:
+        return None
+    dev, n = loaded
+    try:
+        payload = mode.payload(lambda: _device_head(eng, dev, n))
+    except BaseException:
+        eng.device_free(dev)
+        raise
+    if payload is None:
+        eng.device_free(dev)
+        return None
+    return dev, n, payload
+
+
+def _count_sharded(eng, mode, path, rank, world, gather, index=None):
+    """One file that count_files cuts into one range per rank (:func:`shard_files`), in either counting
+    mode (``mode``: :class:`_PlainCount` or :class:`_TrimmedCount`); ``index``: the member index of a BGZF
+    file, None for a plain file.  Lines, reads and records are numbered from the start of the FILE
+    (tagdigger_fun.py:250-254), so a range cannot be counted on its own:
+
+    1. every rank loads its range into device memory (:func:`_load_share`: a byte range of a plain file, the
+       owned text of a BGZF file, inflated on the device), with ``mode.extra`` bytes of room behind it, and
+       counts its line starts there (``tdg_count_lines_device``);
     2. one ``gather`` of [ok, line starts, ``mode.payload``] tells every rank where its range lies in the
        file (``mode.place``);
-    3. if some rank cannot take part (no cut point or an empty range, a failed load, no payload) or
+    3. if some rank cannot take part (no cut point or an empty range, a failed load or inflate, no payload,
+       a byte >= 0x80 in BGZF text of the plain mode) or
        ``mode.place`` refuses, rank 0 counts the file whole (``mode.whole``), exactly as a file dealt whole:
        nothing has touched the matrix yet;
     4. otherwise every rank counts its range (``mode.own``);
@@ -525,14 +713,10 @@ def _count_sharded(eng, mode, path, rank, world, gather):
         raise ValueError("sharding a file across ranks needs a gather callable (see dist_gather)")
     dev, n, lines, payload = None, 0, 0, None
     try:
-        bounds = range_bounds(path, world)
-        if bounds is not None and bounds[rank] < bounds[rank + 1]:
-            lo, hi = bounds[rank], bounds[rank + 1]
-            n = hi - lo
-            payload = mode.payload(path, lo, hi)
-            if payload is not None:
-                dev = _load_range(eng, path, lo, n, extra=mode.extra)
-                lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
+        loaded = _load_share(eng, mode, path, rank, world, index)
+        if loaded is not None:
+            dev, n, payload = loaded
+            lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
     except (OSError, _native.TdgError):
         if dev is not None:
             eng.device_free(dev)

@@ -1592,6 +1592,47 @@ int tdg_gz_inflate_host(tdg_ctx *ctx, const char *path, void *dst, size_t cap, u
     return TDG_OK;
 }
 
+// The member chain of a BGZF file, walked on the host with the feeder's header parser (no context: errors go
+// to tdg_last_error(NULL)).  *n receives the number of members; off / isize receive them when cap holds them.
+int tdg_bgzf_index(const char *path, uint64_t *off, uint32_t *isize, size_t cap, size_t *n)
+{
+    if (!path || !n || (cap && (!off || !isize))) return fail(nullptr, TDG_ERR_ARG, "null argument");
+    GzMap map;
+    if (!gz_map_file(map, path)) return fail(nullptr, TDG_ERR_IO, std::string("cannot open ") + path);
+    std::vector<uint64_t> o;
+    std::vector<uint32_t> s;
+    const std::string why = bgzf_chain(map, o, s);
+    if (!why.empty()) return fail(nullptr, TDG_ERR_GZIP, std::string(path) + " is not a BGZF member chain: " + why);
+    *n = o.size();
+    if (!cap) return TDG_OK;
+    if (cap < o.size()) return fail(nullptr, TDG_ERR_ARG, "tdg_bgzf_index: room for " + std::to_string(cap) + " members, the file has " +
+                                                                std::to_string(o.size()));
+    memcpy(off, o.data(), o.size() * 8);
+    memcpy(isize, s.data(), s.size() * 4);
+    return TDG_OK;
+}
+
+// The BGZF members in [c_lo, c_hi) of `path`, inflated on the device into caller device memory (gz_bgzf_inflate_range).
+int tdg_bgzf_inflate_device(tdg_ctx *ctx, const char *path, uint64_t c_lo, uint64_t c_hi, void *dst, size_t cap, uint64_t *n, int *high)
+{
+    int rc = need_device(ctx);
+    if (rc) return rc;
+    if (!path || !n || !high || (!dst && cap)) return fail(ctx, TDG_ERR_ARG, "null argument");
+    CK(cudaSetDevice(ctx->device));
+    rc = ensure_slots(ctx);
+    if (rc) return rc;
+    ctx->ahead.reset();                      // the read-ahead thread writes into the pinned file buffers the upload uses
+    rc = ensure_file_bufs(ctx, 0);
+    if (rc) return rc;
+    uint64_t got = 0;
+    bool hi = false;
+    rc = gz_bgzf_inflate_range(ctx, path, (size_t)c_lo, (size_t)c_hi, (uint8_t *)dst, cap, got, hi);
+    if (rc) return rc;
+    *n = got;
+    *high = hi ? 1 : 0;
+    return TDG_OK;
+}
+
 // ---------------------------------------------------------------------------
 // Trim decision (barcode splitter), csrc/tdg_trim.cuh
 

@@ -1,5 +1,6 @@
 // Host side of the device gzip feed: rounds, uploads, the checks against trailers, the hand-over to
-// the host feeder, the read limit, and the two sinks (counting; copying out).  The kernels are in
+// the host feeder, the read limit, the sinks (counting; copying out to the host or to device memory), and the
+// BGZF member chain and member ranges that shard one BGZF file across GPUs.  The kernels are in
 // tdg_gzdev.cuh, the per-lane inflater in tdg_gzlane.h, the chain of a round in tdg_gzchain.h.
 //
 // This file is PART OF tdg_api.cu (included there, inside its anonymous namespace, behind the
@@ -192,9 +193,11 @@ struct GzFeed {
     int cur = 0;                 // which compressed buffer the round reads
     bool pre_valid = false;      // the other one holds [pre_off, pre_end) of the file
     size_t pre_off = 0, pre_end = 0;
-    // BGZF: the next member, and the bytes of text in front of it
-    size_t off = 0;
+    // BGZF: the next member, where the members end (the file's end, or a caller's stop offset), the
+    // bytes of text in front of the next member, and whether any of them is >= 0x80
+    size_t off = 0, stop = 0;
     uint64_t delivered = 0;
+    bool high = false;
 
     int upload(int which, size_t from, size_t end, cudaStream_t stream) { return gz_upload(ctx, map, path, threads, up_i, which, from, end, stream); }
     int to_sink(uint64_t text_len)
@@ -322,9 +325,9 @@ int gz_bgzf_round(GzFeed &f)
     auto t0 = GzClock::now();
     std::vector<Member> mem;
     size_t end = f.off;
-    while (end < map.n && mem.size() < f.max_chunks && end - f.off < ((size_t)1 << 30)) {
+    while (end < f.stop && mem.size() < f.max_chunks && end - f.off < ((size_t)1 << 30)) {
         uint32_t csize = 0, hlen = 0;
-        if (!Feeder::bgzf_member(map.p + end, std::min<size_t>(map.n - end, 1024), csize, hlen) || end + csize > map.n) {
+        if (!Feeder::bgzf_member(map.p + end, std::min<size_t>(map.n - end, 1024), csize, hlen) || end + csize > f.stop) {
             f.handover = true;
             break;
         }
@@ -413,13 +416,14 @@ int gz_bgzf_round(GzFeed &f)
         for (uint32_t k = 0; k < n; k++)
             if (h[1 + k] != mem[k].crc) return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + f.path + ": corrupt BGZF member");
         if ((rc = gz_check_utf8(f, h[0], text_len))) return rc;
+        f.high |= (h[0] & 0x80u) != 0;
         if ((rc = f.to_sink(text_len))) return rc;
     } else {
         ctx->launches++;                                                                 // gz_decode
     }
     f.delivered += text_len;
     f.off = end;
-    f.done = f.off == map.n;
+    f.done = f.off == f.stop;
     f.stats.rounds++;
     f.stats.chunks += n;
     f.stats.accepted += n;
@@ -645,24 +649,26 @@ int gz_stream_round(GzFeed &f)
 // text to `sink`.  handled = false: nothing was done (a header this feed does not take: the host
 // feeder starts from the beginning).  Otherwise the text went to the sink up to the end of the
 // file, or up to the place `ho` describes (ho.active), where the host feeder continues.
-int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, GzHandover &ho, size_t &carry, GzStats &stats,
-                   tdg::Utf8State *u8)
+// Maps `path` (an empty file: map.p stays null).  false: it cannot be opened or mapped, or it is not a regular file.
+bool gz_map_file(GzMap &map, const char *path)
+{
+    map.fd = ::open(path, O_RDONLY);
+    if (map.fd < 0) return false;
+    struct stat sb;
+    if (fstat(map.fd, &sb) != 0 || !S_ISREG(sb.st_mode)) return false;
+    map.n = (size_t)sb.st_size;
+    if (!map.n) return true;
+    void *mp = mmap(nullptr, map.n, PROT_READ, MAP_PRIVATE, map.fd, 0);
+    if (mp == MAP_FAILED) return false;
+    map.p = (const uint8_t *)mp;
+    return true;
+}
+
+// The device tables and slots a feed needs, and its settings (round size, test and debug switches).
+int gz_feed_setup(GzFeed &f)
 {
     using namespace tdg;
-    handled = false;
-    ho = GzHandover();
-    GzFeed f{ctx, path, sink, carry, stats, u8};
-    GzMap &map = f.map;
-    map.fd = ::open(path, O_RDONLY);
-    if (map.fd < 0) return TDG_OK;                       // the host feeder reports it
-    struct stat sb;
-    if (fstat(map.fd, &sb) != 0 || !S_ISREG(sb.st_mode) || sb.st_size < 32) return TDG_OK;
-    map.n = (size_t)sb.st_size;
-    void *mp = mmap(nullptr, map.n, PROT_READ, MAP_PRIVATE, map.fd, 0);
-    if (mp == MAP_FAILED) return TDG_OK;
-    map.p = (const uint8_t *)mp;
-    const bool bgzf = Feeder::is_bgzf(map.p, std::min<size_t>(map.n, 1024));
-    if (!bgzf && !f.st.open(map.p, map.n)) return TDG_OK;
+    tdg_ctx *ctx = f.ctx;
     int rc = gz_tables(ctx);
     if (rc) return rc;
     rc = ensure_slots(ctx);
@@ -673,6 +679,23 @@ int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, 
     if (const char *e = getenv("TDG_GZDEV_SYMCAP")) f.fixed_cap = (uint32_t)std::max<unsigned long long>(1024, strtoull(e, nullptr, 10));
     f.debug = getenv("TDG_GZDEV_DEBUG") != nullptr;
     f.threads = gz_io_threads();
+    return TDG_OK;
+}
+
+int gz_device_feed(tdg_ctx *ctx, const char *path, GzSink &sink, bool &handled, GzHandover &ho, size_t &carry, GzStats &stats,
+                   tdg::Utf8State *u8)
+{
+    using namespace tdg;
+    handled = false;
+    ho = GzHandover();
+    GzFeed f{ctx, path, sink, carry, stats, u8};
+    const GzMap &map = f.map;
+    if (!gz_map_file(f.map, path) || map.n < 32) return TDG_OK;          // the host feeder reports it
+    f.stop = map.n;
+    const bool bgzf = Feeder::is_bgzf(map.p, std::min<size_t>(map.n, 1024));
+    if (!bgzf && !f.st.open(map.p, map.n)) return TDG_OK;
+    int rc = gz_feed_setup(f);
+    if (rc) return rc;
     uint8_t *d_window = (uint8_t *)ctx->gz_tabs.p + 512 + 1024;
     if (!bgzf) CK(cudaMemsetAsync(d_window, 0, gzl::WIN, ctx->stream));      // a stream has no history in front of it
     handled = true;
@@ -756,6 +779,70 @@ struct GzCopySink : GzSink {
         return TDG_OK;
     }
 };
+
+// tdg_bgzf_inflate_device's sink: the text goes to caller device memory, behind the text before it
+struct GzDeviceSink : GzSink {
+    uint8_t *dst;
+    size_t cap, used = 0;
+    GzDeviceSink(uint8_t *d, size_t c) : dst(d), cap(c) {}
+    int text(tdg_ctx *ctx, uint8_t *d_buf, size_t &carry, size_t len) override
+    {
+        if (used + len > cap) return fail(ctx, TDG_ERR_ARG, "output buffer too small");
+        CK(cudaMemcpyAsync(dst + used, d_buf + carry, len, cudaMemcpyDeviceToDevice, ctx->stream));
+        used += len;
+        carry = 0;
+        return TDG_OK;
+    }
+};
+
+// The BGZF members in [c_lo, c_hi) of `path`, inflated on the device into dst[0 .. cap) (device memory), by the
+// rounds of gz_bgzf_round.  Nothing goes to the host feeder: a member header that is not BGZF, a member that
+// runs past c_hi and a corrupt member are TDG_ERR_GZIP, a buffer that cannot be had is TDG_ERR_NOMEM.
+int gz_bgzf_inflate_range(tdg_ctx *ctx, const char *path, size_t c_lo, size_t c_hi, uint8_t *dst, size_t cap, uint64_t &n,
+                          bool &high)
+{
+    GzDeviceSink sink(dst, cap);
+    GzStats stats;
+    size_t carry = 0;
+    GzFeed f{ctx, path, sink, carry, stats, nullptr};
+    if (!gz_map_file(f.map, path)) return fail(ctx, TDG_ERR_IO, std::string("cannot open ") + path);
+    if (c_lo > c_hi || c_hi > f.map.n) return fail(ctx, TDG_ERR_ARG, "member range outside the file");
+    int rc = gz_feed_setup(f);
+    if (rc) return rc;
+    f.off = c_lo;
+    f.stop = c_hi;
+    f.done = c_lo == c_hi;
+    while (!f.done) {
+        if ((rc = gz_bgzf_round(f))) return rc;
+        if (f.handover)
+            return fail(ctx, TDG_ERR_GZIP, std::string("gzip error in ") + path + ": no BGZF member chain from offset " +
+                                               std::to_string(f.off) + " to " + std::to_string(c_hi));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    n = sink.used;
+    high = f.high;
+    return TDG_OK;
+}
+
+// The member chain of a BGZF file from offset 0 to its end: every member's offset and ISIZE.  Empty when the
+// file is such a chain, otherwise why it is not.
+std::string bgzf_chain(const GzMap &map, std::vector<uint64_t> &off, std::vector<uint32_t> &isize)
+{
+    size_t at = 0;
+    while (at < map.n) {
+        uint32_t csize = 0, hlen = 0;
+        if (!tdg::Feeder::bgzf_member(map.p + at, std::min<size_t>(map.n - at, 1024), csize, hlen))
+            return "no BGZF member header at offset " + std::to_string(at);
+        if (at + csize > map.n) return "the member at offset " + std::to_string(at) + " runs past the end of the file";
+        uint32_t len;
+        memcpy(&len, map.p + at + csize - 4, 4);
+        if (len > 65536) return "the member at offset " + std::to_string(at) + " holds more than 64 KiB";
+        off.push_back(at);
+        isize.push_back(len);
+        at += csize;
+    }
+    return off.empty() ? "an empty file" : "";
+}
 
 bool gz_device_wanted(const tdg_ctx *ctx, const char *path, uint64_t reads_limit)
 {
