@@ -32,7 +32,8 @@
 extern "C" {
 #endif
 
-/* The splitter's BGZF entry points (tdg_split_bgzf, tdg_bgzf_append, tdg_bgzf_finish) were added
+/* The splitter's BGZF entry points (tdg_split_bgzf, tdg_bgzf_append, tdg_bgzf_finish) and later
+ * ones (tdg_split_count_device, tdg_bgzf_index, tdg_bgzf_inflate_device, tdg_split_device) were added
  * to version 2 without changing any existing signature or behaviour: every version-2 caller keeps
  * working, and the version stays 2 because the test suite pins the ABI at 2.  A library built
  * before them fails at symbol lookup when the binding loads it, not silently. */
@@ -357,6 +358,19 @@ int         tdg_split_count_batch(tdg_ctx *ctx, const char *seqs, const uint64_t
 int         tdg_split_count_device(tdg_ctx *ctx, const void *dev_bytes, size_t n, int final_block,
                                    uint64_t max_records, uint64_t *n_records, uint64_t *consumed,
                                    int *needs_host, uint64_t totals[4]);
+
+/* tdg_split_device: tdg_split_block on bytes already in DEVICE memory (no alignment or padding asked
+ * of dev_bytes; at most 1 GiB per call), with the same *n_records, *consumed, *needs_host, *out,
+ * *out_off and *flags.  totals[] receives the block's reads, reads with barcode and cut site and reads
+ * clipped on the 3' end (0 with *needs_host = 1).  sizes_only != 0 sizes the block without writing
+ * it: *out and *flags stay NULL and out_off[0 .. nbar] are the offsets the block's bytes of every
+ * barcode would have in *out, so out_off[b+1] - out_off[b] is what barcode b's file gains.  Used to
+ * split one rank's text of a file sharded across GPUs: a first pass sizes every barcode's share, a
+ * second writes it at its offset.  Fails with TDG_ERR_STATE while BGZF output is on. */
+int         tdg_split_device(tdg_ctx *ctx, const void *dev_bytes, size_t n, int final_block,
+                             uint64_t max_records, int sizes_only, uint64_t *n_records, uint64_t *consumed,
+                             int *needs_host, const uint8_t **out, const uint64_t **out_off,
+                             const uint8_t **flags, uint64_t totals[3]);
 
 /* BGZF output files for the streaming splitter (the reference writes plain text only).  Every
  * barcode's file is the series of gzip members bgzip writes: member k holds bytes

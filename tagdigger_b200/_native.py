@@ -38,7 +38,7 @@ tdg_count_lines_device tdg_count_file tdg_count_file2 tdg_last_file_info tdg_gz_
 tdg_matrix_device_ptr tdg_stream tdg_stream_wait tdg_other_stream_wait tdg_host_alloc
 tdg_host_free tdg_device_alloc tdg_device_free tdg_memcpy_h2d tdg_memcpy_d2h tdg_launch_count
 tdg_timing_begin tdg_timing_end tdg_set_trim tdg_trim_batch tdg_split_batch tdg_split_begin tdg_split_block
-tdg_split_count_begin tdg_split_count_block tdg_split_count_device tdg_split_count_batch tdg_split_bgzf tdg_bgzf_append tdg_bgzf_finish tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
+tdg_split_count_begin tdg_split_count_block tdg_split_count_device tdg_split_count_batch tdg_split_device tdg_split_bgzf tdg_bgzf_append tdg_bgzf_finish tdg_feed_open tdg_feed_read tdg_feed_close tdg_match_batch tdg_write_counts_csv tdg_write_geno_csv""".split()
 
 
 class TdgError(RuntimeError):
@@ -149,6 +149,8 @@ def lib():
         "tdg_split_count_block": (i32, [vp, vp, sz, i32, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32), vp]),
         "tdg_split_count_device": (i32, [vp, vp, sz, i32, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32), vp]),
         "tdg_split_count_batch": (i32, [vp, vp, vp, vp, u32, vp]),
+        "tdg_split_device": (i32, [vp, vp, sz, i32, u64, i32, ctypes.POINTER(u64), ctypes.POINTER(u64), ctypes.POINTER(i32),
+                                   ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp), vp]),
         "tdg_split_bgzf": (i32, [vp, i32]),
         "tdg_bgzf_append": (i32, [vp, vp, vp, ctypes.POINTER(vp), ctypes.POINTER(vp)]),
         "tdg_bgzf_finish": (i32, [vp, ctypes.POINTER(vp), ctypes.POINTER(vp)]),
@@ -559,6 +561,30 @@ class Engine(object):
         pieces = self._pieces(out, off)
         fl = np.ctypeslib.as_array(ctypes.cast(flags, ctypes.POINTER(ctypes.c_uint8)), shape=(max(nrec.value, 1),))[:nrec.value]
         return nrec.value, used.value, False, pieces, fl
+
+    def split_device(self, dev_ptr, n, final, max_records, sizes_only=False):
+        """split_block on ``n`` bytes already in device memory at ``dev_ptr`` (any alignment; at most 1 GiB
+        per call; not while BGZF output is on).  Returns (records, consumed bytes, needs_host, pieces, flags,
+        totals): pieces and flags as split_block's; with ``sizes_only`` pieces is instead the uint64 array of
+        nbar + 1 offsets (what barcode b's file gains is offs[b+1] - offs[b]) and flags is None.  totals =
+        [reads, with barcode and cut site, clipped on the 3' end] of the block; all None but totals [0, 0, 0]
+        when needs_host."""
+        u64, vp = ctypes.c_uint64, ctypes.c_void_p
+        nrec, used, host = u64(0), u64(0), ctypes.c_int(0)
+        out, off, flags = vp(), vp(), vp()
+        tot = np.zeros(3, dtype=np.uint64)
+        self._ck(self._L.tdg_split_device(self._h, dev_ptr, n, 1 if final else 0, min(int(max_records), (1 << 64) - 1),
+                                          1 if sizes_only else 0, ctypes.byref(nrec), ctypes.byref(used), ctypes.byref(host),
+                                          ctypes.byref(out), ctypes.byref(off), ctypes.byref(flags), tot.ctypes.data))
+        totals = [int(x) for x in tot]
+        if host.value or not off.value:
+            return nrec.value, used.value, bool(host.value), None, None, totals
+        if sizes_only:
+            offs = np.ctypeslib.as_array(ctypes.cast(off, ctypes.POINTER(ctypes.c_uint64)), shape=(self._split_nbar + 1,))
+            return nrec.value, used.value, False, offs.copy(), None, totals
+        pieces = self._pieces(out, off)
+        fl = np.ctypeslib.as_array(ctypes.cast(flags, ctypes.POINTER(ctypes.c_uint8)), shape=(max(nrec.value, 1),))[:nrec.value]
+        return nrec.value, used.value, False, pieces, fl, totals
 
     def split_count_begin(self, patterns, tag_offs, rows, any_base=False):
         """Count mode of the split started by split_begin (after set_tags and set_matrix): the

@@ -317,11 +317,33 @@ class _PlainCount:
         return eng.file_totals()[:3]
 
 
-class _TrimmedCount:
+class _RecordShards:
+    """How a sharded file is placed when its ranges must be cut on RECORD boundaries (the splitter's device
+    front decides whole records): the members ``extra`` / ``payload`` / ``place`` / ``ascii_only`` of
+    :class:`_PlainCount` for the one-pass mode and for :func:`splitter.split_files`.  ``maxreads`` is the
+    split's record limit."""
+    ascii_only = False        # non-ASCII records go to the host (the split entry points' needs_host)
+
+    @property
+    def extra(self):
+        return HEAD_CAP           # room for the lines of the next range that complete the last record
+
+    def payload(self, head):
+        """The range's head (``head()``: :func:`range_head` for a plain file, the loaded text's for a BGZF
+        file), or None when it is too long to send."""
+        h = head()
+        return None if h is None else list(h)
+
+    def place(self, lines, payloads, rank):
+        """The range's owned text and record budget (:func:`plan_trimmed_shards`); None to handle the file whole."""
+        shards = plan_trimmed_shards(lines, [bytes(p) for p in payloads], _native.limit_from_maxreads(self.maxreads))
+        return None if shards is None else shards[rank]
+
+
+class _TrimmedCount(_RecordShards):
     """count_files' one-pass split-trim-count mode (``adapter``), with the members of :class:`_PlainCount`.
     Set-up errors surface in the order of the two-stage run: every file's split, then the count."""
     line = "{0}: Reads: {1} With barcode and cut site: {2} Clipped on 3' end: {3} With tag: {4}"
-    ascii_only = False        # non-ASCII records go to the host (tdg_split_count_device's needs_host)
 
     def __init__(self, bckeys, files, rows, tags, cutsite, maxreads, adapter, split_cutsite, split_maxreads):
         from . import hostio, splitter
@@ -342,26 +364,11 @@ class _TrimmedCount:
         self.tags = self.plan.tags
         self.bckeys, self.rows, self.maxreads = bckeys, rows, split_maxreads
 
-    @property
-    def extra(self):
-        return HEAD_CAP           # room for the lines of the next range that complete the last record
-
     def whole(self, eng, f, next_file=None):
         """[reads, with barcode and cut site, clipped on the 3' end, with tag] of file ``f``."""
         from . import splitter
         return splitter.count_trimmed_file(eng, f, self.bckeys[f][0], self.rows[f], self.plan, cutsite=self.cutsite,
                                            adapter=self.adapter, maxreads=self.maxreads)
-
-    def payload(self, head):
-        """The range's head (``head()``: :func:`range_head` for a plain file, the loaded text's for a BGZF
-        file), or None when it is too long to send."""
-        h = head()
-        return None if h is None else list(h)
-
-    def place(self, lines, payloads, rank):
-        """The range's owned text and record budget (:func:`plan_trimmed_shards`); None to count the file whole."""
-        shards = plan_trimmed_shards(lines, [bytes(p) for p in payloads], _native.limit_from_maxreads(self.maxreads))
-        return None if shards is None else shards[rank]
 
     def own(self, eng, f, rank, dev, n, shard):
         from . import splitter
@@ -689,6 +696,46 @@ def _load_share(eng, mode, path, rank, world, index):
     return dev, n, payload
 
 
+def _place_share(eng, mode, path, rank, world, gather, index=None):
+    """Steps 1 to 3 of :func:`_count_sharded`, which :func:`splitter.split_files` shares: this rank's text of
+    ``path`` loaded (``mode.extra`` bytes of room behind it), its line starts counted, the first ``gather``
+    and ``mode.place``.  Returns (device pointer, length, share), or None on every rank when the file is to
+    be handled whole by rank 0 (nothing is left allocated then)."""
+    if gather is None:
+        raise ValueError("sharding a file across ranks needs a gather callable (see dist_gather)")
+    dev, n, lines, payload = None, 0, 0, None
+    try:
+        loaded = _load_share(eng, mode, path, rank, world, index)
+        if loaded is not None:
+            dev, n, payload = loaded
+            lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
+    except (OSError, _native.TdgError):
+        if dev is not None:
+            eng.device_free(dev)
+            dev = None                          # this rank votes for handling the file whole
+    every = gather([0] if dev is None else [1, lines] + payload)
+    share = None
+    if all(x[0] for x in every):
+        share = mode.place([x[1] for x in every], [x[2:] for x in every], rank)
+    if share is None:
+        if dev is not None:
+            eng.device_free(dev)
+        return None
+    return dev, n, share
+
+
+def _gather_checked(gather, path, err, values, doing):
+    """A ``gather`` of [failed, values...] after a step every rank ran on its own share: raises ``err`` on the
+    rank that failed, a RuntimeError naming the first failed rank on the others.  Returns every rank's values."""
+    every = gather([0 if err is None else 1] + list(values))
+    if err is not None:
+        raise err
+    failed = [k for k, x in enumerate(every) if x[0]]
+    if failed:
+        raise RuntimeError("%s: rank %d failed while %s its byte range" % (path, failed[0], doing))
+    return [x[1:] for x in every]
+
+
 def _count_sharded(eng, mode, path, rank, world, gather, index=None):
     """One file that count_files cuts into one range per rank (:func:`shard_files`), in either counting
     mode (``mode``: :class:`_PlainCount` or :class:`_TrimmedCount`); ``index``: the member index of a BGZF
@@ -704,31 +751,16 @@ def _count_sharded(eng, mode, path, rank, world, gather, index=None):
        a byte >= 0x80 in BGZF text of the plain mode) or
        ``mode.place`` refuses, rank 0 counts the file whole (``mode.whole``), exactly as a file dealt whole:
        nothing has touched the matrix yet;
+    (steps 1 to 3 are :func:`_place_share`)
     4. otherwise every rank counts its range (``mode.own``);
     5. a second ``gather`` of [failed, totals] sums the totals.  A rank that failed in step 4 raises its
        own exception after that gather, the others a RuntimeError naming it.
 
     Returns the file's totals, or None on the ranks other than 0 when rank 0 counted the file whole."""
-    if gather is None:
-        raise ValueError("sharding a file across ranks needs a gather callable (see dist_gather)")
-    dev, n, lines, payload = None, 0, 0, None
-    try:
-        loaded = _load_share(eng, mode, path, rank, world, index)
-        if loaded is not None:
-            dev, n, payload = loaded
-            lines, _last = eng.count_lines_device(dev, n, 0, _native.TDG_PREV_NONE if rank == 0 else _native.TDG_PREV_LF)
-    except (OSError, _native.TdgError):
-        if dev is not None:
-            eng.device_free(dev)
-            dev = None                          # this rank votes for counting the file whole
-    every = gather([0] if dev is None else [1, lines] + payload)
-    share = None
-    if all(x[0] for x in every):
-        share = mode.place([x[1] for x in every], [x[2:] for x in every], rank)
-    if share is None:
-        if dev is not None:
-            eng.device_free(dev)
+    placed = _place_share(eng, mode, path, rank, world, gather, index)
+    if placed is None:
         return mode.whole(eng, path) if rank == 0 else None
+    dev, n, share = placed
     tot, err = [], None
     try:
         tot = mode.own(eng, path, rank, dev, n, share)
@@ -736,13 +768,8 @@ def _count_sharded(eng, mode, path, rank, world, gather, index=None):
         err = e
     finally:
         eng.device_free(dev)
-    every = gather([0 if err is None else 1] + [int(t) for t in tot])
-    if err is not None:
-        raise err
-    failed = [k for k, x in enumerate(every) if x[0]]
-    if failed:
-        raise RuntimeError("%s: rank %d failed while counting its byte range" % (path, failed[0]))
-    return [sum(t) for t in zip(*(x[1:] for x in every))]
+    every = _gather_checked(gather, path, err, [int(t) for t in tot], "counting")
+    return [sum(t) for t in zip(*every)]
 
 
 def dist_gather(values):

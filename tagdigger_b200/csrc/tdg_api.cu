@@ -1949,21 +1949,27 @@ int tdg_split_begin(tdg_ctx *ctx, const char *barcodes, const uint32_t *bar_off,
     return TDG_OK;
 }
 
-int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, uint64_t max_records,
-                    uint64_t *n_records, uint64_t *consumed, int *needs_host, const uint8_t **out,
-                    const uint64_t **out_off, const uint8_t **flags)
+// tdg_split_block (host bytes) and tdg_split_device (device bytes, optionally sizes only): one block
+// through split_front, then either the offsets and bytes of every barcode's file (bar_tile_sums ->
+// bar_tile_scan -> bar_bases -> split_write) or, with sizes_only, their sizes alone (split_tally).
+// totals (may be null) receive the block's reads, reads with barcode and cut site and reads clipped.
+static int split_run(tdg_ctx *ctx, const char *what, const uint8_t *bytes, cudaMemcpyKind kind, size_t n, int final_block,
+                     uint64_t max_records, bool sizes_only, uint64_t *n_records, uint64_t *consumed, int *needs_host,
+                     const uint8_t **out, const uint64_t **out_off, const uint8_t **flags, uint64_t *totals)
 {
     int rc = need_device(ctx);
     if (rc) return rc;
     if (!ctx->have_split || !ctx->have_trim || !ctx->have_bar) return fail(ctx, TDG_ERR_STATE, "tdg_split_begin has not been called");
     if (!n_records || !consumed || !needs_host || !out || !out_off || !flags || (!bytes && n)) return fail(ctx, TDG_ERR_ARG, "null argument");
-    if (n > ((size_t)1 << 30)) return fail(ctx, TDG_ERR_ARG, "tdg_split_block: at most 1 GiB per block");
+    if (n > ((size_t)1 << 30)) return fail(ctx, TDG_ERR_ARG, std::string(what) + ": at most 1 GiB per block");
     *n_records = 0;
     *consumed = 0;
     *needs_host = 0;
     *out = nullptr;
     *out_off = nullptr;
     *flags = nullptr;
+    if (totals)
+        for (int k = 0; k < 3; k++) totals[k] = 0;
     if (n == 0 || max_records == 0) return TDG_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
@@ -1972,7 +1978,45 @@ int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_bloc
     uint64_t nrec = 0;
     uint32_t last_end = 0;
     unsigned long long *bar_total = nullptr;
-    rc = split_front(ctx, bytes, cudaMemcpyHostToDevice, n, final_block, max_records, w, nrec, last_end, [&](uint64_t records) {
+    if (sizes_only) {
+        // tally [nbar] bytes per barcode, [3] flag counts, complex flag
+        unsigned long long *tally = nullptr;
+        rc = split_front(ctx, bytes, kind, n, final_block, max_records, w, nrec, last_end, [&](uint64_t) {
+            int rc;
+            if ((rc = grow(ctx, ctx->sp_base, (size_t)(nbar + 4) * sizeof(unsigned long long), false))) return rc;
+            if ((rc = grow(ctx, ctx->sp_hbase, (size_t)(nbar + 4) * sizeof(unsigned long long), true))) return rc;
+            tally = (unsigned long long *)ctx->sp_base.p;
+            w.complex_flag = (uint32_t *)(tally + nbar + 3);
+            CK(cudaMemsetAsync(tally, 0, (size_t)(nbar + 3) * sizeof(unsigned long long), st));
+            return TDG_OK;
+        });
+        if (rc || nrec == 0) return rc;
+        const uint32_t grid = (uint32_t)std::min<uint64_t>((nrec + tdg::SPLIT_REC_TILE - 1) / tdg::SPLIT_REC_TILE, 1024);
+        tdg::split_tally<<<grid, tdg::SPLIT_REC_TILE, nbar * sizeof(uint32_t), st>>>(w, tally);
+        ctx->launches += 1;
+        unsigned long long *h = (unsigned long long *)ctx->sp_hbase.p;
+        CK(cudaMemcpyAsync(h, tally, (size_t)(nbar + 4) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        CK(cudaGetLastError());
+        *n_records = nrec;
+        *consumed = last_end >= n ? n : (uint64_t)last_end + 1;
+        if ((uint32_t)h[nbar + 3] != 0) {
+            *needs_host = 1;
+            return TDG_OK;
+        }
+        if (totals)
+            for (int k = 0; k < 3; k++) totals[k] = h[nbar + k];
+        unsigned long long run = 0;                  // the sizes become offsets, in place
+        for (uint32_t b = 0; b < nbar; b++) {
+            const unsigned long long c = h[b];
+            h[b] = run;
+            run += c;
+        }
+        h[nbar] = run;
+        *out_off = (const uint64_t *)h;
+        return TDG_OK;
+    }
+    rc = split_front(ctx, bytes, kind, n, final_block, max_records, w, nrec, last_end, [&](uint64_t records) {
         const uint32_t n_rtiles = (uint32_t)((records + tdg::SPLIT_REC_TILE - 1) / tdg::SPLIT_REC_TILE);
         int rc;
         if ((rc = grow(ctx, ctx->sp_sums, (size_t)n_rtiles * nbar * sizeof(uint32_t), false))) return rc;
@@ -2024,7 +2068,32 @@ int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_bloc
     *out = (const uint8_t *)ctx->sp_hout.p;
     *out_off = (const uint64_t *)hbase;
     *flags = (const uint8_t *)ctx->sp_hflags.p;
+    if (totals) {
+        totals[0] = nrec;
+        for (uint64_t r = 0; r < nrec; r++) {
+            totals[1] += (*flags)[r] & tdg::SPLIT_FLAG_BAR ? 1 : 0;
+            totals[2] += (*flags)[r] & tdg::SPLIT_FLAG_CLIP ? 1 : 0;
+        }
+    }
     return TDG_OK;
+}
+
+int tdg_split_block(tdg_ctx *ctx, const uint8_t *bytes, size_t n, int final_block, uint64_t max_records,
+                    uint64_t *n_records, uint64_t *consumed, int *needs_host, const uint8_t **out,
+                    const uint64_t **out_off, const uint8_t **flags)
+{
+    return split_run(ctx, "tdg_split_block", bytes, cudaMemcpyHostToDevice, n, final_block, max_records, false, n_records,
+                     consumed, needs_host, out, out_off, flags, nullptr);
+}
+
+int tdg_split_device(tdg_ctx *ctx, const void *dev_bytes, size_t n, int final_block, uint64_t max_records, int sizes_only,
+                     uint64_t *n_records, uint64_t *consumed, int *needs_host, const uint8_t **out,
+                     const uint64_t **out_off, const uint8_t **flags, uint64_t totals[3])
+{
+    if (ctx && ctx->bz_on) return fail(ctx, TDG_ERR_STATE, "tdg_split_device: BGZF output is on (tdg_split_bgzf)");
+    if (ctx && !totals) return fail(ctx, TDG_ERR_ARG, "null argument");
+    return split_run(ctx, "tdg_split_device", (const uint8_t *)dev_bytes, cudaMemcpyDeviceToDevice, n, final_block,
+                     max_records, sizes_only != 0, n_records, consumed, needs_host, out, out_off, flags, totals);
 }
 
 int tdg_split_count_begin(tdg_ctx *ctx, const char *bases, const uint32_t *off, const uint32_t *tag_off, uint32_t npat,

@@ -20,6 +20,9 @@
 //   bar_tile_scan   per barcode: exclusive prefix over the tiles, totals, barcode bases
 //   split_write     per tile: in-order offsets of its records inside their barcode's stream,
 //                   then the bytes
+// Sizing a block without writing it (tdg_split_device with sizes_only): the same front up to
+// split_records, then
+//   split_tally     output bytes per barcode and the three flag counts of the block
 //
 // Counting the trimmed reads without writing them (tdg_split_count_block): the same front up to
 // split_records, then
@@ -346,6 +349,43 @@ __global__ void bar_bases(const unsigned long long *bar_total, unsigned long lon
         run += bar_total[b];
     }
     bar_base[nbar] = run;
+}
+
+// Sizes only (tdg_split_device with sizes_only): the bytes every barcode's file gains from the block and
+// its three flag counts, without offsets or output.  Each CTA walks records grid-stride, sums output bytes
+// per barcode in shared memory (32-bit, as bar_tile_scan's in-block offsets) and adds its non-zero sums to
+// tally[0 .. nbar); tally[nbar + 0..2] gain reads, reads with barcode and cut site, reads clipped on the
+// 3' end.  A block split_records left to the host (complex flag) is not tallied: the host sizes it.
+__global__ void __launch_bounds__(SPLIT_REC_TILE) split_tally(const SplitWork w, unsigned long long *tally)
+{
+    if (*w.complex_flag) return;
+    extern __shared__ uint32_t sums[];          // [nbar]
+    __shared__ uint32_t part[3][SPLIT_REC_TILE / 32];
+    for (uint32_t i = threadIdx.x; i < w.nbar; i += SPLIT_REC_TILE) sums[i] = 0;
+    __syncthreads();
+    uint32_t v[3] = {0, 0, 0};
+    for (uint32_t r = blockIdx.x * SPLIT_REC_TILE + threadIdx.x; r < w.n_rec; r += gridDim.x * SPLIT_REC_TILE) {
+        const SplitRec rec = w.rec[r];
+        const uint8_t fl = w.flags[r];
+        v[0] += 1;
+        v[1] += fl & SPLIT_FLAG_BAR ? 1u : 0u;
+        v[2] += fl & SPLIT_FLAG_CLIP ? 1u : 0u;
+        if (rec.bar >= 0) atomicAdd(&sums[rec.bar], split_out_len(rec, w.bar_off));
+    }
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        const uint32_t s = __reduce_add_sync(0xFFFFFFFFu, v[k]);
+        if (lane == 0) part[k][warp] = s;
+    }
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < w.nbar; i += SPLIT_REC_TILE)
+        if (sums[i]) atomicAdd(tally + i, (unsigned long long)sums[i]);
+    if (threadIdx.x < 3) {
+        unsigned long long s = 0;
+        for (uint32_t i = 0; i < SPLIT_REC_TILE / 32; i++) s += part[threadIdx.x][i];
+        if (s) atomicAdd(tally + w.nbar + threadIdx.x, s);
+    }
 }
 
 __device__ __forceinline__ void split_copy(uint8_t *dst, const uint8_t *src, uint32_t n, uint32_t lane, bool upper)
